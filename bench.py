@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the similarity-search hot path on synthetic corpora (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is ONE single-query top-100 scan of the whole corpus (configs[1]: 10M x 256-byte rows
@@ -20,6 +20,9 @@ c1_sqlite= (N = 1) configs[0]: 100k x 256 in SQLite, top-50: verbatim SQL + UDF 
            bare loop, and the GPU path through the Engine mirror including hydration
 --impl reference = the CPU restatement of the reference's scan (oracle/, the reference itself
            needs a Rust toolchain this image does not have) on all host cores.
+--dump-outputs DIR = after the timed steps, write what the last step of each timed path returned as DIR/<name>.npy
+           (single_*: the headline step, e2e_*: the host-buffer step, batched_*: the last batch; see result_arrays).
+           The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -61,7 +64,13 @@ def parse():
     ap.add_argument("--sweep", action="store_true", help="run the configs[4] d x k sweep at N = 1 too (always on for N >= 2)")
     ap.add_argument("--no-sweep", action="store_true", help="skip the configs[4] sweep of a multi-GPU run")
     ap.add_argument("--sweep-rows", type=int, default=SWEEP_ROWS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step of each path as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def peaks():
@@ -276,6 +285,24 @@ def planted_check(res_ids, res_dist):
     return bool(ok)
 
 
+def result_arrays(name, ids, dist, dot, norm2, counts):
+    """--dump-outputs: [nq][k] results as a caller receives them and the [nq] counts.  Entries past a query's count are 0;
+    image ids and the int32 terms are stored as float64, which holds them exactly."""
+    counts = np.asarray(counts, np.int64).reshape(-1)
+    valid = np.arange(np.shape(ids)[-1])[None, :] < counts[:, None]
+    out = {f"{name}_count": counts.astype(np.float64)}
+    for field, v, t in (("image_id", ids, np.float64), ("dist", dist, np.float32), ("dot", dot, np.float64), ("norm2", norm2, np.float64)):
+        out[f"{name}_{field}"] = np.where(valid, np.asarray(v).reshape(len(counts), -1), 0).astype(t)
+    return out
+
+
+def hit_arrays(name, hits, counts):
+    """result_arrays of pbx_hit records (bytes or HIT_DTYPE) as the device-resident API returns them."""
+    from pixelbox_b200 import _native as nat
+    h = np.ascontiguousarray(hits).view(nat.HIT_DTYPE).reshape(len(counts), -1)
+    return result_arrays(name, h["image_id"], h["dist"], h["dot"], h["norm2"], counts)
+
+
 # ---------------------------------------------------------------------------------------------
 # configs[0]: 100k x 256 in SQLite, top-50 (the only configuration the reference itself runs end to end)
 # ---------------------------------------------------------------------------------------------
@@ -408,10 +435,11 @@ def run_ours(args):
 
     def searcher(sc, corpus, dq, d_hits, d_cnt):
         def step_device(q, nq=1):
+            """Returns (hits, counts): on one GPU the whole buffers, in which query q has slot q; sharded, this call's."""
             if sc is None:
                 corpus.search_device(dq.data_ptr() + q * dim, nq, k, 1e3, d_hits.data_ptr() + q * k * 24, d_cnt.data_ptr() + 4 * q, stream.cuda_stream)
-                return d_hits
-            return sc.search_device(dq[q:q + nq].reshape(-1), nq, k, 1e3)[0]
+                return d_hits, d_cnt
+            return sc.search_device(dq[q:q + nq].reshape(-1), nq, k, 1e3)
         return step_device
 
     def time_batch(step, nqb, reps):
@@ -461,10 +489,14 @@ def run_ours(args):
         barrier()
         e0.record(stream)
         for i in range(args.steps):
-            step_device(i % NQ)
+            out = step_device(i % NQ)
         e1.record(stream)
         barrier()
         ms = e0.elapsed_time(e1)
+        dump = {}
+        if args.dump_outputs and rank == 0:
+            slot = (args.steps - 1) % NQ if sc is None else 0
+            dump.update(hit_arrays("single", out[0][slot * k * 24:(slot + 1) * k * 24].cpu().numpy(), out[1][slot:slot + 1].cpu().numpy()))
         # ---- e2e: host buffers through the public API --------------------------------------------
         for i in range(3):
             step_e2e(i)
@@ -476,6 +508,8 @@ def run_ours(args):
         torch.cuda.synchronize()
         e2e_s = time.perf_counter() - t0
         barrier()
+        if args.dump_outputs and rank == 0:
+            dump.update(result_arrays("e2e", last.ids, last.dist, last.dot, last.norm2, [len(last.ids)]))
         clocks = sampler.stop() if rank == 0 else None
     ms, e2e_ms = allmax([ms, e2e_s * 1e3])
 
@@ -512,11 +546,13 @@ def run_ours(args):
         def batch_step():
             if sc is None:
                 corpus.search_device(d_bq.data_ptr(), nqb, k, 1e3, d_bh.data_ptr(), d_bc.data_ptr(), stream.cuda_stream)
-                return d_bh
-            return sc.search_device(d_bq, nqb, k, 1e3)[0]       # every shard contracts its rows against all queries, then the exchange
+                return d_bh, d_bc
+            return sc.search_device(d_bq, nqb, k, 1e3)          # every shard contracts its rows against all queries, then the exchange
 
-        bms, out_b = time_batch(batch_step, nqb, 10)
+        bms, (out_b, out_bc) = time_batch(batch_step, nqb, 10)
         bh = out_b.cpu().numpy().view(nat.HIT_DTYPE).reshape(nqb, k)
+        if args.dump_outputs and rank == 0:
+            dump.update(hit_arrays("batched", bh, out_bc.cpu().numpy()))
         tops = 2.0 * total_rows * nqb * dim / (bms * 1e-3) / 1e12
         peak_tops = ctypes.c_double(0.0)
         nat.check(L.pbx_int8_peak(local_rank, ctypes.byref(peak_tops)))
@@ -707,6 +743,10 @@ def run_ours(args):
             line["northstar"] = northstar
         if sweep is not None:
             line["sweep"] = sweep
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         if world == 1:
             # free the 10M-row corpus before the small-table comparison and the CPU baseline
             corpus.close()

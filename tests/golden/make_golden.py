@@ -68,8 +68,9 @@ def make_pairs():
 def make_topk():
     rng = np.random.default_rng(20260102)
     cases = {}
-    specs = [("uniform_d8", 300, 8, None), ("uniform_d64", 1500, 64, None), ("uniform_d256", 2000, 256, None),
-             ("cluster_d256", 3000, 256, (40, 3)), ("cluster_d64_ties", 2000, 64, (10, 0)), ("cluster_d1024", 600, 1024, (8, 2))]
+    # row counts keep the fixture under 1 MB: its corpora are random bytes and do not compress
+    specs = [("uniform_d8", 300, 8, None), ("uniform_d64", 1200, 64, None), ("uniform_d256", 1000, 256, None),
+             ("cluster_d256", 1000, 256, (40, 3)), ("cluster_d64_ties", 2000, 64, (10, 0)), ("cluster_d1024", 220, 1024, (8, 2))]
     for name, n, d, cl in specs:
         corpus = rng.integers(0, 256, size=(n, d), dtype=np.uint8) if cl is None else clustered_corpus(rng, n, d, *cl)
         ids = np.sort(rng.choice(np.arange(1, 10 * n), size=n, replace=False)).astype(np.int64)

@@ -56,7 +56,7 @@ def bound_and_scores(rows, q, thr):
 @pytest.mark.parametrize("d", [32, 64, 256, 1024])
 @pytest.mark.parametrize("kind", ["uniform", "wild", "near"])
 def test_bound_never_excludes_a_passing_row(d, kind):
-    rng = np.random.default_rng(hash((d, kind)) % (2 ** 32))
+    rng = np.random.default_rng([d, ["uniform", "wild", "near"].index(kind)])     # not hash(): it changes with PYTHONHASHSEED
     checked = 0
     for _ in range(120):
         rows, q = block_case(rng, d, kind)

@@ -1,5 +1,5 @@
-"""Multi-GPU parity (needs >= 2 B200s on the box: NCCL does not put two ranks on one device; on a single-GPU box the test is
-deselected by tests/conftest.py and tests/test_gpu_exchange.py covers the same exchange with ranks sharing cuda:0): launches
+"""Multi-GPU parity (needs >= 2 B200s on the machine: NCCL does not put two ranks on one device; on a single-GPU machine the test
+is skipped by tests/conftest.py and tests/test_gpu_exchange.py covers the same exchange with ranks sharing cuda:0): launches
 tools/shard_check.py with one process per GPU over NCCL."""
 import os
 import subprocess
@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_two_gpu_sharded_search_matches_oracle():
     import torch
     n = torch.cuda.device_count()
-    assert n >= 2, "multigpu tests are deselected on boxes with one GPU (tests/conftest.py)"
+    assert n >= 2, "multigpu tests are skipped on machines with one GPU (tests/conftest.py)"
     world = 2 if n < 4 else 4
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}", "--master-addr", "127.0.0.1",
            "--master-port", "29631", os.path.join(ROOT, "tools", "shard_check.py")]
