@@ -118,6 +118,24 @@ PBX_API int pbx_corpus_flush(pbx_corpus* c);
  * `cuda_stream` (a cudaStream_t; NULL = an internal stream), which is synchronised before the rows are published. */
 PBX_API int pbx_corpus_append_device(pbx_corpus* c, const int64_t* d_image_ids, const uint8_t* d_hashes, uint64_t n, void* cuda_stream);
 
+/* Replaces: `DELETE FROM semantic_hashes WHERE image_id IN (...)` as seen by later scans.  Hook: after the DELETE of a
+ * removed tracked folder commits (the TODO of remove_tracked_folder, src/engine.rs:414), with the folder's image ids; also
+ * what follows an external edit of the table, and the first half of replacing a hash (remove, then append).
+ *   - every committed or pending row whose image_id is in image_ids[0, n) is removed; the corpus does not enforce unique
+ *     ids, so an id on several rows removes all of them.  Ids that match nothing are ignored; an id repeated in the
+ *     request counts once.  *out_removed (may be NULL) receives the number of rows removed.
+ *   - n == 0 returns PBX_OK with 0 removed; NULL c, or NULL image_ids with n > 0, is PBX_E_INVALID.
+ *   - synchronous, and atomic with respect to searches: a search sees all of a removal or none of it.  Work already
+ *     enqueued by pbx_search_device (on any stream) completes against the old rows; every search issued after the call
+ *     returns gives exactly what a corpus freshly loaded with the surviving rows gives (ids, dist bit for bit, dot, norm2).
+ *   - appends that arrived before the call (coalesced pending ones included) are subject to it, later ones are not: remove
+ *     then append of the same id replaces the row.
+ *   - capacity is not released; later appends reuse the freed rows.  Surviving rows may change position: the removed
+ *     rows below the new size n' are filled, in row order, with the surviving rows at or above n', in row order.
+ * Cost: a host sort of the request, one pass over the ids (8 bytes per row) plus the block metadata (8 bytes per row) on
+ * the device, and a copy of the moved rows only. */
+PBX_API int pbx_corpus_remove(pbx_corpus* c, const int64_t* image_ids, uint64_t n, uint64_t* out_removed);
+
 /* Bench/test only: fills the shard on the device with rows [first_row, first_row + n) of the
  * counter-based synthetic corpus (pixelbox_b200/synth.py), image_id = global row + 1. */
 PBX_API int pbx_corpus_fill_synthetic(pbx_corpus* c, uint64_t n, uint64_t seed, uint64_t first_row);
@@ -126,7 +144,8 @@ PBX_API int pbx_corpus_size(const pbx_corpus* c, uint64_t* n_rows);
 PBX_API int pbx_corpus_dim(const pbx_corpus* c, uint32_t* dim);
 
 /* Copies rows [first, first + n) back to the host (tests, and result hydration of
- * IndexedImage.visual_hash, src/engine.rs:385).  Either output may be NULL. */
+ * IndexedImage.visual_hash, src/engine.rs:385).  Either output may be NULL.  Row positions are those of the moment:
+ * pbx_corpus_remove moves surviving rows into the positions of removed ones. */
 PBX_API int pbx_corpus_read_rows(const pbx_corpus* c, uint64_t first, uint64_t n, int64_t* image_ids, uint8_t* hashes);
 
 /* Waits for everything enqueued on the corpus' own stream (pbx_search_device with a NULL stream). */
@@ -194,6 +213,9 @@ PBX_API int pbx_sharded_create(uint32_t dim, uint64_t capacity_hint, const int* 
 PBX_API void pbx_sharded_destroy(pbx_sharded* s);
 PBX_API int pbx_sharded_load(pbx_sharded* s, const int64_t* image_ids, const uint8_t* hashes, uint64_t n);
 PBX_API int pbx_sharded_append(pbx_sharded* s, const int64_t* image_ids, const uint8_t* hashes, uint64_t n);
+/* pbx_corpus_remove over all shards: ids are global and do not name a shard, so every shard applies the whole request
+ * (one after the other, atomic with respect to pbx_sharded_search); *out_removed (may be NULL) is the total. */
+PBX_API int pbx_sharded_remove(pbx_sharded* s, const int64_t* image_ids, uint64_t n, uint64_t* out_removed);
 /* Bench/test only: shard i holds rows [i * rows_per_shard, (i + 1) * rows_per_shard) of the synthetic corpus. */
 PBX_API int pbx_sharded_fill_synthetic(pbx_sharded* s, uint64_t rows_per_shard, uint64_t seed);
 PBX_API int pbx_sharded_size(const pbx_sharded* s, uint64_t* n_rows);

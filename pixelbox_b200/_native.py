@@ -26,7 +26,7 @@ DEFAULT_K = 100          # the literal LIMIT of src/engine.rs:381
 # every symbol include/pixelbox_b200.h declares (tests check the library exports exactly these)
 EXPORTS = [
     "pbx_corpus_create", "pbx_corpus_destroy", "pbx_corpus_load", "pbx_corpus_append", "pbx_corpus_flush", "pbx_corpus_append_device",
-    "pbx_quantize_device", "pbx_corpus_fill_synthetic",
+    "pbx_quantize_device", "pbx_corpus_fill_synthetic", "pbx_corpus_remove", "pbx_sharded_remove",
     "pbx_corpus_size", "pbx_corpus_dim", "pbx_corpus_read_rows", "pbx_corpus_synchronize", "pbx_search", "pbx_search_hits", "pbx_search_device",
     "pbx_merge_hits", "pbx_merge_hits_device", "pbx_exchange_create", "pbx_exchange_handle", "pbx_exchange_connect",
     "pbx_exchange_allgather_merge", "pbx_exchange_search_hits", "pbx_exchange_destroy",
@@ -79,6 +79,8 @@ def lib() -> ctypes.CDLL:
         "pbx_corpus_append_device": (i32, [vp, vp, vp, u64, vp]),
         "pbx_quantize_device": (i32, [i32, vp, u64, vp, vp]),
         "pbx_corpus_fill_synthetic": (i32, [vp, u64, u64, u64]),
+        "pbx_corpus_remove": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
+        "pbx_sharded_remove": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
         "pbx_corpus_size": (i32, [vp, ctypes.POINTER(u64)]),
         "pbx_corpus_dim": (i32, [vp, ctypes.POINTER(u32)]),
         "pbx_corpus_read_rows": (i32, [vp, u64, u64, vp, u8p]),

@@ -32,6 +32,13 @@ def _as_u8_2d(a, dim: int, what: str) -> np.ndarray:
     return a
 
 
+def _remove(fn, handle, image_ids) -> int:
+    ids = np.ascontiguousarray(np.asarray(image_ids, dtype=np.int64)).reshape(-1)
+    removed = ctypes.c_uint64(0)
+    nat.check(fn(handle, nat.ptr(ids), ids.size, ctypes.byref(removed)))
+    return int(removed.value)
+
+
 class Corpus:
     def __init__(self, dim: int, capacity_hint: int = 0, device: int = 0):
         self._h = ctypes.c_void_p(0)
@@ -91,6 +98,11 @@ class Corpus:
         """pbx_corpus_append_device: [n] int64 ids and [n][dim] u8 rows already in device memory (raw pointers)."""
         nat.check(nat.lib().pbx_corpus_append_device(self._h, ctypes.c_void_p(d_ids_ptr), ctypes.c_void_p(d_hashes_ptr), int(n),
                                                      ctypes.c_void_p(stream or 0)))
+
+    def remove(self, image_ids) -> int:
+        """pbx_corpus_remove: removes every row (pending ones included) whose image_id is listed; returns the number of
+        rows removed.  Surviving rows from the tail move into the freed positions (see read_rows)."""
+        return _remove(nat.lib().pbx_corpus_remove, self._h, image_ids)
 
     def fill_synthetic(self, n: int, seed: int, first_row: int = 0) -> None:
         nat.check(nat.lib().pbx_corpus_fill_synthetic(self._h, int(n), int(seed), int(first_row)))
@@ -231,6 +243,10 @@ class MultiDeviceCorpus:
         if ids.shape != (hashes.shape[0],):
             raise nat.PbxError(-1, "append: one image_id per hash row required")
         nat.check(nat.lib().pbx_sharded_append(self._h, nat.ptr(ids), nat.ptr(hashes), hashes.shape[0]))
+
+    def remove(self, image_ids) -> int:
+        """pbx_sharded_remove: every shard removes the listed ids; returns the total number of rows removed."""
+        return _remove(nat.lib().pbx_sharded_remove, self._h, image_ids)
 
     def fill_synthetic(self, rows_per_shard: int, seed: int) -> None:
         nat.check(nat.lib().pbx_sharded_fill_synthetic(self._h, int(rows_per_shard), int(seed)))

@@ -15,6 +15,7 @@
 
 #include "finalize.cuh"
 #include "batch.cuh"
+#include "remove.cuh"
 
 using namespace pbx;
 
@@ -824,6 +825,98 @@ extern "C" int pbx_corpus_read_rows(const pbx_corpus* cc, uint64_t first, uint64
     if (image_ids) CU_TRY(cudaMemcpy(image_ids, c->d_ids + first, n * sizeof(int64_t), cudaMemcpyDeviceToHost));
     if (hashes) CU_TRY(cudaMemcpy2D(hashes, c->dim, c->d_rows + first * c->pitch, c->pitch, c->dim, n, cudaMemcpyDeviceToHost));
     return PBX_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// removal
+// ------------------------------------------------------------------------------------------------
+// The request as the kernels want it: sorted, every id once.  A host std::sort, O(r log r): for large requests it is the
+// largest part of the call (tools/remove_time.py).
+static int sorted_request(const int64_t* image_ids, uint64_t n, std::vector<int64_t>* out) {
+    try { out->assign(image_ids, image_ids + n); } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
+    std::sort(out->begin(), out->end());
+    out->erase(std::unique(out->begin(), out->end()), out->end());
+    return PBX_OK;
+}
+
+// Removes every row whose id is in `req` (sorted, unique) by hole filling from the tail (remove.cuh).  Locks as
+// pbx_corpus_load does: the pending appends are flushed first, so they are subject to the removal; with mu held no search
+// can be enqueued, and the removal stream waits for the last one already enqueued (ev_chain: every search waits for its
+// predecessor, so for all of them) before it touches a row.  The new n is published after the stream is synchronised.
+static int remove_sorted(pbx_corpus* c, const std::vector<int64_t>& req, uint64_t* out_removed) {
+    std::lock_guard<std::mutex> alk(c->append_mu);
+    int rc = flush_pending_locked(c);
+    if (rc != PBX_OK) return rc;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CU_TRY(cudaSetDevice(c->device));
+    const uint64_t n = c->n.load();
+    if (n == 0 || req.empty()) return PBX_OK;
+    cudaStream_t s = c->copy_stream;
+    if (c->chain_valid) CU_TRY(cudaStreamWaitEvent(s, c->ev_chain, 0));
+    const uint64_t tiles = (n + kRemoveTileRows - 1) / kRemoveTileRows;
+    // scratch, stream-ordered (no device-wide synchronisation): [request][removed rows u64, pairs u32][flag words][tile counts x 2]
+    const size_t req_bytes = req.size() * sizeof(int64_t), flag_bytes = (n + 31) / 32 * sizeof(uint32_t);
+    const size_t off_cnt = (req_bytes + 15) / 16 * 16, off_flags = off_cnt + 16, off_tiles = off_flags + (flag_bytes + 15) / 16 * 16;
+    unsigned char* scratch = nullptr;
+    uint32_t* pairs = nullptr;
+    CU_TRY(cudaMallocAsync(reinterpret_cast<void**>(&scratch), off_tiles + 2 * tiles * sizeof(uint32_t), s));
+    int64_t* d_req = reinterpret_cast<int64_t*>(scratch);
+    u64* d_removed = reinterpret_cast<u64*>(scratch + off_cnt);
+    uint32_t* d_pairs = reinterpret_cast<uint32_t*>(scratch + off_cnt + 8);
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(scratch + off_flags);
+    uint32_t* d_tile_holes = reinterpret_cast<uint32_t*>(scratch + off_tiles);
+    uint32_t* d_tile_srcs = d_tile_holes + tiles;
+    u64 m = 0;
+    cudaError_t e = cudaMemcpyAsync(d_req, req.data(), req_bytes, cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_removed, 0, sizeof(u64), s);
+    if (e == cudaSuccess) {
+        remove_mark_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(c->d_ids, n, d_req, req.size(), d_flags, d_removed);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&m, d_removed, sizeof(u64), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);        // the one synchronisation before the end: m sizes the rest
+    if (e == cudaSuccess && m > n) { cudaFreeAsync(scratch, s); cudaStreamSynchronize(s); return fail(PBX_E_INTERNAL, "removal counted %llu of %llu rows", (unsigned long long)m, (unsigned long long)n); }
+    const uint64_t n_keep = n - m;
+    // holes below n_keep == survivors at or above it, at most min(m, n_keep): the exact number stays on the device
+    const uint64_t max_pairs = std::min<uint64_t>(m, n_keep);
+    if (e == cudaSuccess && max_pairs) e = cudaMallocAsync(reinterpret_cast<void**>(&pairs), 2 * max_pairs * sizeof(uint32_t), s);
+    if (e == cudaSuccess && max_pairs) {
+        uint32_t* d_holes = pairs;
+        uint32_t* d_srcs = pairs + max_pairs;
+        remove_count_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(d_flags, n, n_keep, d_tile_holes, d_tile_srcs);
+        remove_scan_kernel<<<1, 1024, 0, s>>>(d_tile_holes, d_tile_srcs, (uint32_t)tiles, d_pairs);
+        remove_place_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(d_flags, n, n_keep, d_tile_holes, d_tile_srcs, d_holes, d_srcs);
+        const uint64_t chunks = max_pairs * c->pitch16;
+        const unsigned grid = (unsigned)std::min<uint64_t>((chunks + 255) / 256, (uint64_t)c->sm_count * 8);
+        remove_move_kernel<<<grid, 256, 0, s>>>(d_holes, d_srcs, d_pairs, c->pitch16, reinterpret_cast<uint4*>(c->d_rows), c->d_ids, c->d_inv, c->d_rsum);
+        e = cudaGetLastError();
+    }
+    // A moved row may lie outside its new block's {norm, rowterm} range, and the batched epilogue trusts that range as a
+    // bound: recompute every block below n_keep (8 bytes per row), the last one over the rows below n_keep only.
+    if (e == cudaSuccess && m && n_keep) {
+        const uint64_t blocks = (n_keep + 31) / 32;
+        block_meta_kernel<<<(unsigned)((blocks + 7) / 8), 256, 0, s>>>(c->d_inv, c->d_rsum, c->dim, 0, blocks, n_keep, c->d_bmeta);
+        e = cudaGetLastError();
+    }
+    if (pairs) cudaFreeAsync(pairs, s);
+    cudaFreeAsync(scratch, s);
+    const cudaError_t e2 = cudaStreamSynchronize(s);
+    if (e == cudaSuccess) e = e2;
+    // on failure n stays: the rows below it may be half moved, but a CUDA error here leaves the context unusable anyway
+    if (e != cudaSuccess) return fail(PBX_E_CUDA, "removal failed: %s", cudaGetErrorString(e));
+    c->n.store(n_keep);
+    if (out_removed) *out_removed = m;
+    return PBX_OK;
+}
+
+extern "C" int pbx_corpus_remove(pbx_corpus* c, const int64_t* image_ids, uint64_t n, uint64_t* out_removed) {
+    if (out_removed) *out_removed = 0;
+    if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (n && !image_ids) return fail(PBX_E_INVALID, "NULL image_ids with n > 0");
+    if (n == 0) return PBX_OK;
+    std::vector<int64_t> req;
+    int rc = sorted_request(image_ids, n, &req);
+    return rc == PBX_OK ? remove_sorted(c, req, out_removed) : rc;
 }
 
 // ------------------------------------------------------------------------------------------------

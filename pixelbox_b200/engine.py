@@ -195,3 +195,25 @@ class Engine:
                 self.corpus.append(np.array([appended[0]], np.int64), np.frombuffer(appended[1], np.uint8).reshape(1, -1))
             else:
                 self.skipped_rows += 1
+
+    def remove_images(self, ids) -> None:
+        """Deletes images from the two tables the similarity query joins (`images`, `semantic_hashes`) in one
+        transaction, then removes their hashes from the device corpus: the hook the TODO in remove_tracked_folder
+        (src/engine.rs:414) would call with the folder's image ids."""
+        ids = [int(i) for i in np.asarray(ids, dtype=np.int64).reshape(-1)]
+        if not ids:
+            return
+        conn = self.write_connection
+        try:
+            for first in range(0, len(ids), 500):                        # SQLite's bound-parameter limit
+                part = ids[first:first + 500]
+                marks = ",".join("?" * len(part))
+                conn.execute(f"DELETE FROM semantic_hashes WHERE image_id IN ({marks})", part)
+                conn.execute(f"DELETE FROM images WHERE id IN ({marks})", part)
+            conn.commit()
+        except Exception:
+            conn.rollback()
+            raise
+        # as for inserts, the device corpus follows only what has been committed
+        if self.corpus is not None:
+            self.corpus.remove(np.asarray(ids, np.int64))

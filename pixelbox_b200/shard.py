@@ -112,6 +112,12 @@ class ShardedCorpus:
         """Shard r holds global rows [r*rows_per_shard, (r+1)*rows_per_shard) of the synthetic corpus."""
         self.local.fill_synthetic(rows_per_shard, seed, self.rank * rows_per_shard)
 
+    def remove(self, image_ids) -> int:
+        """Every rank passes the same ids (they are global: any shard may hold them) and removes them from its shard;
+        returns the number of rows removed over all ranks, on every rank."""
+        mine = np.array([self.local.remove(image_ids)], np.int64)
+        return int(self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).sum())
+
     def total_rows(self) -> int:
         t = torch.tensor([len(self.local)], dtype=torch.int64, device=self._comm_dev())
         dist.all_reduce(t, group=self.group)
