@@ -54,6 +54,12 @@ extern "C" {
 #define PBX_COUNT_EXCHANGE_TIMEOUT 0xFFFFFFFFu    /* a peer did not post its records within ~10 s               */
 #define PBX_COUNT_EXACT_LAUNCH_FAILED 0xFFFFFFFEu /* the device-side launch of the exact pass was refused: the  */
                                                   /* hits of this query are the uncertified fast-pass ones      */
+#define PBX_COUNT_FILTER_UNSORTED 0xFFFFFFFDu     /* pbx_search_device_filtered: the filter ids were not sorted */
+                                                  /* ascending; the hits of every query of the call are invalid */
+
+/* Filter modes of the *_filtered searches. */
+#define PBX_FILTER_INCLUDE 0u   /* only rows whose image_id is listed      */
+#define PBX_FILTER_EXCLUDE 1u   /* every row except those whose id is listed */
 
 /* DEFAULT_MAX_QUERY_DISTANCE and the literal LIMIT of the reference (src/engine.rs:23, :381). */
 #define PBX_DEFAULT_MAX_DIST 1e3
@@ -185,6 +191,36 @@ PBX_API int pbx_search_hits(pbx_corpus* c, const uint8_t* queries, uint32_t nq, 
 PBX_API int pbx_search_device(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist,
                               pbx_hit* d_hits, uint32_t* d_count, void* cuda_stream);
 
+/* ---- filtered search: the k nearest rows among a set of image ids ----------------------------------------------------
+ * Replaces: the similarity query with an id condition added,
+ *   ... FROM semantic_hashes ... WHERE dist < ? AND semantic_hashes.image_id IN (...)      (PBX_FILTER_INCLUDE)
+ *   ... FROM semantic_hashes ... WHERE dist < ? AND semantic_hashes.image_id NOT IN (...)  (PBX_FILTER_EXCLUDE)
+ *   ORDER BY dist ASC LIMIT k
+ * which the `similar:` term of Engine::query (src/engine.rs:282-292) meant to combine with filename and tag terms, and
+ * which a folder search ("similar images in this folder") needs; the host turns such conditions into ids.
+ *   - Each call takes the arguments of its unfiltered twin plus (filter_ids, n_filter, filter_mode).  One filter applies
+ *     to all nq queries of the call.
+ *   - Contract: the result is exactly what the unfiltered twin returns on a corpus loaded with only the allowed rows:
+ *     count, ids, order, dist bit for bit, dot, norm2, ties by image_id, and the plateau rule applied to allowed rows.
+ *   - The filter applies to the rows that exist when the call is made, coalesced pending appends included; rows that
+ *     pbx_corpus_remove moved are found by id.  Ids that match no row are ignored, a repeated id counts once, and an id
+ *     on several rows includes or excludes all of them.
+ *   - An empty INCLUDE set gives count 0 for every query; an empty EXCLUDE set is the unfiltered search.
+ *   - NULL filter_ids with n_filter > 0, an unknown filter_mode or n_filter > PBX_MAX_ROWS: PBX_E_INVALID.
+ *   - Host forms accept the ids in any order (a sorted copy is made; ids already in order cost one check pass).
+ * Cost: the unfiltered search (the whole shard is streamed, whatever the filter selects: a selective filter is not
+ * faster) plus one mark pass over the row ids (8 bytes per row, a binary search in the set per row).  On the batched
+ * path (many queries per call) a very selective filter costs several times the unfiltered call (DESIGN.md section 10). */
+PBX_API int pbx_search_filtered(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
+                                int64_t* out_ids, float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count,
+                                const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode);
+/* Device-resident form, with the contract of pbx_search_device.  d_filter_ids is a DEVICE pointer on the corpus' device,
+ * read in stream order on `cuda_stream`; it must be sorted ascending (duplicates allowed).  The order is checked on the
+ * device, without a host synchronisation: unsorted ids set every count of the call to PBX_COUNT_FILTER_UNSORTED. */
+PBX_API int pbx_search_device_filtered(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist,
+                                       pbx_hit* d_hits, uint32_t* d_count, void* cuda_stream,
+                                       const int64_t* d_filter_ids, uint64_t n_filter, uint32_t filter_mode);
+
 /* Merge step after the all-gather (SURVEY.md section 8e): gathered is [n_shards][nq][k] hits and
  * counts is [n_shards][nq], both in HOST memory; every shard list is already ordered by
  * (dist, image_id).  Writes the global first k per query under the same order.  Pure host
@@ -227,6 +263,11 @@ PBX_API int pbx_sharded_search(pbx_sharded* s, const uint8_t* queries, uint32_t 
                                int64_t* out_ids, float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count);
 PBX_API int pbx_sharded_search_hits(pbx_sharded* s, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
                                     pbx_hit* out_hits, uint32_t* out_count);
+/* pbx_search_filtered over all shards: ids are global, every shard marks its rows against the same set; the merge is
+ * unchanged (each shard's list is exact for its allowed rows, so the merged list is exact for all of them). */
+PBX_API int pbx_sharded_search_filtered(pbx_sharded* s, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
+                                        int64_t* out_ids, float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count,
+                                        const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode);
 
 /* ---- the exchange step over NVLink peer memory (one process per GPU) ---------------------------------
  * Replaces: nothing upstream (PixelBox is single-process); it is the one exchange step of the row-sharded path
@@ -249,6 +290,10 @@ PBX_API int pbx_exchange_allgather_merge(pbx_exchange* x, const pbx_hit* d_local
  * queries and receives the global result.  nq <= 1024 per call. */
 PBX_API int pbx_exchange_search_hits(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
                                      pbx_hit* out_hits, uint32_t* out_count);
+/* The same step for a filtered search (pbx_search_filtered's filter contract): every rank passes the same global ids. */
+PBX_API int pbx_exchange_search_hits_filtered(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k,
+                                              double max_dist, pbx_hit* out_hits, uint32_t* out_count,
+                                              const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode);
 PBX_API void pbx_exchange_destroy(pbx_exchange* x);
 
 /* ---- the scalar function, for external users of the DB -----------------------------------

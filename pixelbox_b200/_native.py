@@ -22,12 +22,16 @@ PBX_MAX_DIM = 4096
 PBX_MAX_K = 2048
 DEFAULT_MAX_DIST = 1e3   # DEFAULT_MAX_QUERY_DISTANCE, src/engine.rs:23
 DEFAULT_K = 100          # the literal LIMIT of src/engine.rs:381
+PBX_FILTER_INCLUDE = 0   # filtered searches: only the listed image ids
+PBX_FILTER_EXCLUDE = 1   # ... every row except the listed image ids
+PBX_COUNT_FILTER_UNSORTED = 0xFFFFFFFD   # pbx_search_device_filtered: the device filter ids were not sorted
 
 # every symbol include/pixelbox_b200.h declares (tests check the library exports exactly these)
 EXPORTS = [
     "pbx_corpus_create", "pbx_corpus_destroy", "pbx_corpus_load", "pbx_corpus_append", "pbx_corpus_flush", "pbx_corpus_append_device",
     "pbx_quantize_device", "pbx_corpus_fill_synthetic", "pbx_corpus_remove", "pbx_sharded_remove",
     "pbx_corpus_size", "pbx_corpus_dim", "pbx_corpus_read_rows", "pbx_corpus_synchronize", "pbx_search", "pbx_search_hits", "pbx_search_device",
+    "pbx_search_filtered", "pbx_search_device_filtered", "pbx_sharded_search_filtered", "pbx_exchange_search_hits_filtered",
     "pbx_merge_hits", "pbx_merge_hits_device", "pbx_exchange_create", "pbx_exchange_handle", "pbx_exchange_connect",
     "pbx_exchange_allgather_merge", "pbx_exchange_search_hits", "pbx_exchange_destroy",
     "pbx_sharded_create", "pbx_sharded_destroy", "pbx_sharded_load", "pbx_sharded_append", "pbx_sharded_fill_synthetic", "pbx_sharded_size",
@@ -88,6 +92,8 @@ def lib() -> ctypes.CDLL:
         "pbx_search": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp]),
         "pbx_search_hits": (i32, [vp, u8p, u32, u32, f64, vp, vp]),
         "pbx_search_device": (i32, [vp, vp, u32, u32, f64, vp, vp, vp]),
+        "pbx_search_filtered": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp, vp, u64, u32]),
+        "pbx_search_device_filtered": (i32, [vp, vp, u32, u32, f64, vp, vp, vp, vp, u64, u32]),
         "pbx_merge_hits": (i32, [vp, vp, u32, u32, u32, vp, vp]),
         "pbx_merge_hits_device": (i32, [i32, vp, vp, u32, u32, u32, vp, vp, vp]),
         "pbx_exchange_create": (i32, [i32, u32, u32, u32, u32, ctypes.POINTER(vp)]),
@@ -95,6 +101,7 @@ def lib() -> ctypes.CDLL:
         "pbx_exchange_connect": (i32, [vp, vp]),
         "pbx_exchange_allgather_merge": (i32, [vp, vp, u32, u32, vp, vp, vp]),
         "pbx_exchange_search_hits": (i32, [vp, vp, u8p, u32, u32, f64, vp, vp]),
+        "pbx_exchange_search_hits_filtered": (i32, [vp, vp, u8p, u32, u32, f64, vp, vp, vp, u64, u32]),
         "pbx_exchange_destroy": (None, [vp]),
         "pbx_sharded_create": (i32, [u32, u64, vp, i32, ctypes.POINTER(vp)]),
         "pbx_sharded_destroy": (None, [vp]),
@@ -106,6 +113,7 @@ def lib() -> ctypes.CDLL:
         "pbx_sharded_shard": (i32, [vp, u32, ctypes.POINTER(vp)]),
         "pbx_sharded_search": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp]),
         "pbx_sharded_search_hits": (i32, [vp, u8p, u32, u32, f64, vp, vp]),
+        "pbx_sharded_search_filtered": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp, vp, u64, u32]),
         "pbx_cosine_distance_pairs": (i32, [i32, u8p, u8p, u64, u32, vp, vp, vp, vp]),
         "pbx_byte_distance_pairs": (i32, [i32, u8p, u8p, u64, u32, vp, vp]),
         "pbx_hamming_distance_pairs": (i32, [i32, u8p, u8p, u64, u32, vp, vp]),
@@ -131,6 +139,16 @@ def lib() -> ctypes.CDLL:
 def check(rc: int) -> None:
     if rc != PBX_OK:
         raise PbxError(rc, lib().pbx_last_error().decode("utf-8", "replace"))
+
+
+def filter_args(within, excluding):
+    """(ids int64 array, mode) of the `within=` / `excluding=` keywords of the search methods: the image ids a search
+    is restricted to, or the ids it must skip.  Passing both is an error."""
+    if within is not None and excluding is not None:
+        raise ValueError("pass `within` or `excluding`, not both")
+    ids = within if within is not None else excluding
+    ids = np.ascontiguousarray(np.asarray(ids, dtype=np.int64)).reshape(-1)
+    return ids, (PBX_FILTER_INCLUDE if within is not None else PBX_FILTER_EXCLUDE)
 
 
 def ptr(a) -> ctypes.c_void_p:

@@ -114,12 +114,19 @@ class Corpus:
         return ids, rows
 
     # -- search ------------------------------------------------------------------------------
-    def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST) -> List[SearchResult]:
+    def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None,
+               excluding=None) -> List[SearchResult]:
         """pbx_search: host buffers in, host buffers out; one SearchResult per query.
+
+        within / excluding (image ids, any order; at most one of them): pbx_search_filtered, the k nearest rows among
+        the rows whose id is listed, or among all rows except those -- exactly what a corpus holding only those rows
+        would return.
 
         This is the call the latency of a single interactive query goes through, so the wrapper keeps its own cost
         down: output arrays and their raw pointers are cached per thread and (nq, k), the query pointer is taken from
         the array interface (ndarray.ctypes costs ~1 us per use)."""
+        if within is not None or excluding is not None:
+            return self._search_filtered(queries, k, max_dist, within, excluding)
         if type(queries) is np.ndarray and queries.dtype == np.uint8 and queries.flags.c_contiguous and (
                 (queries.ndim == 2 and queries.shape[1] == self.dim) or (queries.ndim == 1 and queries.size == self.dim)):
             q = queries if queries.ndim == 2 else queries.reshape(1, self.dim)
@@ -148,6 +155,16 @@ class Corpus:
         counts = cnt.tolist()
         return [SearchResult(ids[i, :c].copy(), dist[i, :c].copy(), dot[i, :c].copy(), n2[i, :c].copy()) for i, c in enumerate(counts)]
 
+    def _search_filtered(self, queries, k, max_dist, within, excluding) -> List[SearchResult]:
+        fids, mode = nat.filter_args(within, excluding)
+        q = _as_u8_2d(queries, self.dim, "search")
+        nq, k = q.shape[0], int(k)
+        ids, dist, dot, n2 = (np.zeros((nq, k), t) for t in (np.int64, np.float32, np.int32, np.int32))
+        cnt = np.zeros(nq, np.uint32)
+        nat.check(nat.lib().pbx_search_filtered(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(ids), nat.ptr(dist), nat.ptr(dot),
+                                                nat.ptr(n2), nat.ptr(cnt), nat.ptr(fids), fids.size, mode))
+        return [SearchResult(ids[i, :c].copy(), dist[i, :c].copy(), dot[i, :c].copy(), n2[i, :c].copy()) for i, c in enumerate(cnt.tolist())]
+
     def search_hits(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST) -> Tuple[np.ndarray, np.ndarray]:
         """pbx_search_hits: ([nq][k] pbx_hit records, [nq] counts) -- the per-shard half of a sharded search."""
         q = _as_u8_2d(queries, self.dim, "search_hits")
@@ -171,6 +188,20 @@ class Corpus:
         nat.check(nat.lib().pbx_search_device(self._h, ctypes.c_void_p(d_queries_ptr), int(nq), int(k), float(max_dist),
                                               ctypes.c_void_p(d_hits_ptr), ctypes.c_void_p(d_count_ptr),
                                               ctypes.c_void_p(stream)))
+
+    def search_device_filtered(self, d_queries_ptr: int, nq: int, k: int, max_dist: float, d_hits_ptr: int, d_count_ptr: int,
+                               d_filter_ids_ptr: int, n_filter: int, mode: int = nat.PBX_FILTER_INCLUDE,
+                               stream: Optional[int] = None) -> None:
+        """pbx_search_device_filtered: search_device restricted by [n_filter] int64 image ids at d_filter_ids_ptr (device
+        memory, sorted ascending; mode PBX_FILTER_INCLUDE or PBX_FILTER_EXCLUDE).  Unsorted ids are reported on the
+        device: every count of the call becomes PBX_COUNT_FILTER_UNSORTED."""
+        if stream is None:
+            stream = 0
+        elif stream == 0:
+            stream = 1
+        nat.check(nat.lib().pbx_search_device_filtered(self._h, ctypes.c_void_p(d_queries_ptr), int(nq), int(k), float(max_dist),
+                                                       ctypes.c_void_p(d_hits_ptr), ctypes.c_void_p(d_count_ptr), ctypes.c_void_p(stream),
+                                                       ctypes.c_void_p(d_filter_ids_ptr), int(n_filter), int(mode)))
 
     def synchronize(self) -> None:
         """Waits for everything enqueued on the corpus' own stream."""
@@ -264,7 +295,12 @@ class MultiDeviceCorpus:
             nat.check(nat.lib().pbx_sharded_shard(self._h, i, ctypes.byref(h)))
             nat.check(nat.lib().pbx_set_candidate_slack(h, int(slack)))
 
-    def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST) -> List[SearchResult]:
+    def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None,
+               excluding=None) -> List[SearchResult]:
+        """pbx_sharded_search; within / excluding as in Corpus.search (pbx_sharded_search_filtered)."""
+        filtered = within is not None or excluding is not None
+        if filtered:
+            fids, mode = nat.filter_args(within, excluding)
         q = _as_u8_2d(queries, self.dim, "search")
         nq, k = q.shape[0], int(k)
         ids = np.zeros((nq, k), np.int64)
@@ -272,8 +308,12 @@ class MultiDeviceCorpus:
         dot = np.zeros((nq, k), np.int32)
         n2 = np.zeros((nq, k), np.int32)
         cnt = np.zeros(nq, np.uint32)
-        nat.check(nat.lib().pbx_sharded_search(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(ids), nat.ptr(dist), nat.ptr(dot),
-                                               nat.ptr(n2), nat.ptr(cnt)))
+        if filtered:
+            nat.check(nat.lib().pbx_sharded_search_filtered(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(ids), nat.ptr(dist),
+                                                            nat.ptr(dot), nat.ptr(n2), nat.ptr(cnt), nat.ptr(fids), fids.size, mode))
+        else:
+            nat.check(nat.lib().pbx_sharded_search(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(ids), nat.ptr(dist), nat.ptr(dot),
+                                                   nat.ptr(n2), nat.ptr(cnt)))
         return [SearchResult(ids[i, :c].copy(), dist[i, :c].copy(), dot[i, :c].copy(), n2[i, :c].copy()) for i, c in enumerate(cnt.tolist())]
 
 

@@ -177,6 +177,14 @@ struct pbx_corpus {
     uint32_t* d_tile_counter = nullptr;
     uint32_t* d_hist = nullptr;       // kappa histogram of the scan CTAs' final lists (zeroed by the finalize kernel)
     unsigned long long* d_exact_passes = nullptr;
+    // filtered searches (stream-ordered after ev_chain like the rest of the search scratch)
+    uint32_t* d_allow = nullptr;      // bit per row: the row may be returned
+    size_t allow_words = 0;
+    u64* d_filter_words = nullptr;    // [0] allowed rows (mark_ids_kernel), [1] low word: a device filter was unsorted
+    int64_t* d_filter_ids = nullptr;  // the sorted ids of a host-form filter
+    size_t filter_ids_cap = 0;
+    const uint32_t* cur_allow = nullptr;  // filter of the search being enqueued (NULL: none); exact_setup picks it up
+    const u64* cur_allowed = nullptr;
     // pinned staging
     uint8_t* h_queries = nullptr;
     size_t h_queries_cap = 0;
@@ -410,6 +418,26 @@ static int ensure_cand(pbx_corpus* c, size_t bytes) {
     return PBX_OK;
 }
 
+// Row bitmap of filtered searches for `words` 32-row words, and room for `n_ids` host-form filter ids.
+static int ensure_filter_scratch(pbx_corpus* c, size_t words, uint64_t n_ids) {
+    if (!c->d_filter_words) CU_TRY(cudaMalloc(&c->d_filter_words, 2 * sizeof(u64)));
+    if (words > c->allow_words) {
+        words = std::max(words, c->allow_words + c->allow_words / 2);
+        CU_TRY(cudaDeviceSynchronize());
+        cudaFree(c->d_allow); c->d_allow = nullptr; c->allow_words = 0;
+        CU_TRY(cudaMalloc(&c->d_allow, words * sizeof(uint32_t)));
+        c->allow_words = words;
+    }
+    if (n_ids > c->filter_ids_cap) {
+        const uint64_t want = std::max<uint64_t>(n_ids, c->filter_ids_cap + c->filter_ids_cap / 2);
+        CU_TRY(cudaDeviceSynchronize());
+        cudaFree(c->d_filter_ids); c->d_filter_ids = nullptr; c->filter_ids_cap = 0;
+        CU_TRY(cudaMalloc(&c->d_filter_ids, want * sizeof(int64_t)));
+        c->filter_ids_cap = want;
+    }
+    return PBX_OK;
+}
+
 // Dynamic shared memory limits are per function and per device, and static shared memory counts
 // against the 48 KB default as well: raise every kernel's cap once, when a corpus is created on a device.
 template <typename Kern>
@@ -424,21 +452,27 @@ static cudaError_t init_kernel_attributes() {
     const size_t scan_cap = 8192 * sizeof(KeyX) + PBX_MAX_DIM * 2 + 1024;       // largest cap (keep 4096 + tile) + generic query stage
     const size_t fin_cap = 200 * 1024;
     cudaError_t e = cudaSuccess;
-#define PBX_ALLOW(LL, CC)                                                          \
-    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false>, scan_cap);    \
+#define PBX_ALLOW(LL, CC)                                                                                       \
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false>, scan_cap);                                 \
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, scan_minb(LL * CC), false, true>, scan_cap); \
     if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, true>, scan_cap);
     PBX_ALLOW(1, 1) PBX_ALLOW(2, 1) PBX_ALLOW(4, 1) PBX_ALLOW(8, 1) PBX_ALLOW(16, 1) PBX_ALLOW(32, 1) PBX_ALLOW(32, 2) PBX_ALLOW(32, 4)
 #undef PBX_ALLOW
-#define PBX_ALLOW_M(LL, CC, MM)                                                        \
-    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, MM>, scan_cap);    \
+#define PBX_ALLOW_M(LL, CC, MM)                                                                   \
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, MM>, scan_cap);               \
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, MM, false, true>, scan_cap);  \
     if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, true, MM>, scan_cap);
     PBX_EXTRA_SHAPES(PBX_ALLOW_M)
 #undef PBX_ALLOW_M
-#define PBX_ALLOW_R(LL, CC, MM) if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, MM, true>, scan_cap);
+#define PBX_ALLOW_R(LL, CC, MM)                                                                  \
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, MM, true>, scan_cap);        \
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<LL, CC, false, MM, true, true>, scan_cap);
     PBX_RAGGED_SHAPES(PBX_ALLOW_R)
 #undef PBX_ALLOW_R
     if (e == cudaSuccess) e = allow_smem(scan_kernel<16, 1, false, 3>, scan_cap);
     if (e == cudaSuccess) e = allow_smem(scan_kernel<16, 1, false, 4>, scan_cap);
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<16, 1, false, 3, false, true>, scan_cap);
+    if (e == cudaSuccess) e = allow_smem(scan_kernel<16, 1, false, 4, false, true>, scan_cap);
     if (e == cudaSuccess) e = allow_smem(scan_generic_kernel<false>, scan_cap);
     if (e == cudaSuccess) e = allow_smem(scan_generic_kernel<true>, scan_cap);
     if (e == cudaSuccess) e = allow_smem(prep_seed_kernel, PBX_MAX_DIM * 2 + 1024);
@@ -565,6 +599,7 @@ extern "C" void pbx_corpus_destroy(pbx_corpus* c) {
     cudaFree(c->d_qpad); cudaFree(c->d_colterm); cudaFree(c->d_thr); cudaFree(c->d_bcnt); cudaFree(c->d_boverflow); cudaFree(c->d_bcand);
     cudaFree(c->d_bhist); cudaFree(c->d_binvq); cudaFree(c->d_seedlb);
     cudaFree(c->d_hits); cudaFree(c->d_cand); cudaFree(c->d_cand_cnt); cudaFree(c->d_tile_counter); cudaFree(c->d_hist);
+    cudaFree(c->d_allow); cudaFree(c->d_filter_words); cudaFree(c->d_filter_ids);
     cudaFreeHost(c->h_queries); cudaFreeHost(c->h_hits); cudaFreeHost(c->h_stage); cudaFreeHost(c->h_flag);
     if (c->ev_chain) cudaEventDestroy(c->ev_chain);
     if (c->ev_t0) cudaEventDestroy(c->ev_t0);
@@ -831,10 +866,11 @@ extern "C" int pbx_corpus_read_rows(const pbx_corpus* cc, uint64_t first, uint64
 // removal
 // ------------------------------------------------------------------------------------------------
 // The request as the kernels want it: sorted, every id once.  A host std::sort, O(r log r): for large requests it is the
-// largest part of the call (tools/remove_time.py).
+// largest part of the call (tools/remove_time.py).  Ids that are already in order (a folder's ids as SQLite returns them
+// from an index, searched again and again) cost one check pass instead.
 static int sorted_request(const int64_t* image_ids, uint64_t n, std::vector<int64_t>* out) {
     try { out->assign(image_ids, image_ids + n); } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
-    std::sort(out->begin(), out->end());
+    if (!std::is_sorted(out->begin(), out->end())) std::sort(out->begin(), out->end());
     out->erase(std::unique(out->begin(), out->end()), out->end());
     return PBX_OK;
 }
@@ -870,7 +906,7 @@ static int remove_sorted(pbx_corpus* c, const std::vector<int64_t>& req, uint64_
     cudaError_t e = cudaMemcpyAsync(d_req, req.data(), req_bytes, cudaMemcpyHostToDevice, s);
     if (e == cudaSuccess) e = cudaMemsetAsync(d_removed, 0, sizeof(u64), s);
     if (e == cudaSuccess) {
-        remove_mark_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(c->d_ids, n, d_req, req.size(), d_flags, d_removed);
+        mark_ids_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(c->d_ids, n, d_req, req.size(), 0u, d_flags, d_removed);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(&m, d_removed, sizeof(u64), cudaMemcpyDeviceToHost, s);
@@ -948,11 +984,14 @@ static cudaError_t launch_pdl(void (*kern)(const P), int grid, int block, size_t
     return cudaLaunchKernelEx(&cfg, kern, params);
 }
 
-template <bool EXACT>
-static cudaError_t launch_scan(const pbx_corpus* c, const ScanParams& p, int grid, size_t smem, cudaStream_t s) {
-#define PBX_SCAN_CASE(LL, CC)                                                                                   \
-    {                                                                                                           \
-        return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT>, grid, kScanThreads, smem, s, p);               \
+// FILTER: the fast pass of a filtered search (scan_kernel's FILTER instantiations); the exact pass and the generic kernel
+// test p.allow at run time.
+template <bool EXACT, bool FILTER>
+static cudaError_t launch_scan_as(const pbx_corpus* c, const ScanParams& p, int grid, size_t smem, cudaStream_t s) {
+    static_assert(!(EXACT && FILTER), "the exact pass has no FILTER instantiation");
+#define PBX_SCAN_CASE(LL, CC)                                                                                                     \
+    {                                                                                                                             \
+        return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, scan_minb(LL * CC), false, FILTER>, grid, kScanThreads, smem, s, p); \
     }
     switch (c->pitch16) {
         case 1: PBX_SCAN_CASE(1, 1)
@@ -961,21 +1000,21 @@ static cudaError_t launch_scan(const pbx_corpus* c, const ScanParams& p, int gri
         case 8: PBX_SCAN_CASE(8, 1)
         case 16:
             if constexpr (!EXACT) {                  // occupancy variants of the d=256 fast pass (pbx_set_scan_ctas_per_sm)
-                if (c->ctas_per_sm == 3 || c->ctas_per_sm == 0) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 3>, grid, kScanThreads, smem, s, p);
-                if (c->ctas_per_sm >= 4) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 4>, grid, kScanThreads, smem, s, p);
+                if (c->ctas_per_sm == 3 || c->ctas_per_sm == 0) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 3, false, FILTER>, grid, kScanThreads, smem, s, p);
+                if (c->ctas_per_sm >= 4) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 4, false, FILTER>, grid, kScanThreads, smem, s, p);
             }
             PBX_SCAN_CASE(16, 1)
         case 32: PBX_SCAN_CASE(32, 1)
         case 64: PBX_SCAN_CASE(32, 2)
         case 128: PBX_SCAN_CASE(32, 4)
-#define PBX_SCAN_CASE_M(LL, CC, MM) case (LL) * (CC): return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, MM>, grid, kScanThreads, smem, s, p);
+#define PBX_SCAN_CASE_M(LL, CC, MM) case (LL) * (CC): return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, MM, false, FILTER>, grid, kScanThreads, smem, s, p);
         PBX_EXTRA_SHAPES(PBX_SCAN_CASE_M)
 #undef PBX_SCAN_CASE_M
         default: {
             if constexpr (!EXACT) {
                 // any other row length: the smallest lane layout that holds it, with the row stride at run time
 #define PBX_SCAN_CASE_R(LL, CC, MM) \
-    if (c->pitch16 <= (LL) * (CC)) return launch_pdl<ScanParams>(scan_kernel<LL, CC, false, MM, true>, grid, kScanThreads, smem, s, p);
+    if (c->pitch16 <= (LL) * (CC)) return launch_pdl<ScanParams>(scan_kernel<LL, CC, false, MM, true, FILTER>, grid, kScanThreads, smem, s, p);
                 PBX_RAGGED_SHAPES(PBX_SCAN_CASE_R)
 #undef PBX_SCAN_CASE_R
             }
@@ -984,6 +1023,14 @@ static cudaError_t launch_scan(const pbx_corpus* c, const ScanParams& p, int gri
         }
     }
 #undef PBX_SCAN_CASE
+}
+
+template <bool EXACT>
+static cudaError_t launch_scan(const pbx_corpus* c, const ScanParams& p, int grid, size_t smem, cudaStream_t s) {
+    if constexpr (!EXACT) {
+        if (p.allow) return launch_scan_as<false, true>(c, p, grid, smem, s);
+    }
+    return launch_scan_as<EXACT, false>(c, p, grid, smem, s);
 }
 
 // true for the row pitches with a compile-time lane layout (1, 3, 5, 6, 8 times a power of two, see scan.cuh)
@@ -1186,7 +1233,7 @@ static ExactSetup exact_setup(const pbx_corpus* c, uint32_t q, uint32_t k, doubl
     sp.pitch16 = c->pitch16; sp.dim = c->dim;
     sp.q16 = c->d_q16 + (size_t)q * c->pitch; sp.qbytes = c->d_qbytes + (size_t)q * c->pitch; sp.qh = c->d_qh + q;
     sp.keep = k; sp.cap = cap_scan_x; sp.cand = c->d_cand; sp.cand_cnt = c->d_cand_cnt; sp.tile_counter = c->d_tile_counter;
-    sp.hist = c->d_hist; sp.status = c->d_status + q; sp.max_dist = max_dist;
+    sp.hist = c->d_hist; sp.status = c->d_status + q; sp.max_dist = max_dist; sp.allow = c->cur_allow;
     FinalizeExactParams& xp = x.fin;
     xp.cand = reinterpret_cast<const KeyX*>(c->d_cand); xp.cand_cnt = c->d_cand_cnt; xp.grid = (uint32_t)x.grid; xp.k = k;
     xp.cap = cap_merge_x; xp.dim = c->dim; xp.pitch = c->pitch; xp.rows = c->d_rows; xp.qbytes = sp.qbytes;
@@ -1262,7 +1309,7 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
     mp.cand = c->d_bcand; mp.cand_cnt = c->d_bcnt; mp.overflow = c->d_boverflow;
     mp.bhist = c->d_bhist; mp.inv_q = c->d_binvq; mp.thr_live = c->d_thr; mp.keep = keep; mp.cap = cap;
     mp.n = n; mp.dim = c->dim; mp.w = bp.w; mp.kc = bp.kc; mp.qg = bp.qg; mp.groups = bp.groups; mp.stages = bp.stages; mp.tn = bp.tn;
-    mp.seed_lb = c->d_seedlb; mp.nq_pad = bp.nq_pad;
+    mp.seed_lb = c->d_seedlb; mp.nq_pad = bp.nq_pad; mp.allow = c->cur_allow;
     // L2 prefetch ahead of the shared-memory ring: measured counter-productive (10M x 256, 8 queries: 0.55 ms without, 0.56 /
     // 0.73 / 0.78 ms at 6 / 12 / 24 tiles ahead) -- the small-batch pass is bound by the MMA thread's serial
     // wait -> issue -> commit loop per 128-row tile, not by the stream.  Kept as an experiment knob, off.
@@ -1326,7 +1373,7 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
         memset(&fp, 0, sizeof(fp));
         fp.x = exact_launch(xs);
         fp.bcand = c->d_bcand; fp.bcnt = c->d_bcnt; fp.boverflow = c->d_boverflow; fp.bticket = c->d_tile_counter + 100;
-        fp.bcap = cap; fp.nq = nq; fp.keep = keep; fp.k = k; fp.n = n; fp.dim = c->dim; fp.pitch = pitch;
+        fp.bcap = cap; fp.nq = nq; fp.keep = keep; fp.k = k; fp.n = n; fp.n_allowed = c->cur_allowed; fp.dim = c->dim; fp.pitch = pitch;
         fp.rows = c->d_rows; fp.ids = c->d_ids; fp.qbytes = c->d_qbytes; fp.q16 = c->d_q16; fp.qh = c->d_qh;
         fp.max_dist = max_dist; fp.margin = certificate_margin(c->dim);
         fp.hits = d_hits; fp.count = d_count; fp.status = c->d_status;
@@ -1347,7 +1394,7 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
         const size_t fin_smem = off_stage + stage_bytes;
         FinalizeParams fp;
         memset(&fp, 0, sizeof(fp));
-        fp.grid = (uint32_t)grid_scan; fp.keep = keep; fp.cap = cap_merge; fp.chunk = chunk; fp.k = k; fp.n = n;
+        fp.grid = (uint32_t)grid_scan; fp.keep = keep; fp.cap = cap_merge; fp.chunk = chunk; fp.k = k; fp.n = n; fp.n_allowed = c->cur_allowed;
         fp.dim = c->dim; fp.pitch = pitch; fp.stage_rows = stage_rows; fp.slice16 = slice16;
         fp.off_sorted = (uint32_t)off_sorted; fp.off_ent = 0; fp.off_dots = (uint32_t)off_dots; fp.off_q = (uint32_t)off_q; fp.off_stage = (uint32_t)off_stage;
         fp.rows = c->d_rows; fp.ids = c->d_ids; fp.qbytes = c->d_qbytes; fp.q16 = c->d_q16; fp.qh = c->d_qh;
@@ -1380,15 +1427,76 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
     return PBX_OK;
 }
 
+// A search restricted to a set of image ids (pbx_search_filtered and its twins).
+struct SearchFilter {
+    const int64_t* ids;     // ascending, duplicates allowed: host memory, or device memory if `device`
+    uint64_t n;
+    uint32_t mode;          // PBX_FILTER_INCLUDE / PBX_FILTER_EXCLUDE
+    bool device;            // device ids: their order is checked on the device (PBX_COUNT_FILTER_UNSORTED)
+};
+
+static int check_filter_args(const int64_t* ids, uint64_t n, uint32_t mode) {
+    if (n && !ids) return fail(PBX_E_INVALID, "filter_ids is NULL with n_filter = %llu", (unsigned long long)n);
+    if (mode != PBX_FILTER_INCLUDE && mode != PBX_FILTER_EXCLUDE) return fail(PBX_E_INVALID, "unknown filter mode %u", mode);
+    if (n > PBX_MAX_ROWS) return fail(PBX_E_INVALID, "n_filter = %llu exceeds PBX_MAX_ROWS", (unsigned long long)n);
+    return PBX_OK;
+}
+
+// The filter of a host-form call: the ids sorted and deduplicated into *sorted.  *out = NULL for an empty EXCLUDE set,
+// which is an unfiltered search.
+static int host_filter(const int64_t* ids, uint64_t n, uint32_t mode, std::vector<int64_t>* sorted, SearchFilter* f, const SearchFilter** out) {
+    *out = nullptr;
+    int rc = check_filter_args(ids, n, mode);
+    if (rc != PBX_OK) return rc;
+    if (mode == PBX_FILTER_EXCLUDE && n == 0) return PBX_OK;
+    if (n) { rc = sorted_request(ids, n, sorted); if (rc != PBX_OK) return rc; }
+    f->ids = sorted->data(); f->n = sorted->size(); f->mode = mode; f->device = false;
+    *out = f;
+    return PBX_OK;
+}
+
+// Stream-ordered mark pass of a filtered search over rows [0, n): the row bitmap and the allowed count, both corpus
+// scratch that the next search on any stream only touches after this one (ev_chain).  Caller holds c->mu.
+static int enqueue_filter_mark(pbx_corpus* c, const SearchFilter& f, uint32_t n, cudaStream_t s) {
+    const size_t words = ((size_t)n + kTileRows - 1) / kTileRows * kTileRows / 32;    // every row a kernel may look at
+    int rc = ensure_filter_scratch(c, std::max<size_t>(words, 1), f.device ? 0 : f.n);
+    if (rc != PBX_OK) return rc;
+    const int64_t* d_set = f.ids;
+    if (!f.device && f.n) {
+        CU_TRY(cudaMemcpyAsync(c->d_filter_ids, f.ids, f.n * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        d_set = c->d_filter_ids;
+    }
+    CU_TRY(cudaMemsetAsync(c->d_filter_words, 0, 2 * sizeof(u64), s));
+    if (f.device && f.n > 1) {
+        const unsigned blocks = (unsigned)std::min<uint64_t>((f.n + 255) / 256, (uint64_t)c->sm_count * 8);
+        ids_unsorted_kernel<<<blocks, 256, 0, s>>>(d_set, f.n, reinterpret_cast<uint32_t*>(c->d_filter_words + 1));
+        CU_TRY(cudaGetLastError());
+    }
+    if (n) {
+        mark_ids_kernel<<<(n + kMarkTileRows - 1) / kMarkTileRows, kMarkTileRows, 0, s>>>(c->d_ids, n, d_set, f.n,
+                                                                                       f.mode == PBX_FILTER_EXCLUDE ? 1u : 0u, c->d_allow, c->d_filter_words);
+        CU_TRY(cudaGetLastError());
+    }
+    c->cur_allow = c->d_allow;
+    c->cur_allowed = c->d_filter_words;
+    return PBX_OK;
+}
+
 // Enqueues the whole search for nq queries already on the device.  Caller holds c->mu.
 static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
-                          uint32_t* d_count, cudaStream_t s, bool timed, uint32_t* done_flag = nullptr, uint32_t done_seq = 0) {
+                          uint32_t* d_count, cudaStream_t s, bool timed, uint32_t* done_flag = nullptr, uint32_t done_seq = 0,
+                          const SearchFilter* filter = nullptr) {
     const uint32_t n = (uint32_t)c->n.load();
     c->cur_done_flag = done_flag; c->cur_done_seq = done_seq;    // only the single-query kernels publish to it
+    c->cur_allow = nullptr; c->cur_allowed = nullptr;
     c->last_n = n;
     c->scan_timed = false;
     if (c->chain_valid) CU_TRY(cudaStreamWaitEvent(s, c->ev_chain, 0));
     if (timed) CU_TRY(cudaEventRecord(c->ev_t0, s));
+    if (filter) {
+        int rc = enqueue_filter_mark(c, *filter, n, s);
+        if (rc != PBX_OK) return rc;
+    }
     if (n == 0) {
         empty_result_kernel<<<64, 256, 0, s>>>(d_hits, d_count, nq, k);
         CU_TRY(cudaGetLastError());
@@ -1445,6 +1553,7 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
             sp.hist = c->d_hist;
             sp.status = c->d_status + q;
             sp.max_dist = max_dist;
+            sp.allow = c->cur_allow;
             {
                 PrepSeedParams ps;
                 ps.query = d_queries + (size_t)q * c->dim;
@@ -1455,6 +1564,7 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
                 ps.rows = sp.rows; ps.inv_norm = sp.inv_norm; ps.n = n; ps.keep = keep;
                 ps.do_seed = seeded ? 1u : 0u;
                 ps.seed_hist = c->d_hist + kHistBins; ps.ticket = c->d_tile_counter + 96; ps.gbin = c->d_tile_counter + 32;
+                ps.allow = c->cur_allow;
                 CU_TRY(launch_pdl<PrepSeedParams>(prep_seed_kernel, seeded ? seed_grid : 1, kSeedThreads, (size_t)c->pitch * 2, s, ps));
             }
             const bool time_scan = timed && q + 1 == nq;
@@ -1470,6 +1580,7 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
             fp.cap = cap_merge;
             fp.k = k;
             fp.n = n;
+            fp.n_allowed = c->cur_allowed;
             fp.dim = c->dim;
             fp.pitch = c->pitch;
             fp.rows = c->d_rows;
@@ -1533,6 +1644,12 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
         }
         c->last_grid = grid;
     }
+    if (filter && filter->device) {
+        // after every kernel of the search, tail-launched exact passes included: an unsorted filter voids every count
+        filter_unsorted_count_kernel<<<(nq + 255) / 256, 256, 0, s>>>(reinterpret_cast<const uint32_t*>(c->d_filter_words + 1), d_count, nq,
+                                                                      PBX_COUNT_FILTER_UNSORTED);
+        CU_TRY(cudaGetLastError());
+    }
     if (timed) CU_TRY(cudaEventRecord(c->ev_t1, s));
     CU_TRY(cudaEventRecord(c->ev_chain, s));
     c->chain_valid = true;
@@ -1549,8 +1666,8 @@ static int check_search_args(const pbx_corpus* c, const void* queries, uint32_t 
     return PBX_OK;
 }
 
-extern "C" int pbx_search_device(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
-                                 uint32_t* d_count, void* cuda_stream) {
+static int search_device_impl(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
+                              uint32_t* d_count, void* cuda_stream, const SearchFilter* filter) {
     int rc = check_search_args(c, d_queries, nq, k);
     if (rc != PBX_OK) return rc;
     if (nq == 0) return PBX_OK;
@@ -1560,11 +1677,27 @@ extern "C" int pbx_search_device(pbx_corpus* c, const uint8_t* d_queries, uint32
     std::lock_guard<std::mutex> lk(c->mu);
     CU_TRY(cudaSetDevice(c->device));
     cudaStream_t s = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : c->stream;
-    return enqueue_search(c, d_queries, nq, k, max_dist, d_hits, d_count, s, false);
+    return enqueue_search(c, d_queries, nq, k, max_dist, d_hits, d_count, s, false, nullptr, 0, filter);
 }
 
-extern "C" int pbx_search_hits(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* out_hits,
-                               uint32_t* out_count) {
+extern "C" int pbx_search_device(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
+                                 uint32_t* d_count, void* cuda_stream) {
+    return search_device_impl(c, d_queries, nq, k, max_dist, d_hits, d_count, cuda_stream, nullptr);
+}
+
+extern "C" int pbx_search_device_filtered(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
+                                          uint32_t* d_count, void* cuda_stream, const int64_t* d_filter_ids, uint64_t n_filter,
+                                          uint32_t filter_mode) {
+    int rc = check_filter_args(d_filter_ids, n_filter, filter_mode);
+    if (rc != PBX_OK) return rc;
+    const SearchFilter f = {d_filter_ids, n_filter, filter_mode, true};
+    // an empty EXCLUDE set is the unfiltered search
+    return search_device_impl(c, d_queries, nq, k, max_dist, d_hits, d_count, cuda_stream,
+                              filter_mode == PBX_FILTER_EXCLUDE && n_filter == 0 ? nullptr : &f);
+}
+
+static int search_hits_impl(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* out_hits,
+                            uint32_t* out_count, const SearchFilter* filter) {
     int rc = check_search_args(c, queries, nq, k);
     if (rc != PBX_OK) return rc;
     if (nq == 0) return PBX_OK;
@@ -1616,7 +1749,7 @@ extern "C" int pbx_search_hits(pbx_corpus* c, const uint8_t* queries, uint32_t n
             flag_dev = static_cast<uint32_t*>(df);
             ++c->flag_seq;
         }
-        rc = enqueue_search(c, q_dev, b, k, max_dist, hits_dev, d_cnt, c->stream, c->profiling, flag_dev, c->flag_seq);
+        rc = enqueue_search(c, q_dev, b, k, max_dist, hits_dev, d_cnt, c->stream, c->profiling, flag_dev, c->flag_seq, filter);
         if (rc != PBX_OK) return rc;
         if (polled) {
             // spin on the sequence number; look at the stream now and then so that a faulted kernel cannot hang the caller
@@ -1670,16 +1803,14 @@ extern "C" int pbx_search_hits(pbx_corpus* c, const uint8_t* queries, uint32_t n
     return PBX_OK;
 }
 
-extern "C" int pbx_search(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, int64_t* out_ids,
-                          float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count) {
-    int rc = check_search_args(c, queries, nq, k);
-    if (rc != PBX_OK) return rc;
-    if (nq == 0) return PBX_OK;
-    if (!out_ids || !out_count) return fail(PBX_E_INVALID, "NULL output");
-    std::vector<pbx_hit> hits;
-    try { hits.resize((size_t)nq * k); } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
-    rc = pbx_search_hits(c, queries, nq, k, max_dist, hits.data(), out_count);
-    if (rc != PBX_OK) return rc;
+extern "C" int pbx_search_hits(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* out_hits,
+                               uint32_t* out_count) {
+    return search_hits_impl(c, queries, nq, k, max_dist, out_hits, out_count, nullptr);
+}
+
+// [nq][k] records -> the column outputs of pbx_search (slots past a query's count are zero)
+static void split_hits(const std::vector<pbx_hit>& hits, uint32_t k, const uint32_t* out_count, int64_t* out_ids, float* out_dist,
+                       int32_t* out_dot, int32_t* out_norm2) {
     for (size_t i = 0; i < hits.size(); ++i) {
         const bool valid = (i % k) < out_count[i / k];
         out_ids[i] = valid ? hits[i].image_id : 0;
@@ -1687,7 +1818,36 @@ extern "C" int pbx_search(pbx_corpus* c, const uint8_t* queries, uint32_t nq, ui
         if (out_dot) out_dot[i] = valid ? hits[i].dot : 0;
         if (out_norm2) out_norm2[i] = valid ? hits[i].norm2 : 0;
     }
+}
+
+static int search_impl(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, int64_t* out_ids,
+                       float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count, const SearchFilter* filter) {
+    int rc = check_search_args(c, queries, nq, k);
+    if (rc != PBX_OK) return rc;
+    if (nq == 0) return PBX_OK;
+    if (!out_ids || !out_count) return fail(PBX_E_INVALID, "NULL output");
+    std::vector<pbx_hit> hits;
+    try { hits.resize((size_t)nq * k); } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
+    rc = search_hits_impl(c, queries, nq, k, max_dist, hits.data(), out_count, filter);
+    if (rc != PBX_OK) return rc;
+    split_hits(hits, k, out_count, out_ids, out_dist, out_dot, out_norm2);
     return PBX_OK;
+}
+
+extern "C" int pbx_search(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, int64_t* out_ids,
+                          float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count) {
+    return search_impl(c, queries, nq, k, max_dist, out_ids, out_dist, out_dot, out_norm2, out_count, nullptr);
+}
+
+extern "C" int pbx_search_filtered(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, int64_t* out_ids,
+                                   float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count,
+                                   const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode) {
+    std::vector<int64_t> sorted;
+    SearchFilter f;
+    const SearchFilter* fp = nullptr;
+    int rc = host_filter(filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
+    if (rc != PBX_OK) return rc;
+    return search_impl(c, queries, nq, k, max_dist, out_ids, out_dist, out_dot, out_norm2, out_count, fp);
 }
 
 extern "C" int pbx_merge_hits(const pbx_hit* gathered, const uint32_t* counts, uint32_t n_shards, uint32_t nq, uint32_t k,
@@ -1854,8 +2014,8 @@ extern "C" int pbx_exchange_allgather_merge(pbx_exchange* x, const pbx_hit* d_lo
 // the fused exchange + merge kernel, D2H of the merged result, one synchronisation -- all on the corpus' stream, no
 // other host work in between (the Python driver's torch copies cost ~30 us per query more).  Every rank makes the same
 // call with the same queries; every rank receives the global result.
-extern "C" int pbx_exchange_search_hits(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
-                                        pbx_hit* out_hits, uint32_t* out_count) {
+static int exchange_search_hits_impl(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
+                                     pbx_hit* out_hits, uint32_t* out_count, const SearchFilter* filter) {
     if (!x) return fail(PBX_E_INVALID, "exchange is NULL");
     int rc = check_search_args(c, queries, nq, k);
     if (rc != PBX_OK) return rc;
@@ -1887,7 +2047,7 @@ extern "C" int pbx_exchange_search_hits(pbx_exchange* x, pbx_corpus* c, const ui
     memcpy(c->h_queries, queries, qbytes);
     CU_TRY(cudaMemcpyAsync(c->d_queries, c->h_queries, qbytes, cudaMemcpyHostToDevice, c->stream));
     uint32_t* d_cnt_local = reinterpret_cast<uint32_t*>(c->d_hits + (size_t)nq * k);
-    rc = enqueue_search(c, c->d_queries, nq, k, max_dist, c->d_hits, d_cnt_local, c->stream, false);
+    rc = enqueue_search(c, c->d_queries, nq, k, max_dist, c->d_hits, d_cnt_local, c->stream, false, nullptr, 0, filter);
     if (rc != PBX_OK) return rc;
     // one query: the merge kernel writes the merged records, both counts and a sequence number into pinned memory and this
     // thread polls it (as pbx_search_hits does on one device); otherwise two copies back and a synchronisation
@@ -1938,6 +2098,22 @@ extern "C" int pbx_exchange_search_hits(pbx_exchange* x, pbx_corpus* c, const ui
     memcpy(out_hits, x->h_out, (size_t)nq * k * sizeof(pbx_hit));
     memcpy(out_count, h_cnt, (size_t)nq * sizeof(uint32_t));
     return PBX_OK;
+}
+
+extern "C" int pbx_exchange_search_hits(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
+                                        pbx_hit* out_hits, uint32_t* out_count) {
+    return exchange_search_hits_impl(x, c, queries, nq, k, max_dist, out_hits, out_count, nullptr);
+}
+
+extern "C" int pbx_exchange_search_hits_filtered(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k,
+                                                 double max_dist, pbx_hit* out_hits, uint32_t* out_count, const int64_t* filter_ids,
+                                                 uint64_t n_filter, uint32_t filter_mode) {
+    std::vector<int64_t> sorted;
+    SearchFilter f;
+    const SearchFilter* fp = nullptr;
+    int rc = host_filter(filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
+    if (rc != PBX_OK) return rc;
+    return exchange_search_hits_impl(x, c, queries, nq, k, max_dist, out_hits, out_count, fp);
 }
 
 extern "C" void pbx_exchange_destroy(pbx_exchange* x) {

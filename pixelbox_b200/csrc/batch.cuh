@@ -368,6 +368,8 @@ struct BatchMmaParams {
     const float* inv_q;         // [nq_pad] 1 / |c(q)|  (0 for padding queries)
     float* thr_live;            // == thr, written: thresholds tightened while the pass runs
     float* seed_lb;             // SEED: [sample blocks][nq_pad] lower bounds of the best kappa' of each 32-row block
+    const uint32_t* allow;      // filtered search: bit per row, NULL = every row.  Read from L2 on the seed and survivor
+                                // paths only; the 32-row bound test of the main pass is unchanged (a looser bound is valid)
     uint32_t nq_pad;
     uint32_t keep;
     uint32_t cap;               // candidate buffer entries per query
@@ -794,7 +796,7 @@ batch_mma_kernel(const __grid_constant__ BatchMmaParams p) {
                 const int2 rc = *reinterpret_cast<const int2*>(src + 36);
                 const int sc = src[lane];
                 const uint32_t row = (uint32_t)rc.x + (uint32_t)lane;
-                if (sc >= h.x && row < p.n) {
+                if (sc >= h.x && row < p.n && row_allowed(p.allow, row)) {
                     const uint32_t mi = ms * TN + (uint32_t)rc.y + (uint32_t)lane;
                     const int dot_i = 4 * sc + dterm + 2 * s_mrs[mi] + h.z;
                     const float kf = __fmul_rn((float)dot_i, s_minv[mi]);
@@ -880,13 +882,27 @@ batch_mma_kernel(const __grid_constant__ BatchMmaParams p) {
                         const uint32_t qi = qbase + j;
                         const int ct = s_colterm[j];
                         const size_t blk = (size_t)((i * TN + col0) >> 5);
-                        const float d0 = (float)(4 * mx0 + __float_as_int(bm0.w) + ct);
-                        const float lb0 = d0 >= 0.0f ? __fdiv_rn(d0, bm0.y) : __fdiv_rn(d0, bm0.x);
-                        if (p.seed_lb) p.seed_lb[blk * p.nq_pad + qi] = lb0 - fabsf(lb0) * 4.0e-6f - 1.0e-3f;   // 32 queries per warp: one line
+                        // Filtered search: the bound of a block is that of its best ALLOWED row (the other columns do not
+                        // count), -inf for a block without one.  The block's norm and rowterm range still brackets that
+                        // row, so the bound stays valid, and `keep` finite bounds still stand for `keep` distinct rows.
+                        auto block_lb = [&](const uint32_t* rb, int mx, const float4 bm, const uint32_t row0) {
+                            if (p.allow) {
+                                const uint32_t aw = __ldg(p.allow + (row0 >> 5));       // the 32 rows of the block
+                                if (aw == 0u) return -__int_as_float(0x7f800000);
+                                int m = (int)0x80000000;
+#pragma unroll
+                                for (int c = 0; c < 32; ++c) m = ((aw >> c) & 1u) ? max(m, (int)rb[c]) : m;
+                                mx = m;
+                            }
+                            const float d = (float)(4 * mx + __float_as_int(bm.w) + ct);
+                            const float lb = d >= 0.0f ? __fdiv_rn(d, bm.y) : __fdiv_rn(d, bm.x);
+                            return lb - fabsf(lb) * 4.0e-6f - 1.0e-3f;
+                        };
+                        const float lb0 = block_lb(r, mx0, bm0, t * TN + col0);
+                        if (p.seed_lb) p.seed_lb[blk * p.nq_pad + qi] = lb0;   // 32 queries per warp: one line
                         if constexpr (WIDTH == 64) {                      // (seed_lb is null only in the pipeline-rate experiment)
-                            const float d1 = (float)(4 * mx1 + __float_as_int(bm1.w) + ct);
-                            const float lb1 = d1 >= 0.0f ? __fdiv_rn(d1, bm1.y) : __fdiv_rn(d1, bm1.x);
-                            if (p.seed_lb) p.seed_lb[(blk + 1) * p.nq_pad + qi] = lb1 - fabsf(lb1) * 4.0e-6f - 1.0e-3f;
+                            const float lb1 = block_lb(r + WIDTH - 32, mx1, bm1, t * TN + col0 + 32u);
+                            if (p.seed_lb) p.seed_lb[(blk + 1) * p.nq_pad + qi] = lb1;
                         }
                     } else {
                         const int v0 = bound(t4, cq, bm0);
@@ -1094,6 +1110,7 @@ struct BatchFinalizeParams {
     const uint32_t* boverflow;  // [nq]
     uint32_t* bticket;          // zero on entry and on exit
     uint32_t bcap, nq, keep, k, n, dim, pitch;
+    const u64* n_allowed;       // filtered search: allowed rows among the n (device word), NULL = n
     const uint8_t* rows;
     const int64_t* ids;
     const uint8_t* qbytes;      // [nq][pitch]
@@ -1235,7 +1252,7 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
         p.count[q] = passing < p.k ? passing : p.k;
         SearchStatus st;
         st.n_candidates = nc; st.reserved = 0; st.need_exact = 0; st.theta = 0.0f;
-        if (p.n > nc) {
+        if ((p.n_allowed ? *p.n_allowed : (u64)p.n) > nc) {
             const bool plateau_reachable = p.max_dist > (double)PBX_PLATEAU_DIST && s_nonplateau < p.k;
             const bool separated = (double)s_kappa_last < (double)s_kappa_k - (double)p.margin;
             if (plateau_reachable) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }

@@ -141,6 +141,11 @@ __device__ inline uint32_t hist_threshold_warp(const uint32_t* hist, uint32_t ke
     return m ? __shfl_sync(0xFFFFFFFFu, b, __ffs(m) - 1) : 0u;
 }
 
+// ---- filtered searches: one bit per row (mark_ids_kernel, filter.cuh); NULL = every row is allowed -----------------
+__device__ __forceinline__ bool row_allowed(const uint32_t* allow, uint32_t row) {
+    return allow == nullptr || ((__ldg(allow + (row >> 5)) >> (row & 31u)) & 1u) != 0u;
+}
+
 // ---- candidate keys ----------------------------------------------------------------------
 // fast pass: 64-bit key, larger is better: (ord(kappa) << 32) | ~row  (higher cosine first, then lower row)
 __device__ __forceinline__ u64 make_key64(float kappa, uint32_t row) {

@@ -3,7 +3,8 @@
 // With m rows removed out of n and n' = n - m, the j-th removed row below n' (in row order) receives the j-th surviving
 // row at or above n' (in row order).  Only those rows move, sources (>= n') and destinations (< n') never overlap, and
 // the layout is a pure function of the old layout and the request.  Steps, all on one stream:
-//   remove_mark_kernel    one pass over the ids: a bit per row (binary search in the sorted request), the total m
+//   mark_ids_kernel       one pass over the ids: a bit per row (binary search in the sorted request), the total m
+//                         (filter.cuh, shared with the filtered searches)
 //   remove_count_kernel   per 1024-row tile: holes below n', survivors at or above n'
 //   remove_scan_kernel    exclusive scan of both counts over the tiles (one CTA)
 //   remove_place_kernel   global rank of every hole / source (warp ballots inside the tile): the (hole, source) pairs
@@ -11,31 +12,11 @@
 // followed by block_meta_kernel (batch.cuh) over the blocks below n'.
 #pragma once
 #include "common.cuh"
+#include "filter.cuh"
 
 namespace pbx {
 
-constexpr int kRemoveTileRows = 1024;        // one CTA of 1024 threads, one row per thread
-
-__device__ __forceinline__ bool sorted_contains(const int64_t* __restrict__ set, u64 n_set, int64_t v) {
-    u64 lo = 0, hi = n_set;
-    while (lo < hi) {
-        const u64 mid = (lo + hi) >> 1;
-        if (set[mid] < v) lo = mid + 1;
-        else hi = mid;
-    }
-    return lo < n_set && set[lo] == v;
-}
-
-// flags[w] bit l: row 32 w + l is removed.  *removed += number of removed rows.
-__global__ void __launch_bounds__(kRemoveTileRows) remove_mark_kernel(const int64_t* __restrict__ ids, u64 n, const int64_t* __restrict__ req,
-                                                                      u64 n_req, uint32_t* __restrict__ flags, u64* __restrict__ removed) {
-    const u64 row = (u64)blockIdx.x * kRemoveTileRows + threadIdx.x;
-    const bool gone = row < n && sorted_contains(req, n_req, ids[row]);
-    const uint32_t word = __ballot_sync(0xFFFFFFFFu, gone);
-    if ((threadIdx.x & 31) == 0 && row < n) flags[row >> 5] = word;
-    const int cnt = __syncthreads_count(gone);
-    if (threadIdx.x == 0 && cnt) atomicAdd(removed, (u64)cnt);
-}
+constexpr int kRemoveTileRows = kMarkTileRows;   // one CTA of 1024 threads, one row per thread
 
 // A hole is a removed row below n_keep; a source is a surviving row at or above n_keep.
 __device__ __forceinline__ void remove_roles(const uint32_t* __restrict__ flags, u64 row, u64 n, u64 n_keep, bool* hole, bool* src) {

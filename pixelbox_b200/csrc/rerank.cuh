@@ -56,6 +56,7 @@ struct FinalizeParams {
     uint32_t chunk;             // fallback merge: elements per round, a multiple of kFinalThreads
     uint32_t k;
     uint32_t n;                 // rows searched
+    const u64* n_allowed;       // filtered search: the number of allowed rows among them (device word), NULL = n
     uint32_t dim;
     uint32_t pitch;             // bytes
     uint32_t stage_rows;        // candidates per staging group (<= kFinalThreads: one thread per candidate)
@@ -798,7 +799,8 @@ finalize_kernel(const FinalizeParams p) {
         st.reserved = 0;
         st.need_exact = 0;
         st.theta = 0.0f;
-        if (p.n > nc) {                                   // some rows are not candidates
+        const u64 searchable = p.n_allowed ? *p.n_allowed : (u64)p.n;
+        if (searchable > nc) {                            // some (allowed) rows are not candidates
             const bool plateau_reachable = p.max_dist > (double)PBX_PLATEAU_DIST && s_nonplateau < p.k;
             const bool separated = (double)s_kappa_last < (double)s_kappa_k - (double)p.margin;
             if (plateau_reachable) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }

@@ -53,6 +53,8 @@ struct ScanParams {
     uint32_t* hist;             // [kHistBins] fast pass: kappa histogram of every pushed key (global + merge threshold)
     const SearchStatus* status; // EXACT only
     double max_dist;            // EXACT only
+    const uint32_t* allow;      // filtered search: bit per row (row_allowed), NULL = every row; the fast pass reads it
+                                // only in its FILTER instantiations
 };
 
 // 16 corpus bytes against 16 centred query values: 8 x IDP.2A
@@ -178,12 +180,19 @@ struct ScanShared {
     SelectScratch sel;
 };
 
+constexpr int scan_minb(int pitch16) { return pitch16 >= 16 ? 2 : 4; }
+
 // Fast shapes: pitch16 == L * C, L lanes per row, C chunks per lane.  RAGGED: the same lane layout for any
 // pitch16 <= L * C (row stride taken from the parameters, lane slots beyond the row neither load nor count), so
 // that every row length streams with coalesced 16-byte loads; only the idle slots are lost.
-template <int L, int C, bool EXACT, int MINB = ((L * C >= 16) ? 2 : 4), bool RAGGED = false>
+// FILTER (fast pass only): a row is pushed -- and so counted in the histograms every threshold comes from -- only if
+// its bit in p.allow is set.  The 32 rows of a warp iteration are consecutive: one broadcast word per iteration.  A
+// template flag, so that the unfiltered instantiations are the same code as without filters.  The exact pass tests
+// p.allow at run time, before the replay of a row.
+template <int L, int C, bool EXACT, int MINB = scan_minb(L * C), bool RAGGED = false, bool FILTER = false>
 __global__ void __launch_bounds__(kScanThreads, MINB)
 scan_kernel(const ScanParams p) {
+    static_assert(!(FILTER && EXACT), "the exact pass tests the filter at run time");
     using K = typename std::conditional<EXACT, KeyX, u64>::type;
     constexpr int G = 32 / L;                 // rows handled by one warp-wide load
     constexpr int P16 = L * C;                // row pitch in chunks (compile time for fast shapes)
@@ -279,6 +288,8 @@ scan_kernel(const ScanParams p) {
             for (int it = 0; it < kItersPerChunk; ++it) {
                 const uint32_t row0 = chunk_row0 + (uint32_t)it * kRowsPerWarpIter;
                 const uint32_t my_row = row0 + (uint32_t)(j * G + g);
+                uint32_t allow_word = 0;
+                if constexpr (FILTER) allow_word = __ldg(p.allow + (row0 >> 5));   // rows [row0, row0 + 32), row0 % 32 == 0
                 float gthr = -__int_as_float(0x7f800000);
                 uint32_t gb_new = 0;
                 if constexpr (!EXACT) {
@@ -312,7 +323,8 @@ scan_kernel(const ScanParams p) {
 #ifdef PBX_EXP_NOPUSH
                     if (key == 0x1234567ull) buf[0] = key;
 #else
-                    const bool pass = my_row < p.n && key > tau && kappa_shift(kappa) >= gthr;
+                    bool pass = my_row < p.n && key > tau && kappa_shift(kappa) >= gthr;
+                    if constexpr (FILTER) pass = pass && ((allow_word >> (my_row & 31u)) & 1u);
                     tb.push_warp(pass, key);
                     if (pass) atomicAdd(p.hist + kappa_bin(kappa), 1u);
 #ifdef PBX_EXP_PROFILE
@@ -322,7 +334,7 @@ scan_kernel(const ScanParams p) {
                 } else {
                     bool pass = false;
                     KeyX key = KeyOps<KeyX>::lowest();
-                    if (my_row < p.n && kappa >= theta) {
+                    if (my_row < p.n && kappa >= theta && row_allowed(p.allow, my_row)) {
                         const ReplayOut ro = replay_row<false>(reinterpret_cast<const uint8_t*>(p.rows) + (size_t)my_row * ((size_t)PR * 16),
                                                                p.qbytes, p.q16, p.dim, qh.sum_cq, sh.lut);
                         float dist = ref_distance(qh.sa, ro.sb, ro.dot);
@@ -428,13 +440,13 @@ scan_generic_kernel(const ScanParams p) {
             const float kappa = __fmul_rn(__fmul_rn((float)dot_i, inv_r), qh.inv_q);
             if constexpr (!EXACT) {
                 const u64 key = make_key64(kappa, my_row);
-                const bool pass = my_row < p.n && key > tau;
+                const bool pass = my_row < p.n && key > tau && row_allowed(p.allow, my_row);
                 tb.push_warp(pass, key);
                 if (pass) atomicAdd(p.hist + kappa_bin(kappa), 1u);
             } else {
                 bool pass = false;
                 KeyX key = KeyOps<KeyX>::lowest();
-                if (my_row < p.n && kappa >= theta) {
+                if (my_row < p.n && kappa >= theta && row_allowed(p.allow, my_row)) {
                     const ReplayOut ro = replay_row<false>(reinterpret_cast<const uint8_t*>(p.rows) + (size_t)my_row * ((size_t)p.pitch16 * 16),
                                                            p.qbytes, p.q16, p.dim, qh.sum_cq, sh.lut);
                     float dist = ref_distance(qh.sa, ro.sb, ro.dot);

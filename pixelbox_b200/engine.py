@@ -162,6 +162,34 @@ class Engine:
         self.cached_search_results = results
         sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(results)}\n")
 
+    def query_by_image_hash_within_folder(self, indexed_image: IndexedImage, folder: str) -> None:
+        """query_by_image_hash_from_image restricted to the images under `folder`: the similarity SQL with
+        `AND substr(images.path, 1, length(?)) = ?` added (folder with a trailing separator, so that /a/b does not match
+        /a/bc; no LIKE, whose % and _ occur in real paths).  The folder's ids come from `images`, so a hash without an
+        image row is never among them: one filtered search of k = 100 answers the query, no k-doubling."""
+        if indexed_image.visual_hash is None:
+            sys.stderr.write("TODO: IndexedImage is somehow missing a hash!\n")
+            return
+        self.cached_search_results = None
+        t0 = time.perf_counter()
+        results: List[IndexedImage] = []
+        if self.corpus is not None:
+            prefix = folder if folder.endswith(("/", "\\")) else folder + "/"
+            folder_ids = np.fromiter((r[0] for r in self.read_connection.execute(
+                "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
+            query = np.frombuffer(indexed_image.visual_hash, np.uint8)
+            res = self.corpus.search(query, DEFAULT_MAX_SEARCH_RESULTS, self.max_distance_from_query, within=folder_ids)[0]
+            sql = (f"SELECT {SELECT_FIELDS}, semantic_hashes.hash FROM images "
+                   "JOIN semantic_hashes ON images.id = semantic_hashes.image_id WHERE images.id = ?")
+            for image_id, dist in zip(res.ids, res.dist):
+                row = self.read_connection.execute(sql, (int(image_id),)).fetchone()
+                if row is None:
+                    continue                     # deleted between the id query and the search
+                results.append(IndexedImage(id=row[0], filename=row[1], path=row[2], resolution=(row[3], row[4]),
+                                            thumbnail=row[5], visual_hash=row[6], distance_from_query=float(dist)))
+        self.cached_search_results = results
+        sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(results)}\n")
+
     def get_query_results(self) -> Optional[List[IndexedImage]]:
         return None if self.cached_search_results is None else list(self.cached_search_results)   # :398-400
 
