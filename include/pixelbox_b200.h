@@ -221,6 +221,33 @@ PBX_API int pbx_search_device_filtered(pbx_corpus* c, const uint8_t* d_queries, 
                                        pbx_hit* d_hits, uint32_t* d_count, void* cuda_stream,
                                        const int64_t* d_filter_ids, uint64_t n_filter, uint32_t filter_mode);
 
+/* ---- paged search: the k rows after a (dist, image_id) cursor ----------------------------------------------------------
+ * Replaces: keyset pagination of the similarity query ("show more", or more than PBX_MAX_K rows in all),
+ *   ... FROM semantic_hashes ... WHERE dist < :max_dist AND (dist > :d0 OR (dist = :d0 AND image_id > :id0))
+ *   [AND image_id IN / NOT IN (...)]  ORDER BY dist ASC, image_id ASC LIMIT k
+ *   - Each call takes its twin's arguments plus the cursors and the filter triple of the *_filtered searches
+ *     (n_filter = 0 with PBX_FILTER_EXCLUDE: unfiltered; same argument rules).  Outputs are pbx_hit records.
+ *   - after[q] is query q's cursor: only its image_id (id0) and dist (d0) are read, so the next cursor is the last hit of
+ *     the previous page.  after == NULL: the first page of every query.  {dist = -inf, image_id = INT64_MIN} is also "from
+ *     the start" (no row sorts at or before it); dist = +inf gives count 0.  The cursor need not be a row of the table:
+ *     any (d0, id0) works, an id that was removed or never existed included.
+ *   - A NaN d0: PBX_E_INVALID on the host forms; on the device form that query gets count 0.
+ *   - Contract: exactly the SQL above -- count, ids, order, dist bit for bit, dot, norm2, ties by image_id, and the plateau
+ *     rule applied to the rows after the cursor.  The pages of one iteration concatenate to the first rows of one deep
+ *     top-K for any K, past PBX_MAX_K included, with or without a filter.
+ *   - Pages follow the table at the time of each call (nothing is stored between calls): a row appended between two calls
+ *     shows up on a later page if it sorts after the cursor, and is never seen if it sorts before it.
+ *   - Image ids need not be unique: rows with the same (dist, image_id) are all on the same side of a cursor, as in the SQL.
+ * Cost: one search; a page at depth D adds about D candidate tests per query on the batched path (DESIGN.md section 10). */
+PBX_API int pbx_search_page(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, const pbx_hit* after,
+                            const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode, pbx_hit* out_hits, uint32_t* out_count);
+/* Device-resident form, with the contract of pbx_search_device_filtered.  d_after [nq] (or NULL) is a DEVICE pointer on the
+ * corpus' device, read in stream order on `cuda_stream` with no host read: a pipeline can pass the previous call's d_hits
+ * (the record at slot count - 1 of each query) as the next cursors. */
+PBX_API int pbx_search_device_page(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist,
+                                   const pbx_hit* d_after, const int64_t* d_filter_ids, uint64_t n_filter, uint32_t filter_mode,
+                                   pbx_hit* d_hits, uint32_t* d_count, void* cuda_stream);
+
 /* Merge step after the all-gather (SURVEY.md section 8e): gathered is [n_shards][nq][k] hits and
  * counts is [n_shards][nq], both in HOST memory; every shard list is already ordered by
  * (dist, image_id).  Writes the global first k per query under the same order.  Pure host
@@ -268,6 +295,11 @@ PBX_API int pbx_sharded_search_hits(pbx_sharded* s, const uint8_t* queries, uint
 PBX_API int pbx_sharded_search_filtered(pbx_sharded* s, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
                                         int64_t* out_ids, float* out_dist, int32_t* out_dot, int32_t* out_norm2, uint32_t* out_count,
                                         const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode);
+/* pbx_search_page over all shards: every shard applies the same global cursor; the merge is unchanged (the global next k
+ * rows after a cursor are the first k of the union of every shard's next k rows after it). */
+PBX_API int pbx_sharded_search_page(pbx_sharded* s, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
+                                    const pbx_hit* after, const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode,
+                                    pbx_hit* out_hits, uint32_t* out_count);
 
 /* ---- the exchange step over NVLink peer memory (one process per GPU) ---------------------------------
  * Replaces: nothing upstream (PixelBox is single-process); it is the one exchange step of the row-sharded path
@@ -294,6 +326,10 @@ PBX_API int pbx_exchange_search_hits(pbx_exchange* x, pbx_corpus* c, const uint8
 PBX_API int pbx_exchange_search_hits_filtered(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k,
                                               double max_dist, pbx_hit* out_hits, uint32_t* out_count,
                                               const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode);
+/* The same step for a paged search (pbx_search_page's contract): every rank passes the same cursors and filter. */
+PBX_API int pbx_exchange_search_hits_page(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k,
+                                          double max_dist, const pbx_hit* after, const int64_t* filter_ids, uint64_t n_filter,
+                                          uint32_t filter_mode, pbx_hit* out_hits, uint32_t* out_count);
 PBX_API void pbx_exchange_destroy(pbx_exchange* x);
 
 /* ---- the scalar function, for external users of the DB -----------------------------------

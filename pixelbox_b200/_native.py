@@ -32,6 +32,7 @@ EXPORTS = [
     "pbx_quantize_device", "pbx_corpus_fill_synthetic", "pbx_corpus_remove", "pbx_sharded_remove",
     "pbx_corpus_size", "pbx_corpus_dim", "pbx_corpus_read_rows", "pbx_corpus_synchronize", "pbx_search", "pbx_search_hits", "pbx_search_device",
     "pbx_search_filtered", "pbx_search_device_filtered", "pbx_sharded_search_filtered", "pbx_exchange_search_hits_filtered",
+    "pbx_search_page", "pbx_search_device_page", "pbx_sharded_search_page", "pbx_exchange_search_hits_page",
     "pbx_merge_hits", "pbx_merge_hits_device", "pbx_exchange_create", "pbx_exchange_handle", "pbx_exchange_connect",
     "pbx_exchange_allgather_merge", "pbx_exchange_search_hits", "pbx_exchange_destroy",
     "pbx_sharded_create", "pbx_sharded_destroy", "pbx_sharded_load", "pbx_sharded_append", "pbx_sharded_fill_synthetic", "pbx_sharded_size",
@@ -94,6 +95,8 @@ def lib() -> ctypes.CDLL:
         "pbx_search_device": (i32, [vp, vp, u32, u32, f64, vp, vp, vp]),
         "pbx_search_filtered": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp, vp, u64, u32]),
         "pbx_search_device_filtered": (i32, [vp, vp, u32, u32, f64, vp, vp, vp, vp, u64, u32]),
+        "pbx_search_page": (i32, [vp, u8p, u32, u32, f64, vp, vp, u64, u32, vp, vp]),
+        "pbx_search_device_page": (i32, [vp, vp, u32, u32, f64, vp, vp, u64, u32, vp, vp, vp]),
         "pbx_merge_hits": (i32, [vp, vp, u32, u32, u32, vp, vp]),
         "pbx_merge_hits_device": (i32, [i32, vp, vp, u32, u32, u32, vp, vp, vp]),
         "pbx_exchange_create": (i32, [i32, u32, u32, u32, u32, ctypes.POINTER(vp)]),
@@ -102,6 +105,7 @@ def lib() -> ctypes.CDLL:
         "pbx_exchange_allgather_merge": (i32, [vp, vp, u32, u32, vp, vp, vp]),
         "pbx_exchange_search_hits": (i32, [vp, vp, u8p, u32, u32, f64, vp, vp]),
         "pbx_exchange_search_hits_filtered": (i32, [vp, vp, u8p, u32, u32, f64, vp, vp, vp, u64, u32]),
+        "pbx_exchange_search_hits_page": (i32, [vp, vp, u8p, u32, u32, f64, vp, vp, u64, u32, vp, vp]),
         "pbx_exchange_destroy": (None, [vp]),
         "pbx_sharded_create": (i32, [u32, u64, vp, i32, ctypes.POINTER(vp)]),
         "pbx_sharded_destroy": (None, [vp]),
@@ -114,6 +118,7 @@ def lib() -> ctypes.CDLL:
         "pbx_sharded_search": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp]),
         "pbx_sharded_search_hits": (i32, [vp, u8p, u32, u32, f64, vp, vp]),
         "pbx_sharded_search_filtered": (i32, [vp, u8p, u32, u32, f64, vp, vp, vp, vp, vp, vp, u64, u32]),
+        "pbx_sharded_search_page": (i32, [vp, u8p, u32, u32, f64, vp, vp, u64, u32, vp, vp]),
         "pbx_cosine_distance_pairs": (i32, [i32, u8p, u8p, u64, u32, vp, vp, vp, vp]),
         "pbx_byte_distance_pairs": (i32, [i32, u8p, u8p, u64, u32, vp, vp]),
         "pbx_hamming_distance_pairs": (i32, [i32, u8p, u8p, u64, u32, vp, vp]),
@@ -149,6 +154,36 @@ def filter_args(within, excluding):
     ids = within if within is not None else excluding
     ids = np.ascontiguousarray(np.asarray(ids, dtype=np.int64)).reshape(-1)
     return ids, (PBX_FILTER_INCLUDE if within is not None else PBX_FILTER_EXCLUDE)
+
+
+def page_filter_args(within, excluding):
+    """filter_args for the paged searches, which always take the filter triple: no filter is an empty EXCLUDE set."""
+    if within is None and excluding is None:
+        return np.zeros(0, np.int64), PBX_FILTER_EXCLUDE
+    return filter_args(within, excluding)
+
+
+def page_cursors(after, nq: int) -> np.ndarray:
+    """[nq] pbx_hit cursors of the `after=` keyword of the search methods: one (dist, image_id) per query -- the last
+    row of that query's previous page -- or None for its first page ({-inf, INT64_MIN}: no row sorts at or before it).
+    A HIT_DTYPE array of nq records (e.g. the last hits of a search_hits call) is taken as is."""
+    if isinstance(after, np.ndarray) and after.dtype == HIT_DTYPE:
+        cur = np.ascontiguousarray(after.reshape(-1))
+        if cur.shape != (nq,):
+            raise ValueError(f"after: expected {nq} cursors, got {cur.shape[0]}")
+        return cur
+    after = list(after)
+    if len(after) != nq:
+        raise ValueError(f"after: expected one cursor per query ({nq}), got {len(after)}")
+    cur = np.zeros(nq, HIT_DTYPE)
+    for i, a in enumerate(after):
+        if a is None:
+            cur[i]["dist"], cur[i]["image_id"] = -np.inf, np.iinfo(np.int64).min
+            continue
+        if isinstance(a, (str, bytes)) or not hasattr(a, "__len__") or len(a) != 2:
+            raise ValueError(f"after[{i}]: expected a (dist, image_id) pair or None, got {a!r}")
+        cur[i]["dist"], cur[i]["image_id"] = np.float32(a[0]), int(a[1])
+    return cur
 
 
 def ptr(a) -> ctypes.c_void_p:

@@ -32,6 +32,12 @@ def _as_u8_2d(a, dim: int, what: str) -> np.ndarray:
     return a
 
 
+def _hits_results(hits: np.ndarray, cnt: np.ndarray) -> List[SearchResult]:
+    """[nq][k] pbx_hit records and [nq] counts -> one SearchResult per query."""
+    return [SearchResult(hits[i]["image_id"][:c].copy(), hits[i]["dist"][:c].copy(), hits[i]["dot"][:c].copy(),
+                         hits[i]["norm2"][:c].copy()) for i, c in enumerate(cnt.tolist())]
+
+
 def _remove(fn, handle, image_ids) -> int:
     ids = np.ascontiguousarray(np.asarray(image_ids, dtype=np.int64)).reshape(-1)
     removed = ctypes.c_uint64(0)
@@ -115,16 +121,22 @@ class Corpus:
 
     # -- search ------------------------------------------------------------------------------
     def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None,
-               excluding=None) -> List[SearchResult]:
+               excluding=None, after=None) -> List[SearchResult]:
         """pbx_search: host buffers in, host buffers out; one SearchResult per query.
 
         within / excluding (image ids, any order; at most one of them): pbx_search_filtered, the k nearest rows among
         the rows whose id is listed, or among all rows except those -- exactly what a corpus holding only those rows
         would return.
 
+        after (one (dist, image_id) per query, None for a query's first page): pbx_search_page, the k rows that follow
+        that position in the (dist, image_id) order -- the next page after a page whose last row was (dist, image_id).
+        Combines with within / excluding.
+
         This is the call the latency of a single interactive query goes through, so the wrapper keeps its own cost
         down: output arrays and their raw pointers are cached per thread and (nq, k), the query pointer is taken from
         the array interface (ndarray.ctypes costs ~1 us per use)."""
+        if after is not None:
+            return self._search_page(queries, k, max_dist, after, within, excluding)
         if within is not None or excluding is not None:
             return self._search_filtered(queries, k, max_dist, within, excluding)
         if type(queries) is np.ndarray and queries.dtype == np.uint8 and queries.flags.c_contiguous and (
@@ -165,6 +177,17 @@ class Corpus:
                                                 nat.ptr(n2), nat.ptr(cnt), nat.ptr(fids), fids.size, mode))
         return [SearchResult(ids[i, :c].copy(), dist[i, :c].copy(), dot[i, :c].copy(), n2[i, :c].copy()) for i, c in enumerate(cnt.tolist())]
 
+    def _search_page(self, queries, k, max_dist, after, within, excluding) -> List[SearchResult]:
+        fids, mode = nat.page_filter_args(within, excluding)
+        q = _as_u8_2d(queries, self.dim, "search")
+        nq, k = q.shape[0], int(k)
+        cur = nat.page_cursors(after, nq)
+        hits = np.zeros((nq, k), nat.HIT_DTYPE)
+        cnt = np.zeros(nq, np.uint32)
+        nat.check(nat.lib().pbx_search_page(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(cur), nat.ptr(fids), fids.size, mode,
+                                            nat.ptr(hits), nat.ptr(cnt)))
+        return _hits_results(hits, cnt)
+
     def search_hits(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST) -> Tuple[np.ndarray, np.ndarray]:
         """pbx_search_hits: ([nq][k] pbx_hit records, [nq] counts) -- the per-shard half of a sharded search."""
         q = _as_u8_2d(queries, self.dim, "search_hits")
@@ -202,6 +225,22 @@ class Corpus:
         nat.check(nat.lib().pbx_search_device_filtered(self._h, ctypes.c_void_p(d_queries_ptr), int(nq), int(k), float(max_dist),
                                                        ctypes.c_void_p(d_hits_ptr), ctypes.c_void_p(d_count_ptr), ctypes.c_void_p(stream),
                                                        ctypes.c_void_p(d_filter_ids_ptr), int(n_filter), int(mode)))
+
+    def search_device_page(self, d_queries_ptr: int, nq: int, k: int, max_dist: float, d_hits_ptr: int, d_count_ptr: int,
+                           d_after_ptr: int = 0, d_filter_ids_ptr: int = 0, n_filter: int = 0, mode: int = nat.PBX_FILTER_EXCLUDE,
+                           stream: Optional[int] = None) -> None:
+        """pbx_search_device_page: search_device for the rows after [nq] pbx_hit cursors at d_after_ptr (device memory, read
+        in stream order; 0 = first pages), optionally filtered as in search_device_filtered (n_filter = 0 with
+        PBX_FILTER_EXCLUDE: no filter).  The cursors may be the previous call's records (slot count - 1 of each query):
+        pages chain without a host read.  A NaN cursor dist gives that query count 0."""
+        if stream is None:
+            stream = 0
+        elif stream == 0:
+            stream = 1
+        nat.check(nat.lib().pbx_search_device_page(self._h, ctypes.c_void_p(d_queries_ptr), int(nq), int(k), float(max_dist),
+                                                   ctypes.c_void_p(d_after_ptr), ctypes.c_void_p(d_filter_ids_ptr), int(n_filter),
+                                                   int(mode), ctypes.c_void_p(d_hits_ptr), ctypes.c_void_p(d_count_ptr),
+                                                   ctypes.c_void_p(stream)))
 
     def synchronize(self) -> None:
         """Waits for everything enqueued on the corpus' own stream."""
@@ -296,8 +335,19 @@ class MultiDeviceCorpus:
             nat.check(nat.lib().pbx_set_candidate_slack(h, int(slack)))
 
     def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None,
-               excluding=None) -> List[SearchResult]:
-        """pbx_sharded_search; within / excluding as in Corpus.search (pbx_sharded_search_filtered)."""
+               excluding=None, after=None) -> List[SearchResult]:
+        """pbx_sharded_search; within / excluding and after as in Corpus.search (pbx_sharded_search_filtered,
+        pbx_sharded_search_page)."""
+        if after is not None:
+            fids, mode = nat.page_filter_args(within, excluding)
+            q = _as_u8_2d(queries, self.dim, "search")
+            nq, k = q.shape[0], int(k)
+            cur = nat.page_cursors(after, nq)
+            hits = np.zeros((nq, k), nat.HIT_DTYPE)
+            cnt = np.zeros(nq, np.uint32)
+            nat.check(nat.lib().pbx_sharded_search_page(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(cur), nat.ptr(fids), fids.size,
+                                                        mode, nat.ptr(hits), nat.ptr(cnt)))
+            return _hits_results(hits, cnt)
         filtered = within is not None or excluding is not None
         if filtered:
             fids, mode = nat.filter_args(within, excluding)

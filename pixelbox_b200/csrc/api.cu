@@ -16,6 +16,7 @@
 #include "finalize.cuh"
 #include "batch.cuh"
 #include "remove.cuh"
+#include "page.cuh"
 
 using namespace pbx;
 
@@ -185,6 +186,11 @@ struct pbx_corpus {
     size_t filter_ids_cap = 0;
     const uint32_t* cur_allow = nullptr;  // filter of the search being enqueued (NULL: none); exact_setup picks it up
     const u64* cur_allowed = nullptr;
+    // paged searches (stream-ordered like the rest of the search scratch)
+    PageCut* d_cut = nullptr;         // [cut_cap] cut and cursor per query (page_cut_kernel)
+    pbx_hit* d_after = nullptr;       // [cut_cap] the cursors of a host-form call
+    uint32_t cut_cap = 0;
+    PageCut* cur_cut = nullptr;       // cuts of the search (or batch) being enqueued, one per query (NULL: first pages)
     // pinned staging
     uint8_t* h_queries = nullptr;
     size_t h_queries_cap = 0;
@@ -438,6 +444,19 @@ static int ensure_filter_scratch(pbx_corpus* c, size_t words, uint64_t n_ids) {
     return PBX_OK;
 }
 
+// Cut and cursor of every query of a paged search, and room for the cursors of a host-form call.
+static int ensure_page_scratch(pbx_corpus* c, uint32_t nq) {
+    if (nq <= c->cut_cap) return PBX_OK;
+    // + 1024: the batched kernels address the cuts of a 1024-query chunk by query slot, padding slots included
+    const uint32_t want = std::max<uint32_t>(nq + 1024u, c->cut_cap + c->cut_cap / 2);
+    CU_TRY(cudaDeviceSynchronize());
+    cudaFree(c->d_cut); cudaFree(c->d_after); c->d_cut = nullptr; c->d_after = nullptr; c->cut_cap = 0;
+    CU_TRY(cudaMalloc(&c->d_cut, (size_t)want * sizeof(PageCut)));
+    CU_TRY(cudaMalloc(&c->d_after, (size_t)want * sizeof(pbx_hit)));
+    c->cut_cap = want;
+    return PBX_OK;
+}
+
 // Dynamic shared memory limits are per function and per device, and static shared memory counts
 // against the 48 KB default as well: raise every kernel's cap once, when a corpus is created on a device.
 template <typename Kern>
@@ -599,7 +618,7 @@ extern "C" void pbx_corpus_destroy(pbx_corpus* c) {
     cudaFree(c->d_qpad); cudaFree(c->d_colterm); cudaFree(c->d_thr); cudaFree(c->d_bcnt); cudaFree(c->d_boverflow); cudaFree(c->d_bcand);
     cudaFree(c->d_bhist); cudaFree(c->d_binvq); cudaFree(c->d_seedlb);
     cudaFree(c->d_hits); cudaFree(c->d_cand); cudaFree(c->d_cand_cnt); cudaFree(c->d_tile_counter); cudaFree(c->d_hist);
-    cudaFree(c->d_allow); cudaFree(c->d_filter_words); cudaFree(c->d_filter_ids);
+    cudaFree(c->d_allow); cudaFree(c->d_filter_words); cudaFree(c->d_filter_ids); cudaFree(c->d_cut); cudaFree(c->d_after);
     cudaFreeHost(c->h_queries); cudaFreeHost(c->h_hits); cudaFreeHost(c->h_stage); cudaFreeHost(c->h_flag);
     if (c->ev_chain) cudaEventDestroy(c->ev_chain);
     if (c->ev_t0) cudaEventDestroy(c->ev_t0);
@@ -984,14 +1003,14 @@ static cudaError_t launch_pdl(void (*kern)(const P), int grid, int block, size_t
     return cudaLaunchKernelEx(&cfg, kern, params);
 }
 
-// FILTER: the fast pass of a filtered search (scan_kernel's FILTER instantiations); the exact pass and the generic kernel
-// test p.allow at run time.
-template <bool EXACT, bool FILTER>
+// RESTRICT: the fast pass of a filtered or paged search (scan_kernel's RESTRICT instantiations); the exact pass and the
+// generic kernel test p.allow and p.cut at run time.
+template <bool EXACT, bool RESTRICT>
 static cudaError_t launch_scan_as(const pbx_corpus* c, const ScanParams& p, int grid, size_t smem, cudaStream_t s) {
-    static_assert(!(EXACT && FILTER), "the exact pass has no FILTER instantiation");
+    static_assert(!(EXACT && RESTRICT), "the exact pass has no RESTRICT instantiation");
 #define PBX_SCAN_CASE(LL, CC)                                                                                                     \
     {                                                                                                                             \
-        return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, scan_minb(LL * CC), false, FILTER>, grid, kScanThreads, smem, s, p); \
+        return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, scan_minb(LL * CC), false, RESTRICT>, grid, kScanThreads, smem, s, p); \
     }
     switch (c->pitch16) {
         case 1: PBX_SCAN_CASE(1, 1)
@@ -1000,21 +1019,21 @@ static cudaError_t launch_scan_as(const pbx_corpus* c, const ScanParams& p, int 
         case 8: PBX_SCAN_CASE(8, 1)
         case 16:
             if constexpr (!EXACT) {                  // occupancy variants of the d=256 fast pass (pbx_set_scan_ctas_per_sm)
-                if (c->ctas_per_sm == 3 || c->ctas_per_sm == 0) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 3, false, FILTER>, grid, kScanThreads, smem, s, p);
-                if (c->ctas_per_sm >= 4) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 4, false, FILTER>, grid, kScanThreads, smem, s, p);
+                if (c->ctas_per_sm == 3 || c->ctas_per_sm == 0) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 3, false, RESTRICT>, grid, kScanThreads, smem, s, p);
+                if (c->ctas_per_sm >= 4) return launch_pdl<ScanParams>(scan_kernel<16, 1, false, 4, false, RESTRICT>, grid, kScanThreads, smem, s, p);
             }
             PBX_SCAN_CASE(16, 1)
         case 32: PBX_SCAN_CASE(32, 1)
         case 64: PBX_SCAN_CASE(32, 2)
         case 128: PBX_SCAN_CASE(32, 4)
-#define PBX_SCAN_CASE_M(LL, CC, MM) case (LL) * (CC): return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, MM, false, FILTER>, grid, kScanThreads, smem, s, p);
+#define PBX_SCAN_CASE_M(LL, CC, MM) case (LL) * (CC): return launch_pdl<ScanParams>(scan_kernel<LL, CC, EXACT, MM, false, RESTRICT>, grid, kScanThreads, smem, s, p);
         PBX_EXTRA_SHAPES(PBX_SCAN_CASE_M)
 #undef PBX_SCAN_CASE_M
         default: {
             if constexpr (!EXACT) {
                 // any other row length: the smallest lane layout that holds it, with the row stride at run time
 #define PBX_SCAN_CASE_R(LL, CC, MM) \
-    if (c->pitch16 <= (LL) * (CC)) return launch_pdl<ScanParams>(scan_kernel<LL, CC, false, MM, true, FILTER>, grid, kScanThreads, smem, s, p);
+    if (c->pitch16 <= (LL) * (CC)) return launch_pdl<ScanParams>(scan_kernel<LL, CC, false, MM, true, RESTRICT>, grid, kScanThreads, smem, s, p);
                 PBX_RAGGED_SHAPES(PBX_SCAN_CASE_R)
 #undef PBX_SCAN_CASE_R
             }
@@ -1028,7 +1047,7 @@ static cudaError_t launch_scan_as(const pbx_corpus* c, const ScanParams& p, int 
 template <bool EXACT>
 static cudaError_t launch_scan(const pbx_corpus* c, const ScanParams& p, int grid, size_t smem, cudaStream_t s) {
     if constexpr (!EXACT) {
-        if (p.allow) return launch_scan_as<false, true>(c, p, grid, smem, s);
+        if (p.allow || p.cut) return launch_scan_as<false, true>(c, p, grid, smem, s);
     }
     return launch_scan_as<EXACT, false>(c, p, grid, smem, s);
 }
@@ -1215,6 +1234,14 @@ static bool finalize_stage_layout(size_t avail_bytes, uint32_t keep, uint32_t pi
 // The exact (tie-resolving) pass of one query as a pair of launches: the scan that replays every row with
 // kappa >= theta, and the merge of its per-CTA lists.  Launched from the device by the finalize kernels when a
 // certificate fails; from the host only to repair a refused device-side launch.
+// The f32 bound of the exact pass: the smallest float >= max_dist, so that for every f32 dist, dist < bound exactly
+// when (double)dist < max_dist (NaN stays NaN: nothing passes, as in the f64 comparison).
+static float dist_bound(double max_dist) {
+    float f = (float)max_dist;
+    if ((double)f < max_dist) f = std::nextafter(f, std::numeric_limits<float>::infinity());
+    return f;
+}
+
 struct ExactSetup {
     ScanParams scan;
     FinalizeExactParams fin;
@@ -1233,7 +1260,8 @@ static ExactSetup exact_setup(const pbx_corpus* c, uint32_t q, uint32_t k, doubl
     sp.pitch16 = c->pitch16; sp.dim = c->dim;
     sp.q16 = c->d_q16 + (size_t)q * c->pitch; sp.qbytes = c->d_qbytes + (size_t)q * c->pitch; sp.qh = c->d_qh + q;
     sp.keep = k; sp.cap = cap_scan_x; sp.cand = c->d_cand; sp.cand_cnt = c->d_cand_cnt; sp.tile_counter = c->d_tile_counter;
-    sp.hist = c->d_hist; sp.status = c->d_status + q; sp.max_dist = max_dist; sp.allow = c->cur_allow;
+    sp.hist = c->d_hist; sp.status = c->d_status + q; sp.max_dist = dist_bound(max_dist); sp.allow = c->cur_allow;
+    sp.cut = c->cur_cut ? c->cur_cut + q : nullptr;
     FinalizeExactParams& xp = x.fin;
     xp.cand = reinterpret_cast<const KeyX*>(c->d_cand); xp.cand_cnt = c->d_cand_cnt; xp.grid = (uint32_t)x.grid; xp.k = k;
     xp.cap = cap_merge_x; xp.dim = c->dim; xp.pitch = c->pitch; xp.rows = c->d_rows; xp.qbytes = sp.qbytes;
@@ -1309,7 +1337,7 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
     mp.cand = c->d_bcand; mp.cand_cnt = c->d_bcnt; mp.overflow = c->d_boverflow;
     mp.bhist = c->d_bhist; mp.inv_q = c->d_binvq; mp.thr_live = c->d_thr; mp.keep = keep; mp.cap = cap;
     mp.n = n; mp.dim = c->dim; mp.w = bp.w; mp.kc = bp.kc; mp.qg = bp.qg; mp.groups = bp.groups; mp.stages = bp.stages; mp.tn = bp.tn;
-    mp.seed_lb = c->d_seedlb; mp.nq_pad = bp.nq_pad; mp.allow = c->cur_allow;
+    mp.seed_lb = c->d_seedlb; mp.nq_pad = bp.nq_pad; mp.allow = c->cur_allow; mp.cut = c->cur_cut;
     // L2 prefetch ahead of the shared-memory ring: measured counter-productive (10M x 256, 8 queries: 0.55 ms without, 0.56 /
     // 0.73 / 0.78 ms at 6 / 12 / 24 tiles ahead) -- the small-batch pass is bound by the MMA thread's serial
     // wait -> issue -> commit loop per 128-row tile, not by the stream.  Kept as an experiment knob, off.
@@ -1373,7 +1401,7 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
         memset(&fp, 0, sizeof(fp));
         fp.x = exact_launch(xs);
         fp.bcand = c->d_bcand; fp.bcnt = c->d_bcnt; fp.boverflow = c->d_boverflow; fp.bticket = c->d_tile_counter + 100;
-        fp.bcap = cap; fp.nq = nq; fp.keep = keep; fp.k = k; fp.n = n; fp.n_allowed = c->cur_allowed; fp.dim = c->dim; fp.pitch = pitch;
+        fp.bcap = cap; fp.nq = nq; fp.keep = keep; fp.k = k; fp.n = n; fp.n_allowed = c->cur_allowed; fp.cut = c->cur_cut; fp.dim = c->dim; fp.pitch = pitch;
         fp.rows = c->d_rows; fp.ids = c->d_ids; fp.qbytes = c->d_qbytes; fp.q16 = c->d_q16; fp.qh = c->d_qh;
         fp.max_dist = max_dist; fp.margin = certificate_margin(c->dim);
         fp.hits = d_hits; fp.count = d_count; fp.status = c->d_status;
@@ -1394,7 +1422,7 @@ static int enqueue_search_batched(pbx_corpus* c, const uint8_t* d_queries, uint3
         const size_t fin_smem = off_stage + stage_bytes;
         FinalizeParams fp;
         memset(&fp, 0, sizeof(fp));
-        fp.grid = (uint32_t)grid_scan; fp.keep = keep; fp.cap = cap_merge; fp.chunk = chunk; fp.k = k; fp.n = n; fp.n_allowed = c->cur_allowed;
+        fp.grid = (uint32_t)grid_scan; fp.keep = keep; fp.cap = cap_merge; fp.chunk = chunk; fp.k = k; fp.n = n; fp.n_allowed = c->cur_allowed; fp.cut = c->cur_cut;
         fp.dim = c->dim; fp.pitch = pitch; fp.stage_rows = stage_rows; fp.slice16 = slice16;
         fp.off_sorted = (uint32_t)off_sorted; fp.off_ent = 0; fp.off_dots = (uint32_t)off_dots; fp.off_q = (uint32_t)off_q; fp.off_stage = (uint32_t)off_stage;
         fp.rows = c->d_rows; fp.ids = c->d_ids; fp.qbytes = c->d_qbytes; fp.q16 = c->d_q16; fp.qh = c->d_qh;
@@ -1485,10 +1513,10 @@ static int enqueue_filter_mark(pbx_corpus* c, const SearchFilter& f, uint32_t n,
 // Enqueues the whole search for nq queries already on the device.  Caller holds c->mu.
 static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
                           uint32_t* d_count, cudaStream_t s, bool timed, uint32_t* done_flag = nullptr, uint32_t done_seq = 0,
-                          const SearchFilter* filter = nullptr) {
+                          const SearchFilter* filter = nullptr, const pbx_hit* after = nullptr, bool after_on_device = false) {
     const uint32_t n = (uint32_t)c->n.load();
     c->cur_done_flag = done_flag; c->cur_done_seq = done_seq;    // only the single-query kernels publish to it
-    c->cur_allow = nullptr; c->cur_allowed = nullptr;
+    c->cur_allow = nullptr; c->cur_allowed = nullptr; c->cur_cut = nullptr;
     c->last_n = n;
     c->scan_timed = false;
     if (c->chain_valid) CU_TRY(cudaStreamWaitEvent(s, c->ev_chain, 0));
@@ -1497,12 +1525,26 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
         int rc = enqueue_filter_mark(c, *filter, n, s);
         if (rc != PBX_OK) return rc;
     }
+    PageCut* cuts = nullptr;                                    // paged search: one cut per query, derived on the device
+    if (after) {
+        int rc = ensure_page_scratch(c, nq);
+        if (rc != PBX_OK) return rc;
+        cuts = c->d_cut;
+        const pbx_hit* d_after = after;
+        if (!after_on_device) {                                 // host cursors: a stream-ordered copy into corpus scratch
+            CU_TRY(cudaMemcpyAsync(c->d_after, after, (size_t)nq * sizeof(pbx_hit), cudaMemcpyHostToDevice, s));
+            d_after = c->d_after;
+        }
+        page_cut_kernel<<<(nq + 255) / 256, 256, 0, s>>>(d_after, nq, (double)certificate_margin(c->dim), c->d_cut);
+        CU_TRY(cudaGetLastError());
+    }
     if (n == 0) {
         empty_result_kernel<<<64, 256, 0, s>>>(d_hits, d_count, nq, k);
         CU_TRY(cudaGetLastError());
     } else if (batch_eligible(c, nq, n, k)) {
         for (uint32_t q0 = 0; q0 < nq; q0 += 1024) {
             const uint32_t b = std::min<uint32_t>(1024u, nq - q0);
+            c->cur_cut = cuts ? cuts + q0 : nullptr;
             int rc = enqueue_search_batched(c, d_queries + (size_t)q0 * c->dim, b, k, max_dist, d_hits + (size_t)q0 * k, d_count + q0, s, n);
             if (rc != PBX_OK) return rc;
         }
@@ -1533,6 +1575,7 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
         if (off_stage >= fin_budget || !finalize_stage_layout(fin_budget - off_stage, keep, c->pitch16, &stage_rows, &slice16, &stage_bytes))
             return fail(PBX_E_INTERNAL, "finalize layout does not fit shared memory (k=%u dim=%u)", k, c->dim);
         const size_t fin_smem = off_stage + stage_bytes;
+        c->cur_cut = cuts;                                       // exact_setup offsets it by the query
 
         for (uint32_t q = 0; q < nq; ++q) {
             ScanParams sp;
@@ -1552,8 +1595,9 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
             sp.tile_counter = c->d_tile_counter;
             sp.hist = c->d_hist;
             sp.status = c->d_status + q;
-            sp.max_dist = max_dist;
+            sp.max_dist = dist_bound(max_dist);
             sp.allow = c->cur_allow;
+            sp.cut = cuts ? cuts + q : nullptr;
             {
                 PrepSeedParams ps;
                 ps.query = d_queries + (size_t)q * c->dim;
@@ -1565,6 +1609,7 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
                 ps.do_seed = seeded ? 1u : 0u;
                 ps.seed_hist = c->d_hist + kHistBins; ps.ticket = c->d_tile_counter + 96; ps.gbin = c->d_tile_counter + 32;
                 ps.allow = c->cur_allow;
+                ps.cut = sp.cut;
                 CU_TRY(launch_pdl<PrepSeedParams>(prep_seed_kernel, seeded ? seed_grid : 1, kSeedThreads, (size_t)c->pitch * 2, s, ps));
             }
             const bool time_scan = timed && q + 1 == nq;
@@ -1581,6 +1626,7 @@ static int enqueue_search(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, 
             fp.k = k;
             fp.n = n;
             fp.n_allowed = c->cur_allowed;
+            fp.cut = sp.cut;
             fp.dim = c->dim;
             fp.pitch = c->pitch;
             fp.rows = c->d_rows;
@@ -1666,8 +1712,10 @@ static int check_search_args(const pbx_corpus* c, const void* queries, uint32_t 
     return PBX_OK;
 }
 
+// after: the cursors of a paged search (NULL: first pages), in device memory if after_on_device, else in host memory.
 static int search_device_impl(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
-                              uint32_t* d_count, void* cuda_stream, const SearchFilter* filter) {
+                              uint32_t* d_count, void* cuda_stream, const SearchFilter* filter, const pbx_hit* after = nullptr,
+                              bool after_on_device = false) {
     int rc = check_search_args(c, d_queries, nq, k);
     if (rc != PBX_OK) return rc;
     if (nq == 0) return PBX_OK;
@@ -1677,7 +1725,7 @@ static int search_device_impl(pbx_corpus* c, const uint8_t* d_queries, uint32_t 
     std::lock_guard<std::mutex> lk(c->mu);
     CU_TRY(cudaSetDevice(c->device));
     cudaStream_t s = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : c->stream;
-    return enqueue_search(c, d_queries, nq, k, max_dist, d_hits, d_count, s, false, nullptr, 0, filter);
+    return enqueue_search(c, d_queries, nq, k, max_dist, d_hits, d_count, s, false, nullptr, 0, filter, after, after_on_device);
 }
 
 extern "C" int pbx_search_device(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* d_hits,
@@ -1697,7 +1745,7 @@ extern "C" int pbx_search_device_filtered(pbx_corpus* c, const uint8_t* d_querie
 }
 
 static int search_hits_impl(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, pbx_hit* out_hits,
-                            uint32_t* out_count, const SearchFilter* filter) {
+                            uint32_t* out_count, const SearchFilter* filter, const pbx_hit* after = nullptr) {
     int rc = check_search_args(c, queries, nq, k);
     if (rc != PBX_OK) return rc;
     if (nq == 0) return PBX_OK;
@@ -1749,7 +1797,8 @@ static int search_hits_impl(pbx_corpus* c, const uint8_t* queries, uint32_t nq, 
             flag_dev = static_cast<uint32_t*>(df);
             ++c->flag_seq;
         }
-        rc = enqueue_search(c, q_dev, b, k, max_dist, hits_dev, d_cnt, c->stream, c->profiling, flag_dev, c->flag_seq, filter);
+        rc = enqueue_search(c, q_dev, b, k, max_dist, hits_dev, d_cnt, c->stream, c->profiling, flag_dev, c->flag_seq, filter,
+                            after ? after + q0 : nullptr);
         if (rc != PBX_OK) return rc;
         if (polled) {
             // spin on the sequence number; look at the stream now and then so that a faulted kernel cannot hang the caller
@@ -1848,6 +1897,43 @@ extern "C" int pbx_search_filtered(pbx_corpus* c, const uint8_t* queries, uint32
     int rc = host_filter(filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
     if (rc != PBX_OK) return rc;
     return search_impl(c, queries, nq, k, max_dist, out_ids, out_dist, out_dot, out_norm2, out_count, fp);
+}
+
+// ---- paged searches ------------------------------------------------------------------------------------------------------
+// A NaN dist is no position in the (dist, image_id) order: the host forms reject it (the device form gives count 0).
+static int check_page_args(const pbx_hit* after, uint32_t nq) {
+    if (!after) return PBX_OK;
+    for (uint32_t i = 0; i < nq; ++i)
+        if (std::isnan(after[i].dist)) return fail(PBX_E_INVALID, "after[%u].dist is NaN", i);
+    return PBX_OK;
+}
+
+// The filter and cursor checks shared by the host forms of a paged search.
+static int host_page(const pbx_hit* after, uint32_t nq, const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode,
+                     std::vector<int64_t>* sorted, SearchFilter* f, const SearchFilter** fp) {
+    int rc = host_filter(filter_ids, n_filter, filter_mode, sorted, f, fp);
+    if (rc != PBX_OK) return rc;
+    return check_page_args(after, nq);
+}
+
+extern "C" int pbx_search_page(pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist, const pbx_hit* after,
+                               const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode, pbx_hit* out_hits, uint32_t* out_count) {
+    std::vector<int64_t> sorted;
+    SearchFilter f;
+    const SearchFilter* fp = nullptr;
+    int rc = host_page(after, nq, filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
+    if (rc != PBX_OK) return rc;
+    return search_hits_impl(c, queries, nq, k, max_dist, out_hits, out_count, fp, after);
+}
+
+extern "C" int pbx_search_device_page(pbx_corpus* c, const uint8_t* d_queries, uint32_t nq, uint32_t k, double max_dist,
+                                      const pbx_hit* d_after, const int64_t* d_filter_ids, uint64_t n_filter, uint32_t filter_mode,
+                                      pbx_hit* d_hits, uint32_t* d_count, void* cuda_stream) {
+    int rc = check_filter_args(d_filter_ids, n_filter, filter_mode);
+    if (rc != PBX_OK) return rc;
+    const SearchFilter f = {d_filter_ids, n_filter, filter_mode, true};
+    return search_device_impl(c, d_queries, nq, k, max_dist, d_hits, d_count, cuda_stream,
+                              filter_mode == PBX_FILTER_EXCLUDE && n_filter == 0 ? nullptr : &f, d_after, true);
 }
 
 extern "C" int pbx_merge_hits(const pbx_hit* gathered, const uint32_t* counts, uint32_t n_shards, uint32_t nq, uint32_t k,
@@ -2015,7 +2101,7 @@ extern "C" int pbx_exchange_allgather_merge(pbx_exchange* x, const pbx_hit* d_lo
 // other host work in between (the Python driver's torch copies cost ~30 us per query more).  Every rank makes the same
 // call with the same queries; every rank receives the global result.
 static int exchange_search_hits_impl(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
-                                     pbx_hit* out_hits, uint32_t* out_count, const SearchFilter* filter) {
+                                     pbx_hit* out_hits, uint32_t* out_count, const SearchFilter* filter, const pbx_hit* after = nullptr) {
     if (!x) return fail(PBX_E_INVALID, "exchange is NULL");
     int rc = check_search_args(c, queries, nq, k);
     if (rc != PBX_OK) return rc;
@@ -2047,7 +2133,7 @@ static int exchange_search_hits_impl(pbx_exchange* x, pbx_corpus* c, const uint8
     memcpy(c->h_queries, queries, qbytes);
     CU_TRY(cudaMemcpyAsync(c->d_queries, c->h_queries, qbytes, cudaMemcpyHostToDevice, c->stream));
     uint32_t* d_cnt_local = reinterpret_cast<uint32_t*>(c->d_hits + (size_t)nq * k);
-    rc = enqueue_search(c, c->d_queries, nq, k, max_dist, c->d_hits, d_cnt_local, c->stream, false, nullptr, 0, filter);
+    rc = enqueue_search(c, c->d_queries, nq, k, max_dist, c->d_hits, d_cnt_local, c->stream, false, nullptr, 0, filter, after);
     if (rc != PBX_OK) return rc;
     // one query: the merge kernel writes the merged records, both counts and a sequence number into pinned memory and this
     // thread polls it (as pbx_search_hits does on one device); otherwise two copies back and a synchronisation
@@ -2114,6 +2200,17 @@ extern "C" int pbx_exchange_search_hits_filtered(pbx_exchange* x, pbx_corpus* c,
     int rc = host_filter(filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
     if (rc != PBX_OK) return rc;
     return exchange_search_hits_impl(x, c, queries, nq, k, max_dist, out_hits, out_count, fp);
+}
+
+extern "C" int pbx_exchange_search_hits_page(pbx_exchange* x, pbx_corpus* c, const uint8_t* queries, uint32_t nq, uint32_t k,
+                                             double max_dist, const pbx_hit* after, const int64_t* filter_ids, uint64_t n_filter,
+                                             uint32_t filter_mode, pbx_hit* out_hits, uint32_t* out_count) {
+    std::vector<int64_t> sorted;
+    SearchFilter f;
+    const SearchFilter* fp = nullptr;
+    int rc = host_page(after, nq, filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
+    if (rc != PBX_OK) return rc;
+    return exchange_search_hits_impl(x, c, queries, nq, k, max_dist, out_hits, out_count, fp, after);
 }
 
 extern "C" void pbx_exchange_destroy(pbx_exchange* x) {

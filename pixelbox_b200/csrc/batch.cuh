@@ -370,6 +370,8 @@ struct BatchMmaParams {
     float* seed_lb;             // SEED: [sample blocks][nq_pad] lower bounds of the best kappa' of each 32-row block
     const uint32_t* allow;      // filtered search: bit per row, NULL = every row.  Read from L2 on the seed and survivor
                                 // paths only; the 32-row bound test of the main pass is unchanged (a looser bound is valid)
+    PageCut* cut;               // paged search: [nq] cut and cursor per query, NULL = first pages.  Read on the seed and
+                                // survivor paths only (kappa = kappa' * inv_q, the f32 product the finalize ranks by)
     uint32_t nq_pad;
     uint32_t keep;
     uint32_t cap;               // candidate buffer entries per query
@@ -800,7 +802,10 @@ batch_mma_kernel(const __grid_constant__ BatchMmaParams p) {
                     const uint32_t mi = ms * TN + (uint32_t)rc.y + (uint32_t)lane;
                     const int dot_i = 4 * sc + dterm + 2 * s_mrs[mi] + h.z;
                     const float kf = __fmul_rn((float)dot_i, s_minv[mi]);
-                    if (kf >= __int_as_float(h.y)) {
+                    // paged search: a row above the cut sorts before the cursor; it is counted, never pushed
+                    const bool above = p.cut && __fmul_rn(kf, s_invq[(uint32_t)h.w - qbase]) > p.cut[h.w].kappa_hi;
+                    if (above) atomicAdd(&p.cut[h.w].above, 1u);
+                    else if (kf >= __int_as_float(h.y)) {
                         const u64 key = make_key64(kf, row);
                         const uint32_t slot = atomicAdd(my_cnt, 1u);
                         if (slot < kBatchStage) { my_key[slot] = key; my_q[slot] = (uint32_t)h.w; }
@@ -882,12 +887,22 @@ batch_mma_kernel(const __grid_constant__ BatchMmaParams p) {
                         const uint32_t qi = qbase + j;
                         const int ct = s_colterm[j];
                         const size_t blk = (size_t)((i * TN + col0) >> 5);
-                        // Filtered search: the bound of a block is that of its best ALLOWED row (the other columns do not
-                        // count), -inf for a block without one.  The block's norm and rowterm range still brackets that
-                        // row, so the bound stays valid, and `keep` finite bounds still stand for `keep` distinct rows.
-                        auto block_lb = [&](const uint32_t* rb, int mx, const float4 bm, const uint32_t row0) {
-                            if (p.allow) {
-                                const uint32_t aw = __ldg(p.allow + (row0 >> 5));       // the 32 rows of the block
+                        // Filtered or paged search: the bound of a block is that of its best ALLOWED row at or below the
+                        // query's cut (the other columns do not count), -inf for a block without one.  The block's norm
+                        // and rowterm range still brackets that row, so the bound stays valid, and `keep` finite bounds
+                        // still stand for `keep` distinct searchable rows.
+                        auto block_lb = [&](const uint32_t* rb, int mx, const float4 bm, const uint32_t row0, const uint32_t c0) {
+                            if (p.allow || p.cut) {
+                                uint32_t aw = p.allow ? __ldg(p.allow + (row0 >> 5)) : ~0u;       // the 32 rows of the block
+                                if (p.cut && s_invq[j] > 0.0f) {               // (padding queries have no cut)
+                                    const float hi = p.cut[qi].kappa_hi, iq = s_invq[j];
+#pragma unroll
+                                    for (int c = 0; c < 32; ++c) {
+                                        const uint32_t mi = ms * TN + c0 + (uint32_t)c;
+                                        const float kf = __fmul_rn((float)(4 * (int)rb[c] + dterm + 2 * s_mrs[mi] + ct), s_minv[mi]);
+                                        if (__fmul_rn(kf, iq) > hi) aw &= ~(1u << c);
+                                    }
+                                }
                                 if (aw == 0u) return -__int_as_float(0x7f800000);
                                 int m = (int)0x80000000;
 #pragma unroll
@@ -898,10 +913,10 @@ batch_mma_kernel(const __grid_constant__ BatchMmaParams p) {
                             const float lb = d >= 0.0f ? __fdiv_rn(d, bm.y) : __fdiv_rn(d, bm.x);
                             return lb - fabsf(lb) * 4.0e-6f - 1.0e-3f;
                         };
-                        const float lb0 = block_lb(r, mx0, bm0, t * TN + col0);
+                        const float lb0 = block_lb(r, mx0, bm0, t * TN + col0, col0);
                         if (p.seed_lb) p.seed_lb[blk * p.nq_pad + qi] = lb0;   // 32 queries per warp: one line
                         if constexpr (WIDTH == 64) {                      // (seed_lb is null only in the pipeline-rate experiment)
-                            const float lb1 = block_lb(r + WIDTH - 32, mx1, bm1, t * TN + col0 + 32u);
+                            const float lb1 = block_lb(r + WIDTH - 32, mx1, bm1, t * TN + col0 + 32u, col0 + 32u);
                             if (p.seed_lb) p.seed_lb[(blk + 1) * p.nq_pad + qi] = lb1;
                         }
                     } else {
@@ -1111,6 +1126,7 @@ struct BatchFinalizeParams {
     uint32_t* bticket;          // zero on entry and on exit
     uint32_t bcap, nq, keep, k, n, dim, pitch;
     const u64* n_allowed;       // filtered search: allowed rows among the n (device word), NULL = n
+    const PageCut* cut;         // paged search: [nq] cut and cursor per query, NULL = first pages
     const uint8_t* rows;
     const int64_t* ids;
     const uint8_t* qbytes;      // [nq][pitch]
@@ -1136,8 +1152,9 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
     __shared__ uint32_t s_od[kBfThreads];
     __shared__ long long s_id[kBfThreads];
     __shared__ float s_kappa_k, s_kappa_last;
-    __shared__ uint32_t s_pass, s_nonplateau;
+    __shared__ uint32_t s_pass, s_nonplateau, s_excl;
     const uint32_t tid = threadIdx.x, lane = tid & 31u, q = blockIdx.x;
+    const PageCut* cut_q = p.cut ? p.cut + q : nullptr;
     const uint32_t c = min(min(p.bcnt[q], p.bcap), blockDim.x);          // <= keep after the last batch_tighten
     const QueryHeader qh = p.qh[q];
     for (uint32_t i = tid; i < 256u * 32u; i += blockDim.x) s_lut[i] = ref_decode(i >> 5);
@@ -1151,7 +1168,7 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
         key = make_key64(__fmul_rn(key64_kappa(e), qh.inv_q), key64_row(e));
     }
     s_key[tid] = key;
-    if (tid == 0) { s_kappa_k = 0.0f; s_kappa_last = 0.0f; s_pass = 0; s_nonplateau = 0; }
+    if (tid == 0) { s_kappa_k = 0.0f; s_kappa_last = 0.0f; s_pass = 0; s_nonplateau = 0; s_excl = 0; }
     __syncthreads();
     // candidate order by (kappa desc, row asc): what the certificate's two kappas are read from
     const uint32_t nc = min(c, p.keep);
@@ -1168,7 +1185,7 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
     float dist = __int_as_float(0x7f800000);
     int idot = 0, inorm = 0;
     long long id = INT64_MAX;
-    const bool have = tid < c && key != 0ull;
+    bool have = tid < c && key != 0ull;
     if (have) {
         const uint32_t row = key64_row(key);
         const uint4* r4 = reinterpret_cast<const uint4*>(p.rows + (size_t)row * p.pitch);
@@ -1214,6 +1231,13 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
         idot = 2 * acc - 255 * qh.sum_cq;
         inorm = (int)(4u * s2 - 1020u * s1 + 65025u * p.dim);
         id = p.ids[row];
+        if (page_before(cut_q, dist, id)) {
+            // paged search: not on the page.  Taken out of the ranking (with its real dist it would sort first) and out
+            // of the surviving candidates the certificate counts
+            have = false;
+            id = INT64_MAX;
+            atomicAdd(&s_excl, 1u);
+        }
     }
     const uint32_t od = have ? ord_f32(dist) : 0xFFFFFFFFu;
     s_od[tid] = od;
@@ -1241,9 +1265,21 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
             hits_g[pos] = hh;
         }
     }
-    for (uint32_t i = nc + tid; i < p.k; i += blockDim.x) {
+    for (uint32_t i = nc - s_excl + tid; i < p.k; i += blockDim.x) {
         pbx_hit hh; hh.image_id = INT64_MAX; hh.dist = __int_as_float(0x7f800000); hh.dot = 0; hh.norm2 = 0; hh.flags = 0;
         hits_g[i] = hh;
+    }
+    if (s_excl) {
+        // the certificate's kappa_k is that of the k-th best SURVIVING candidate (by kappa)
+        __syncthreads();
+        s_key[tid] = have ? key : 0ull;
+        if (tid == 0) s_kappa_k = 0.0f;
+        __syncthreads();
+        if (have) {
+            uint32_t rank = 0;
+            for (uint32_t j = 0; j < c; ++j) rank += (s_key[j] > key) ? 1u : 0u;
+            if (p.k > 0 && rank == p.k - 1) s_kappa_k = key64_kappa(key);
+        }
     }
     __syncthreads();
     // certificate (DESIGN.md section 5), as in finalize_kernel
@@ -1252,10 +1288,13 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
         p.count[q] = passing < p.k ? passing : p.k;
         SearchStatus st;
         st.n_candidates = nc; st.reserved = 0; st.need_exact = 0; st.theta = 0.0f;
-        if ((p.n_allowed ? *p.n_allowed : (u64)p.n) > nc) {
+        u64 searchable = p.n_allowed ? *p.n_allowed : (u64)p.n;
+        if (cut_q) searchable -= min(searchable, (u64)cut_q->above);     // paged search: rows at or below the cut
+        if (searchable > nc) {
             const bool plateau_reachable = p.max_dist > (double)PBX_PLATEAU_DIST && s_nonplateau < p.k;
             const bool separated = (double)s_kappa_last < (double)s_kappa_k - (double)p.margin;
-            if (plateau_reachable) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }
+            const bool short_page = cut_q != nullptr && nc - s_excl < p.k;     // no k-th surviving candidate to bound with
+            if (plateau_reachable || short_page) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }
             else if (!separated) { st.need_exact = 1; st.theta = (float)((double)s_kappa_k - (double)p.margin - 1e-7); }
         }
         if (p.boverflow[q] || p.bcnt[q] > blockDim.x) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }   // candidates were dropped
@@ -1279,6 +1318,7 @@ batch_finalize_kernel(const BatchFinalizeParams p) {
                 x.scan.qbytes += (size_t)qq * p.pitch;
                 x.scan.qh += qq;
                 x.scan.status += qq;
+                if (x.scan.cut) x.scan.cut += qq;
                 x.fin.qbytes += (size_t)qq * p.pitch;
                 x.fin.hits += (size_t)qq * p.k;
                 x.fin.count += qq;

@@ -146,6 +146,22 @@ __device__ __forceinline__ bool row_allowed(const uint32_t* allow, uint32_t row)
     return allow == nullptr || ((__ldg(allow + (row >> 5)) >> (row & 31u)) & 1u) != 0u;
 }
 
+// ---- paged searches: the rows after a (dist, image_id) cursor (page.cuh derives one PageCut per query) -------------
+// A row with kappa > kappa_hi sorts strictly before the cursor (DESIGN.md section 5): it is never pushed, sampled or
+// replayed.  A row at or below the cut may still sort at or before the cursor; the replay decides (page_before).
+struct PageCut {
+    int64_t id0;                // cursor image_id
+    float d0;                   // cursor dist
+    float kappa_hi;             // +inf: no row is above the cut; -inf: every row is (the page is empty)
+    uint32_t above;             // allowed rows the fast pass skipped for kappa > kappa_hi (an undercount is safe)
+    uint32_t pad;
+};
+__device__ __forceinline__ float page_kappa_hi(const PageCut* cut) { return cut ? cut->kappa_hi : __int_as_float(0x7f800000); }
+// (dist, id) <= (d0, id0): the row sorts at or before the cursor and is not on the page
+__device__ __forceinline__ bool page_before(const PageCut* cut, float dist, int64_t id) {
+    return cut != nullptr && (dist < cut->d0 || (dist == cut->d0 && id <= cut->id0));
+}
+
 // ---- candidate keys ----------------------------------------------------------------------
 // fast pass: 64-bit key, larger is better: (ord(kappa) << 32) | ~row  (higher cosine first, then lower row)
 __device__ __forceinline__ u64 make_key64(float kappa, uint32_t row) {

@@ -35,6 +35,7 @@ struct PrepSeedParams {
     uint32_t* gbin;             // out: the scan's global bin threshold
     const uint32_t* allow;      // filtered search: only allowed sampled rows are counted (NULL = all).  With fewer than
                                 // `keep` of them hist_threshold_warp gives 0: no starting threshold, which is valid
+    const PageCut* cut;         // paged search: only sampled rows at or below the cut are counted (NULL = all)
 };
 
 __global__ void __launch_bounds__(kSeedThreads)
@@ -109,7 +110,7 @@ prep_seed_kernel(const PrepSeedParams p) {
         }
         const int dot_i = 2 * a - 255 * qh.sum_cq;
         const float kappa = __fmul_rn(__fmul_rn((float)dot_i, __ldg(p.inv_norm + row)), qh.inv_q);
-        if (row_allowed(p.allow, row)) atomicAdd(p.seed_hist + kappa_bin(kappa), 1u);
+        if (row_allowed(p.allow, row) && kappa <= page_kappa_hi(p.cut)) atomicAdd(p.seed_hist + kappa_bin(kappa), 1u);
     }
     __threadfence();
     __syncthreads();

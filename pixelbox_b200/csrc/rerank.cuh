@@ -57,6 +57,7 @@ struct FinalizeParams {
     uint32_t k;
     uint32_t n;                 // rows searched
     const u64* n_allowed;       // filtered search: the number of allowed rows among them (device word), NULL = n
+    const PageCut* cut;         // paged search: the cut and cursor of this query (batched: of query 0), NULL = first page
     uint32_t dim;
     uint32_t pitch;             // bytes
     uint32_t stage_rows;        // candidates per staging group (<= kFinalThreads: one thread per candidate)
@@ -419,7 +420,7 @@ finalize_kernel(const FinalizeParams p) {
     int16_t* s_q16 = reinterpret_cast<int16_t*>(smem_raw + p.off_q + 4 * p.pitch); // [pitch] centred query
     unsigned char* stage = smem_raw + p.off_stage;                                 // [stage_rows][slice16 * 16 + 16]
 
-    __shared__ uint32_t s_cnt, s_pushed, s_maxcnt, s_nonplateau, s_bstar, s_mprime, s_total, s_odlo, s_odhi;
+    __shared__ uint32_t s_cnt, s_pushed, s_maxcnt, s_nonplateau, s_bstar, s_mprime, s_total, s_odlo, s_odhi, s_excl, s_scnt;
     __shared__ u64 s_tau;
     __shared__ float s_lut[256];
     __shared__ float s_kappa_k, s_kappa_last, s_sa;
@@ -435,11 +436,12 @@ finalize_kernel(const FinalizeParams p) {
     pbx_hit* hits_g = p.hits + (size_t)q * p.k;
     uint32_t* count_g = p.count + q;
     SearchStatus* status_g = p.status + q;
+    const PageCut* cut_g = p.cut ? p.cut + q : nullptr;
     __shared__ SelectScratch s_sel;
     // No pdl_trigger() here: this grid may tail-launch the exact pass, which must run before anything else in
     // the stream; a next-query kernel that was already started early would wait for it while it waits for them.
     if (tid < 256) s_lut[tid] = ref_decode(tid);
-    if (tid == 0) { s_cnt = 0; s_tau = 0ull; s_maxcnt = 0; s_nonplateau = 0; s_pushed = 0; s_bstar = 0; s_mprime = 0; s_odlo = 0xFFFFFFFFu; s_odhi = 0u; }
+    if (tid == 0) { s_cnt = 0; s_tau = 0ull; s_maxcnt = 0; s_nonplateau = 0; s_pushed = 0; s_bstar = 0; s_mprime = 0; s_odlo = 0xFFFFFFFFu; s_odhi = 0u; s_excl = 0; s_scnt = 0; }
     pdl_wait();                 // the scan is complete: lists, histogram and the query scratch are visible
     for (uint32_t i = tid; i < p.pitch / 8; i += blockDim.x)
         reinterpret_cast<uint4*>(s_q16)[i] = __ldg(reinterpret_cast<const uint4*>(q16_g) + i);
@@ -650,28 +652,45 @@ finalize_kernel(const FinalizeParams p) {
     const float sa = s_sa;
     const uint32_t n2 = next_pow2(nc < 2 ? 2 : nc);
     uint32_t nonplateau = 0;
-    // ent overlays buf/sorted: fetch the image ids through `sorted` first, write ent after a barrier
+    // ent overlays buf/sorted: fetch the image ids (and the keys, for a paged search) through `sorted` first, write ent
+    // after a barrier
     int64_t my_id[kMaxKeep / kFinalThreads];
+    u64 my_key[kMaxKeep / kFinalThreads];
+    uint32_t my_excl = 0;                                   // bit x: candidate tid + x * kFinalThreads sorts at or before the cursor
 #pragma unroll
     for (uint32_t x = 0; x < kMaxKeep / kFinalThreads; ++x) {
         const uint32_t c = tid + x * kFinalThreads;
-        my_id[x] = (c < nc) ? p.ids[key64_row(sorted[c])] : INT64_MAX;
+        my_key[x] = (c < nc) ? sorted[c] : 0ull;
+        my_id[x] = (c < nc) ? p.ids[key64_row(my_key[x])] : INT64_MAX;
     }
     __syncthreads();
+    uint32_t excl = 0;
 #pragma unroll
     for (uint32_t x = 0; x < kMaxKeep / kFinalThreads; ++x) {
         const uint32_t c = tid + x * kFinalThreads;
         if (c < nc) {
             const float dist = ref_distance(sa, sbs[c], fdots[c]);
-            dists[c] = dist;
             RerankEntry e;
-            e.od = ord_f32(dist);
             e.slot = c;
-            e.id = my_id[x];
+            if (page_before(cut_g, dist, my_id[x])) {
+                // Paged search: not on the page.  It is taken out of the ranking -- it sorts after every real row, never
+                // passes, and is not a surviving candidate for the certificate -- rather than only marked: with its
+                // real dist it would sort first.
+                dists[c] = __int_as_float(0x7fffffff);         // NaN: never < max_dist
+                e.od = 0xFFFFFFFFu;
+                e.id = INT64_MAX;
+                my_excl |= 1u << x;
+                ++excl;
+            } else {
+                dists[c] = dist;
+                e.od = ord_f32(dist);
+                e.id = my_id[x];
+                if (dist < PBX_PLATEAU_DIST) nonplateau++;
+            }
             ent[c] = e;
-            if (dist < PBX_PLATEAU_DIST) nonplateau++;
         }
     }
+    if (excl) atomicAdd(&s_excl, excl);
     for (uint32_t c = nc + tid; c < n2; c += blockDim.x) {
         RerankEntry e; e.od = 0xFFFFFFFFu; e.slot = 0xFFFFFFFFu; e.id = INT64_MAX;
         ent[c] = e;
@@ -788,6 +807,27 @@ finalize_kernel(const FinalizeParams p) {
     }
     if (local) atomicAdd(&s_cnt, local);
     __syncthreads();
+    if (s_excl) {
+        // Paged search with candidates at or before the cursor: the certificate's kappa_k is that of the k-th best
+        // SURVIVING candidate (by kappa).  buf is free again (ent is dead); the keys come back from the registers.
+#pragma unroll
+        for (uint32_t x = 0; x < kMaxKeep / kFinalThreads; ++x) {
+            const uint32_t c = tid + x * kFinalThreads;
+            if (c < nc && !((my_excl >> x) & 1u)) buf[atomicAdd(&s_scnt, 1u)] = my_key[x];
+        }
+        __syncthreads();
+        const uint32_t ns = s_scnt;                            // nc - s_excl
+        if (ns >= p.k) {
+            if (ns > p.k) {
+                TopBuf<u64> tk{buf, &s_scnt, &s_tau, p.cap, p.k};
+                block_select_top(tk, &s_sel);
+            }
+            __shared__ u64 s_kmin;
+            block_min_key(buf, p.k, &s_kmin, s_scratch64);
+            if (tid == 0) s_kappa_k = key64_kappa(s_kmin);
+        }
+        __syncthreads();
+    }
 
     PBX_FIN_STAMP(8);
     // ---- certificate (DESIGN.md section 5) ------------------------------------------------------------------
@@ -799,11 +839,14 @@ finalize_kernel(const FinalizeParams p) {
         st.reserved = 0;
         st.need_exact = 0;
         st.theta = 0.0f;
-        const u64 searchable = p.n_allowed ? *p.n_allowed : (u64)p.n;
-        if (searchable > nc) {                            // some (allowed) rows are not candidates
+        u64 searchable = p.n_allowed ? *p.n_allowed : (u64)p.n;
+        // paged search: allowed rows at or below the cut (every row above it sorts before the cursor)
+        if (cut_g) searchable -= min(searchable, (u64)*reinterpret_cast<const volatile uint32_t*>(&cut_g->above));
+        if (searchable > nc) {                            // some (allowed, searchable) rows are not candidates
             const bool plateau_reachable = p.max_dist > (double)PBX_PLATEAU_DIST && s_nonplateau < p.k;
             const bool separated = (double)s_kappa_last < (double)s_kappa_k - (double)p.margin;
-            if (plateau_reachable) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }
+            const bool short_page = cut_g != nullptr && nc - s_excl < p.k;     // no k-th surviving candidate to bound with
+            if (plateau_reachable || short_page) { st.need_exact = 1; st.theta = -__int_as_float(0x7f800000); }
             else if (!separated) { st.need_exact = 1; st.theta = (float)((double)s_kappa_k - (double)p.margin - 1e-7); }
         }
         if constexpr (BATCH) {
@@ -839,6 +882,7 @@ finalize_kernel(const FinalizeParams p) {
                     x.scan.qbytes += (size_t)qq * p.pitch;
                     x.scan.qh += qq;
                     x.scan.status += qq;
+                    if (x.scan.cut) x.scan.cut += qq;
                     x.fin.qbytes += (size_t)qq * p.pitch;
                     x.fin.hits += (size_t)qq * p.k;
                     x.fin.count += qq;

@@ -42,6 +42,7 @@ struct ScanParams {
     uint32_t n;                 // committed rows visible to this search
     uint32_t pitch16;           // row pitch in 16-byte chunks
     uint32_t dim;
+    float max_dist;             // EXACT only: the smallest f32 >= the caller's f64 max_dist (dist < it <=> dist < max_dist)
     const int16_t* q16;         // [pitch] centred query, zero in the padding
     const uint8_t* qbytes;      // [pitch] raw query bytes
     const QueryHeader* qh;
@@ -52,10 +53,14 @@ struct ScanParams {
     uint32_t* tile_counter;     // dynamic tile scheduler (reset by the finalize kernel)
     uint32_t* hist;             // [kHistBins] fast pass: kappa histogram of every pushed key (global + merge threshold)
     const SearchStatus* status; // EXACT only
-    double max_dist;            // EXACT only
+    PageCut* cut;               // paged search: this query's cut and cursor (page.cuh), NULL = first page; the fast pass
+                                // reads it only in its RESTRICT instantiations and adds the rows above the cut to cut->above
     const uint32_t* allow;      // filtered search: bit per row (row_allowed), NULL = every row; the fast pass reads it
-                                // only in its FILTER instantiations
+                                // only in its RESTRICT instantiations
 };
+// 128 bytes, and every field the unrestricted fast pass reads at the offset it had before paged searches: a larger
+// parameter block changes how the compiler reads it (and the fast pass's code)
+static_assert(sizeof(ScanParams) == 128, "ScanParams layout");
 
 // 16 corpus bytes against 16 centred query values: 8 x IDP.2A
 __device__ __forceinline__ int dot16(const uint4& v, const int* q, int acc) {
@@ -185,14 +190,17 @@ constexpr int scan_minb(int pitch16) { return pitch16 >= 16 ? 2 : 4; }
 // Fast shapes: pitch16 == L * C, L lanes per row, C chunks per lane.  RAGGED: the same lane layout for any
 // pitch16 <= L * C (row stride taken from the parameters, lane slots beyond the row neither load nor count), so
 // that every row length streams with coalesced 16-byte loads; only the idle slots are lost.
-// FILTER (fast pass only): a row is pushed -- and so counted in the histograms every threshold comes from -- only if
-// its bit in p.allow is set.  The 32 rows of a warp iteration are consecutive: one broadcast word per iteration.  A
-// template flag, so that the unfiltered instantiations are the same code as without filters.  The exact pass tests
-// p.allow at run time, before the replay of a row.
-template <int L, int C, bool EXACT, int MINB = scan_minb(L * C), bool RAGGED = false, bool FILTER = false>
+// RESTRICT (fast pass only): a filtered and/or paged search.  A row is pushed -- and so counted in the histograms every
+// threshold comes from -- only if its bit in p.allow is set (when there is a filter) and its kappa is at most the cut
+// (when there is a cursor).  The 32 rows of a warp iteration are consecutive: one broadcast bitmap word per iteration.
+// Allowed rows above the cut are counted (one ballot per warp iteration, one atomic per chunk) for the certificate's
+// trivially-exact case.  A template flag, so that the unrestricted instantiations are the same code as before.  The
+// exact pass tests p.allow and the cut at run time, before the replay of a row, and drops the rows at or before the
+// cursor after it.
+template <int L, int C, bool EXACT, int MINB = scan_minb(L * C), bool RAGGED = false, bool RESTRICT = false>
 __global__ void __launch_bounds__(kScanThreads, MINB)
 scan_kernel(const ScanParams p) {
-    static_assert(!(FILTER && EXACT), "the exact pass tests the filter at run time");
+    static_assert(!(RESTRICT && EXACT), "the exact pass tests the filter and the cut at run time");
     using K = typename std::conditional<EXACT, KeyX, u64>::type;
     constexpr int G = 32 / L;                 // rows handled by one warp-wide load
     constexpr int P16 = L * C;                // row pitch in chunks (compile time for fast shapes)
@@ -231,6 +239,8 @@ scan_kernel(const ScanParams p) {
     const int bias = -255 * qh.sum_cq;
     float theta = 0.0f;
     if constexpr (EXACT) theta = p.status->theta;
+    float cut = __int_as_float(0x7f800000);
+    if constexpr (EXACT || RESTRICT) cut = page_kappa_hi(p.cut);
 
     uint32_t* const gbin = p.tile_counter + 32;        // its own 128-byte line, away from the chunk counter
     // sh.gb starts at the global bin threshold seeded by prep_seed_kernel from a strided sample of the shard (fast pass)
@@ -278,6 +288,7 @@ scan_kernel(const ScanParams p) {
             const uint32_t chunk_row0 = cur * kChunkRows;
             ++cur;
             uint32_t gpoll = 0;
+            uint32_t n_above = 0;                       // RESTRICT: allowed rows of this chunk above the cut
             if constexpr (!EXACT) {
                 // warp 0 polls the global word once per chunk (consumed at the end of the chunk, so the L2 round
                 // trip is hidden) and republishes it in shared memory for its siblings
@@ -288,8 +299,10 @@ scan_kernel(const ScanParams p) {
             for (int it = 0; it < kItersPerChunk; ++it) {
                 const uint32_t row0 = chunk_row0 + (uint32_t)it * kRowsPerWarpIter;
                 const uint32_t my_row = row0 + (uint32_t)(j * G + g);
-                uint32_t allow_word = 0;
-                if constexpr (FILTER) allow_word = __ldg(p.allow + (row0 >> 5));   // rows [row0, row0 + 32), row0 % 32 == 0
+                uint32_t allow_word = ~0u;
+                if constexpr (RESTRICT) {
+                    if (p.allow) allow_word = __ldg(p.allow + (row0 >> 5));   // rows [row0, row0 + 32), row0 % 32 == 0
+                }
                 float gthr = -__int_as_float(0x7f800000);
                 uint32_t gb_new = 0;
                 if constexpr (!EXACT) {
@@ -324,7 +337,11 @@ scan_kernel(const ScanParams p) {
                     if (key == 0x1234567ull) buf[0] = key;
 #else
                     bool pass = my_row < p.n && key > tau && kappa_shift(kappa) >= gthr;
-                    if constexpr (FILTER) pass = pass && ((allow_word >> (my_row & 31u)) & 1u);
+                    if constexpr (RESTRICT) {
+                        const bool allowed = my_row < p.n && ((allow_word >> (my_row & 31u)) & 1u);
+                        pass = pass && allowed && kappa <= cut;
+                        n_above += __popc(__ballot_sync(0xFFFFFFFFu, allowed && kappa > cut));
+                    }
                     tb.push_warp(pass, key);
                     if (pass) atomicAdd(p.hist + kappa_bin(kappa), 1u);
 #ifdef PBX_EXP_PROFILE
@@ -334,12 +351,13 @@ scan_kernel(const ScanParams p) {
                 } else {
                     bool pass = false;
                     KeyX key = KeyOps<KeyX>::lowest();
-                    if (my_row < p.n && kappa >= theta && row_allowed(p.allow, my_row)) {
+                    if (my_row < p.n && kappa >= theta && kappa <= cut && row_allowed(p.allow, my_row)) {
                         const ReplayOut ro = replay_row<false>(reinterpret_cast<const uint8_t*>(p.rows) + (size_t)my_row * ((size_t)PR * 16),
                                                                p.qbytes, p.q16, p.dim, qh.sum_cq, sh.lut);
                         float dist = ref_distance(qh.sa, ro.sb, ro.dot);
-                        if ((double)dist < p.max_dist) {
-                            key = make_keyx(dist, __ldg(p.ids + my_row), my_row);
+                        const int64_t id = __ldg(p.ids + my_row);
+                        if (dist < p.max_dist && !page_before(p.cut, dist, id)) {
+                            key = make_keyx(dist, id, my_row);
                             pass = keyx_gt(key, tau);
                         }
                     }
@@ -349,6 +367,9 @@ scan_kernel(const ScanParams p) {
             }
             if constexpr (!EXACT) {
                 if (warp == 0 && lane == 0 && gpoll > sh.gb) sh.gb = gpoll;
+            }
+            if constexpr (RESTRICT) {
+                if (lane == 0 && n_above) atomicAdd(&p.cut->above, n_above);
             }
             continue;
         }
@@ -413,6 +434,7 @@ scan_generic_kernel(const ScanParams p) {
     const int bias = -255 * qh.sum_cq;
     float theta = 0.0f;
     if constexpr (EXACT) theta = p.status->theta;
+    const float cut = page_kappa_hi(p.cut);
     if (threadIdx.x == 0) { sh.cnt = 0; sh.tau = KeyOps<K>::lowest(); }
     TopBuf<K> tb{buf, &sh.cnt, &sh.tau, p.cap, p.keep};
     const uint32_t n_tiles = (p.n + kTileRows - 1) / kTileRows;
@@ -425,6 +447,7 @@ scan_generic_kernel(const ScanParams p) {
         const uint32_t tile = sh.tile[0];
         if (tile >= n_tiles) break;
         const K tau = sh.tau;
+        uint32_t n_above = 0;
         for (int it = 0; it < kItersPerTile; ++it) {
             const uint32_t my_row = tile * kTileRows + (uint32_t)(it * kScanWarps + warp) * kRowsPerWarpIter + lane;
             const float inv_r = __ldg(p.inv_norm + my_row);
@@ -440,23 +463,29 @@ scan_generic_kernel(const ScanParams p) {
             const float kappa = __fmul_rn(__fmul_rn((float)dot_i, inv_r), qh.inv_q);
             if constexpr (!EXACT) {
                 const u64 key = make_key64(kappa, my_row);
-                const bool pass = my_row < p.n && key > tau && row_allowed(p.allow, my_row);
+                const bool allowed = my_row < p.n && row_allowed(p.allow, my_row);
+                const bool pass = allowed && key > tau && kappa <= cut;
+                n_above += __popc(__ballot_sync(0xFFFFFFFFu, allowed && kappa > cut));
                 tb.push_warp(pass, key);
                 if (pass) atomicAdd(p.hist + kappa_bin(kappa), 1u);
             } else {
                 bool pass = false;
                 KeyX key = KeyOps<KeyX>::lowest();
-                if (my_row < p.n && kappa >= theta && row_allowed(p.allow, my_row)) {
+                if (my_row < p.n && kappa >= theta && kappa <= cut && row_allowed(p.allow, my_row)) {
                     const ReplayOut ro = replay_row<false>(reinterpret_cast<const uint8_t*>(p.rows) + (size_t)my_row * ((size_t)p.pitch16 * 16),
                                                            p.qbytes, p.q16, p.dim, qh.sum_cq, sh.lut);
                     float dist = ref_distance(qh.sa, ro.sb, ro.dot);
-                    if ((double)dist < p.max_dist) {
-                        key = make_keyx(dist, __ldg(p.ids + my_row), my_row);
+                    const int64_t id = __ldg(p.ids + my_row);
+                    if (dist < p.max_dist && !page_before(p.cut, dist, id)) {
+                        key = make_keyx(dist, id, my_row);
                         pass = keyx_gt(key, tau);
                     }
                 }
                 tb.push_warp(pass, key);
             }
+        }
+        if constexpr (!EXACT) {
+            if (lane == 0 && n_above) atomicAdd(&p.cut->above, n_above);
         }
     }
     tb.compact();

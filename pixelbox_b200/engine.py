@@ -2,7 +2,7 @@
 
 Same method names, argument meaning and error behaviour as src/engine.rs for the calls the UI makes
 on this path (`open`, `new`, `query_by_image_hash_from_image`, `get_query_results`,
-`clear_query_results`, `insert_image_from_memory`, `max_distance_from_query`), over Python's sqlite3 and
+`clear_query_results`, `insert_image_from_memory`, `max_distance_from_query`), plus `load_more_results`, over Python's sqlite3 and
 the C-ABI library.  The reference's toolchain (Rust) is absent from this image, so this is the
 executable form of the patch INTEGRATION.md describes.  Everything outside the path (text search,
 tags, crawling, image decoding, thumbnails) is not built.
@@ -17,7 +17,6 @@ from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
-from . import _native as nat
 from .corpus import Corpus
 
 # src/engine.rs:22-25
@@ -73,6 +72,7 @@ class Engine:
         self.max_search_results = DEFAULT_MAX_SEARCH_RESULTS            # :91 (unused by queries upstream too)
         self.max_distance_from_query = DEFAULT_MAX_QUERY_DISTANCE       # :92
         self.cached_search_results: Optional[List[IndexedImage]] = None
+        self._last_query: Optional[dict] = None                          # load_more_results continues it
         self.corpus: Optional[Corpus] = None
         self.skipped_rows = 0
         self._load_corpus()
@@ -128,67 +128,78 @@ class Engine:
         self.write_connection.close()
 
     # -- search -------------------------------------------------------------------------------------
+    _JOIN_SQL = (f"SELECT {SELECT_FIELDS}, semantic_hashes.hash FROM images "
+                 "JOIN semantic_hashes ON images.id = semantic_hashes.image_id WHERE images.id = ?")
+
     def query_by_image_hash_from_image(self, indexed_image: IndexedImage) -> None:
         """src/engine.rs:363-396.  Returns silently when the hash is missing (:364-368); otherwise fills
         cached_search_results with at most 100 images (:381) with dist < max_distance_from_query (:379),
-        ordered by dist ascending (:380), each carrying visual_hash and distance_from_query (:385-386)."""
-        if indexed_image.visual_hash is None:
-            sys.stderr.write("TODO: IndexedImage is somehow missing a hash!\n")
-            return
-        self.cached_search_results = None
-        t0 = time.perf_counter()
-        results: List[IndexedImage] = []
-        if self.corpus is not None:
-            sql = (f"SELECT {SELECT_FIELDS}, semantic_hashes.hash FROM images "
-                   "JOIN semantic_hashes ON images.id = semantic_hashes.image_id WHERE images.id = ?")
-            query = np.frombuffer(indexed_image.visual_hash, np.uint8)
-            k = 100                                                           # LIMIT 100, :381
-            while True:
-                res = self.corpus.search(query, k, self.max_distance_from_query)[0]
-                # hydration (SURVEY.md 8f N1): indexed lookups in the GPU's order
-                results = []
-                for image_id, dist in zip(res.ids, res.dist):
-                    row = self.read_connection.execute(sql, (int(image_id),)).fetchone()
-                    if row is None:
-                        continue                 # INNER JOIN semantics: a hash without an image row is dropped
-                    results.append(IndexedImage(id=row[0], filename=row[1], path=row[2], resolution=(row[3], row[4]),
-                                                thumbnail=row[5], visual_hash=row[6], distance_from_query=float(dist)))
-                    if len(results) == 100:
-                        break
-                # upstream applies LIMIT after the join: if orphans ate into the list, ask for more rows
-                if len(results) == 100 or len(res.ids) < k or k >= nat.PBX_MAX_K:
-                    break
-                k = min(nat.PBX_MAX_K, 2 * k)
-        self.cached_search_results = results
-        sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(results)}\n")
+        ordered by dist ascending (:380), each carrying visual_hash and distance_from_query (:385-386).
+        Upstream applies LIMIT 100 after the INNER JOIN with `images`, so a hash without an image row does not use up
+        one of the 100: the GPU rows are taken in pages of 100 after the last one consumed until 100 joined rows are
+        found or the table is exhausted, however many such hashes come first."""
+        self._similarity_query(indexed_image, None)
 
     def query_by_image_hash_within_folder(self, indexed_image: IndexedImage, folder: str) -> None:
         """query_by_image_hash_from_image restricted to the images under `folder`: the similarity SQL with
         `AND substr(images.path, 1, length(?)) = ?` added (folder with a trailing separator, so that /a/b does not match
-        /a/bc; no LIKE, whose % and _ occur in real paths).  The folder's ids come from `images`, so a hash without an
-        image row is never among them: one filtered search of k = 100 answers the query, no k-doubling."""
+        /a/bc; no LIKE, whose % and _ occur in real paths).  The folder's ids come from `images`; a row deleted between
+        the id query and the search is dropped by the join like any other hash without an image row."""
+        self._similarity_query(indexed_image, folder)
+
+    def load_more_results(self, count: int = DEFAULT_MAX_SEARCH_RESULTS) -> None:
+        """"Show more": extends cached_search_results with the next `count` joined rows of the last similarity query
+        (query_by_image_hash_from_image or ..._within_folder), in the same order -- the verbatim SQL with
+        LIMIT count OFFSET (rows shown so far).  Each call is one keyset page after the last GPU row consumed, over the
+        table as it is now; nothing happens without a previous query."""
+        if self._last_query is None or self.cached_search_results is None:
+            return
+        t0 = time.perf_counter()
+        more = self._joined_rows(int(count))
+        self.cached_search_results = self.cached_search_results + more
+        sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(more)} more\n")
+
+    def _similarity_query(self, indexed_image: IndexedImage, folder: Optional[str]) -> None:
         if indexed_image.visual_hash is None:
             sys.stderr.write("TODO: IndexedImage is somehow missing a hash!\n")
             return
         self.cached_search_results = None
+        self._last_query = None
         t0 = time.perf_counter()
         results: List[IndexedImage] = []
         if self.corpus is not None:
-            prefix = folder if folder.endswith(("/", "\\")) else folder + "/"
-            folder_ids = np.fromiter((r[0] for r in self.read_connection.execute(
-                "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
-            query = np.frombuffer(indexed_image.visual_hash, np.uint8)
-            res = self.corpus.search(query, DEFAULT_MAX_SEARCH_RESULTS, self.max_distance_from_query, within=folder_ids)[0]
-            sql = (f"SELECT {SELECT_FIELDS}, semantic_hashes.hash FROM images "
-                   "JOIN semantic_hashes ON images.id = semantic_hashes.image_id WHERE images.id = ?")
-            for image_id, dist in zip(res.ids, res.dist):
-                row = self.read_connection.execute(sql, (int(image_id),)).fetchone()
-                if row is None:
-                    continue                     # deleted between the id query and the search
-                results.append(IndexedImage(id=row[0], filename=row[1], path=row[2], resolution=(row[3], row[4]),
-                                            thumbnail=row[5], visual_hash=row[6], distance_from_query=float(dist)))
+            within = None
+            if folder is not None:
+                prefix = folder if folder.endswith(("/", "\\")) else folder + "/"
+                within = np.fromiter((r[0] for r in self.read_connection.execute(
+                    "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
+            # what load_more_results continues from: the query, its max_dist and folder, the last GPU row consumed
+            self._last_query = dict(query=np.frombuffer(indexed_image.visual_hash, np.uint8), max_dist=self.max_distance_from_query,
+                                    within=within, cursor=None, exhausted=False)
+            results = self._joined_rows(DEFAULT_MAX_SEARCH_RESULTS)                  # LIMIT 100, :381
         self.cached_search_results = results
         sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(results)}\n")
+
+    def _joined_rows(self, count: int) -> List[IndexedImage]:
+        """The next `count` rows of the last similarity query that have an `images` row (INNER JOIN semantics), hydrated
+        by indexed lookups in the GPU's order (SURVEY.md 8f N1).  GPU rows come in pages of 100 after the last row
+        consumed; a page shorter than 100 is the end of the table."""
+        st = self._last_query
+        out: List[IndexedImage] = []
+        while len(out) < count and not st["exhausted"]:
+            after = None if st["cursor"] is None else [st["cursor"]]
+            res = self.corpus.search(st["query"], DEFAULT_MAX_SEARCH_RESULTS, st["max_dist"], within=st["within"], after=after)[0]
+            for image_id, dist in zip(res.ids, res.dist):
+                st["cursor"] = (dist, int(image_id))
+                row = self.read_connection.execute(self._JOIN_SQL, (int(image_id),)).fetchone()
+                if row is not None:
+                    out.append(IndexedImage(id=row[0], filename=row[1], path=row[2], resolution=(row[3], row[4]),
+                                            thumbnail=row[5], visual_hash=row[6], distance_from_query=float(dist)))
+                    if len(out) == count:
+                        break
+            else:
+                st["exhausted"] = len(res.ids) < DEFAULT_MAX_SEARCH_RESULTS
+        return out
 
     def get_query_results(self) -> Optional[List[IndexedImage]]:
         return None if self.cached_search_results is None else list(self.cached_search_results)   # :398-400

@@ -145,16 +145,24 @@ class ShardedCorpus:
         return self._bufs[key]
 
     def search_device(self, d_queries: torch.Tensor, nq: int, k: int, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None,
-                      excluding=None):
+                      excluding=None, after=None):
         """Device-resident sharded search on the current torch stream, no host synchronisation:
         local search -> exchange of the [nq][k] records + merge (one kernel over peer memory, or NCCL
         all-gather + merge kernel).  Returns (hits, counts) device tensors (uint8 view of pbx_hit
         records, int32).  within / excluding: global image ids as in Corpus.search (every rank passes the same
-        ones); each shard searches its allowed rows exactly, so the merge gives the filtered result of the table."""
+        ones); each shard searches its allowed rows exactly, so the merge gives the filtered result of the table.
+        after: cursors as in Corpus.search (every rank passes the same ones); each shard returns its next k rows after
+        the same global cursor, so the merge gives the table's next page."""
         assert self.on_gpu
         b = self._buffers(nq, k)
         stream = torch.cuda.current_stream().cuda_stream
-        if within is not None or excluding is not None:
+        if after is not None:
+            fids, mode = nat.page_filter_args(within, excluding)
+            d_fids = torch.from_numpy(np.unique(fids)).to(self._dev())
+            d_after = torch.from_numpy(nat.page_cursors(after, nq).view(np.uint8)).to(self._dev())
+            self.local.search_device_page(d_queries.data_ptr(), nq, k, max_dist, b["local"].data_ptr(), b["cnt"].data_ptr(),
+                                          d_after.data_ptr(), d_fids.data_ptr() if d_fids.numel() else 0, d_fids.numel(), mode, stream)
+        elif within is not None or excluding is not None:
             fids, mode = nat.filter_args(within, excluding)
             d_fids = torch.from_numpy(np.unique(fids)).to(self._dev())          # the device form wants them sorted
             self.local.search_device_filtered(d_queries.data_ptr(), nq, k, max_dist, b["local"].data_ptr(), b["cnt"].data_ptr(),
@@ -180,9 +188,9 @@ class ShardedCorpus:
         return b["out"], b["out_cnt"]
 
     def search(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None,
-               excluding=None) -> List[SearchResult]:
+               excluding=None, after=None) -> List[SearchResult]:
         """Host buffers in, host buffers out, on every rank (all ranks pass the same queries, and the same
-        within / excluding image ids: see Corpus.search)."""
+        within / excluding image ids and after cursors: see Corpus.search)."""
         filtered = within is not None or excluding is not None
         if filtered:
             fids, mode = nat.filter_args(within, excluding)
@@ -196,7 +204,13 @@ class ShardedCorpus:
             # the whole step inside the library: H2D, local search, exchange + merge kernel, D2H, one synchronisation
             hits = np.empty((nq, k), nat.HIT_DTYPE)
             cnt = np.empty(nq, np.uint32)
-            if filtered:
+            if after is not None:
+                fids, mode = nat.page_filter_args(within, excluding)
+                cur = nat.page_cursors(after, nq)
+                nat.check(nat.lib().pbx_exchange_search_hits_page(self._exchange, self.local.handle, nat.ptr(q), nq, int(k), float(max_dist),
+                                                                  nat.ptr(cur), nat.ptr(fids), fids.size, mode, nat.ptr(hits),
+                                                                  nat.ptr(cnt)))
+            elif filtered:
                 nat.check(nat.lib().pbx_exchange_search_hits_filtered(self._exchange, self.local.handle, nat.ptr(q), nq, int(k),
                                                                       float(max_dist), nat.ptr(hits), nat.ptr(cnt), nat.ptr(fids),
                                                                       fids.size, mode))
@@ -207,7 +221,7 @@ class ShardedCorpus:
             b = self._buffers(nq, k)
             b["hq"].copy_(torch.from_numpy(q.reshape(-1)))
             b["q"].copy_(b["hq"], non_blocking=True)
-            d_hits, d_cnt = self.search_device(b["q"], nq, k, max_dist, within=within, excluding=excluding)
+            d_hits, d_cnt = self.search_device(b["q"], nq, k, max_dist, within=within, excluding=excluding, after=after)
             b["h_out"].copy_(d_hits, non_blocking=True)
             b["h_cnt"].copy_(d_cnt, non_blocking=True)
             torch.cuda.current_stream().synchronize()
@@ -215,8 +229,8 @@ class ShardedCorpus:
             cnt = b["h_cnt"].numpy().astype(np.uint32)
             if (cnt == 0xFFFFFFFF).any():
                 raise nat.PbxError(-8, "peer exchange timed out: a rank did not post its records")
-        elif filtered:
-            raise nat.PbxError(-1, "filtered search needs GPU shards")
+        elif filtered or after is not None:
+            raise nat.PbxError(-1, "filtered or paged search needs GPU shards")
         else:
             l_hits, l_cnt = self.local.search_hits(q, k, max_dist)
             mine = torch.from_numpy(np.ascontiguousarray(l_hits).view(np.uint8).reshape(-1).copy())
