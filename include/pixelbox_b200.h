@@ -126,7 +126,8 @@ PBX_API int pbx_corpus_append_device(pbx_corpus* c, const int64_t* d_image_ids, 
 
 /* Replaces: `DELETE FROM semantic_hashes WHERE image_id IN (...)` as seen by later scans.  Hook: after the DELETE of a
  * removed tracked folder commits (the TODO of remove_tracked_folder, src/engine.rs:414), with the folder's image ids; also
- * what follows an external edit of the table, and the first half of replacing a hash (remove, then append).
+ * what follows an external edit of the table.  To replace a hash, use pbx_corpus_replace: a remove then an append is
+ * not atomic (a search in between misses the image) and moves rows.
  *   - every committed or pending row whose image_id is in image_ids[0, n) is removed; the corpus does not enforce unique
  *     ids, so an id on several rows removes all of them.  Ids that match nothing are ignored; an id repeated in the
  *     request counts once.  *out_removed (may be NULL) receives the number of rows removed.
@@ -141,6 +142,23 @@ PBX_API int pbx_corpus_append_device(pbx_corpus* c, const int64_t* d_image_ids, 
  * Cost: a host sort of the request, one pass over the ids (8 bytes per row) plus the block metadata (8 bytes per row) on
  * the device, and a copy of the moved rows only. */
 PBX_API int pbx_corpus_remove(pbx_corpus* c, const int64_t* image_ids, uint64_t n, uint64_t* out_removed);
+
+/* Replaces: `UPDATE semantic_hashes SET hash = ? WHERE image_id = ?` as seen by later scans, one statement per listed id,
+ * in order.  Hook: after such an UPDATE commits (a re-index of a modified file, a re-hash after a model fix, an external
+ * edit of the table).  hashes is [n][dim] row-major u8: hashes[i] is the new hash of image_ids[i].
+ *   - every committed or pending row whose image_id is listed gets the hash listed for that id, in place: positions, ids
+ *     and the size do not change (pbx_corpus_read_rows shows the new bytes at the same positions).  An id on several
+ *     rows replaces all of them; an id listed more than once takes its LAST hash; ids that match nothing are ignored.
+ *   - *out_replaced (may be NULL) receives the number of rows written, counted as SQLite's changes(): a row counts even
+ *     when its new hash equals the old one.
+ *   - n == 0 returns PBX_OK; NULL c, NULL image_ids or hashes with n > 0, or n > PBX_MAX_ROWS is PBX_E_INVALID.
+ *   - synchronous, and atomic with respect to searches, as pbx_corpus_remove: appends that arrived before the call
+ *     (coalesced pending ones included) are subject to it; work already enqueued by pbx_search_device (on any stream)
+ *     completes against the old hashes; every search issued after the call returns gives exactly what a corpus freshly
+ *     loaded with the updated table, in the same row order, gives (ids, dist bit for bit, dot, norm2).
+ * Cost: a host sort of the request (skipped for ids already strictly ascending) and its upload, one pass over the ids
+ * (8 bytes per row) on the device, and a copy plus the row and 32-row-block metadata of the written rows only. */
+PBX_API int pbx_corpus_replace(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint64_t* out_replaced);
 
 /* Bench/test only: fills the shard on the device with rows [first_row, first_row + n) of the
  * counter-based synthetic corpus (pixelbox_b200/synth.py), image_id = global row + 1. */
@@ -279,6 +297,9 @@ PBX_API int pbx_sharded_append(pbx_sharded* s, const int64_t* image_ids, const u
 /* pbx_corpus_remove over all shards: ids are global and do not name a shard, so every shard applies the whole request
  * (one after the other, atomic with respect to pbx_sharded_search); *out_removed (may be NULL) is the total. */
 PBX_API int pbx_sharded_remove(pbx_sharded* s, const int64_t* image_ids, uint64_t n, uint64_t* out_removed);
+/* pbx_corpus_replace over all shards, in the same way: every shard applies the whole request (one after the other,
+ * atomic with respect to pbx_sharded_search); *out_replaced (may be NULL) is the total. */
+PBX_API int pbx_sharded_replace(pbx_sharded* s, const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint64_t* out_replaced);
 /* Bench/test only: shard i holds rows [i * rows_per_shard, (i + 1) * rows_per_shard) of the synthetic corpus. */
 PBX_API int pbx_sharded_fill_synthetic(pbx_sharded* s, uint64_t rows_per_shard, uint64_t seed);
 PBX_API int pbx_sharded_size(const pbx_sharded* s, uint64_t* n_rows);

@@ -45,6 +45,16 @@ def _remove(fn, handle, image_ids) -> int:
     return int(removed.value)
 
 
+def _replace(fn, handle, dim, image_ids, hashes) -> int:
+    hashes = _as_u8_2d(hashes, dim, "replace")
+    ids = np.ascontiguousarray(np.asarray(image_ids, dtype=np.int64)).reshape(-1)
+    if ids.shape != (hashes.shape[0],):
+        raise nat.PbxError(-1, "replace: one image_id per hash row required")
+    replaced = ctypes.c_uint64(0)
+    nat.check(fn(handle, nat.ptr(ids), nat.ptr(hashes), ids.size, ctypes.byref(replaced)))
+    return int(replaced.value)
+
+
 class Corpus:
     def __init__(self, dim: int, capacity_hint: int = 0, device: int = 0):
         self._h = ctypes.c_void_p(0)
@@ -109,6 +119,11 @@ class Corpus:
         """pbx_corpus_remove: removes every row (pending ones included) whose image_id is listed; returns the number of
         rows removed.  Surviving rows from the tail move into the freed positions (see read_rows)."""
         return _remove(nat.lib().pbx_corpus_remove, self._h, image_ids)
+
+    def replace(self, image_ids, hashes) -> int:
+        """pbx_corpus_replace: every row (pending ones included) whose image_id is listed gets the hash listed for it, in
+        place (an id listed twice takes its last hash); returns the number of rows written.  Positions do not change."""
+        return _replace(nat.lib().pbx_corpus_replace, self._h, self.dim, image_ids, hashes)
 
     def fill_synthetic(self, n: int, seed: int, first_row: int = 0) -> None:
         nat.check(nat.lib().pbx_corpus_fill_synthetic(self._h, int(n), int(seed), int(first_row)))
@@ -317,6 +332,10 @@ class MultiDeviceCorpus:
     def remove(self, image_ids) -> int:
         """pbx_sharded_remove: every shard removes the listed ids; returns the total number of rows removed."""
         return _remove(nat.lib().pbx_sharded_remove, self._h, image_ids)
+
+    def replace(self, image_ids, hashes) -> int:
+        """pbx_sharded_replace: every shard replaces the hashes of the listed ids; returns the total number of rows written."""
+        return _replace(nat.lib().pbx_sharded_replace, self._h, self.dim, image_ids, hashes)
 
     def fill_synthetic(self, rows_per_shard: int, seed: int) -> None:
         nat.check(nat.lib().pbx_sharded_fill_synthetic(self._h, int(rows_per_shard), int(seed)))

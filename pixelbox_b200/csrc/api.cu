@@ -16,6 +16,7 @@
 #include "finalize.cuh"
 #include "batch.cuh"
 #include "remove.cuh"
+#include "replace.cuh"
 #include "page.cuh"
 
 using namespace pbx;
@@ -972,6 +973,111 @@ extern "C" int pbx_corpus_remove(pbx_corpus* c, const int64_t* image_ids, uint64
     std::vector<int64_t> req;
     int rc = sorted_request(image_ids, n, &req);
     return rc == PBX_OK ? remove_sorted(c, req, out_removed) : rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// replacement
+// ------------------------------------------------------------------------------------------------
+// The request as the kernels want it: ids sorted, every id once with the hash of its LAST occurrence (what a sequence of
+// UPDATE statements leaves), and [ids.size()][pitch] rows in that order with zero padding.  Sorting (id, position) pairs
+// puts the last occurrence at the end of each run; ids already strictly in order skip the sort.
+struct ReplaceRequest {
+    std::vector<int64_t> ids;
+    std::vector<uint8_t> rows;
+};
+static int replace_request(const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint32_t dim, uint32_t pitch, ReplaceRequest* out) {
+    if (n > PBX_MAX_ROWS) return fail(PBX_E_INVALID, "replace request of %llu ids (max %llu)", (unsigned long long)n, (unsigned long long)PBX_MAX_ROWS);
+    try {
+        std::vector<std::pair<int64_t, uint32_t>> order(n);
+        for (uint64_t i = 0; i < n; ++i) order[i] = {image_ids[i], (uint32_t)i};
+        if (std::adjacent_find(image_ids, image_ids + n, [](int64_t a, int64_t b) { return a >= b; }) != image_ids + n)
+            std::sort(order.begin(), order.end());
+        out->ids.clear();
+        for (uint64_t i = 0; i < n; ++i)
+            if (i + 1 == n || order[i + 1].first != order[i].first) out->ids.push_back(order[i].first);
+        out->rows.assign(out->ids.size() * (size_t)pitch, 0);
+        for (uint64_t i = 0, j = 0; i < n; ++i)
+            if (i + 1 == n || order[i + 1].first != order[i].first) memcpy(out->rows.data() + (j++) * pitch, hashes + (size_t)order[i].second * dim, dim);
+    } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
+    return PBX_OK;
+}
+
+// Writes the request's hash into every row whose id it lists, in place (replace.cuh).  Locks and orders as remove_sorted:
+// the pending appends are flushed first, so they are subject to the replacement; with mu held no search can be enqueued,
+// and the stream waits for the last one already enqueued (ev_chain) before it touches a row.  Returns after the stream is
+// synchronised.  Positions, ids and n do not change.
+static int replace_sorted(pbx_corpus* c, const ReplaceRequest& req, uint64_t* out_replaced) {
+    std::lock_guard<std::mutex> alk(c->append_mu);
+    int rc = flush_pending_locked(c);
+    if (rc != PBX_OK) return rc;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CU_TRY(cudaSetDevice(c->device));
+    const uint64_t n = c->n.load(), u = req.ids.size();
+    if (n == 0 || u == 0) return PBX_OK;
+    cudaStream_t s = c->copy_stream;
+    if (c->chain_valid) CU_TRY(cudaStreamWaitEvent(s, c->ev_chain, 0));
+    const unsigned tiles = (unsigned)((n + kMarkTileRows - 1) / kMarkTileRows);
+    // scratch, stream-ordered: [request ids][request rows][counts: pairs, blocks], then the pair and block lists sized for
+    // one row per id (ids are unique in the table the corpus caches); more matches size them exactly and mark once more
+    const size_t off_rows = (u * sizeof(int64_t) + 15) / 16 * 16, off_cnt = off_rows + u * c->pitch;
+    unsigned char* scratch = nullptr;
+    unsigned char* lists = nullptr;
+    uint64_t cap = std::min<uint64_t>(n, u);
+    uint32_t counts[2] = {0, 0};
+    CU_TRY(cudaMallocAsync(reinterpret_cast<void**>(&scratch), off_cnt + 16, s));
+    int64_t* d_req = reinterpret_cast<int64_t*>(scratch);
+    uint32_t* d_counts = reinterpret_cast<uint32_t*>(scratch + off_cnt);
+    cudaError_t e = cudaMemcpyAsync(d_req, req.ids.data(), u * sizeof(int64_t), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(scratch + off_rows, req.rows.data(), u * c->pitch, cudaMemcpyHostToDevice, s);
+    for (int pass = 0; pass < 2 && e == cudaSuccess; ++pass) {
+        e = cudaMallocAsync(reinterpret_cast<void**>(&lists), cap * (sizeof(uint2) + sizeof(uint32_t)), s);
+        if (e == cudaSuccess) e = cudaMemsetAsync(d_counts, 0, 2 * sizeof(uint32_t), s);
+        if (e == cudaSuccess) {
+            replace_mark_kernel<<<tiles, kMarkTileRows, 0, s>>>(c->d_ids, n, d_req, u, (uint32_t)cap, reinterpret_cast<uint2*>(lists),
+                                                                reinterpret_cast<uint32_t*>(lists + cap * sizeof(uint2)), d_counts);
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(counts, d_counts, sizeof(counts), cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);    // the count sizes the rest (a second time only if ids repeat)
+        if (e != cudaSuccess || counts[0] <= cap) break;
+        cudaFreeAsync(lists, s);
+        lists = nullptr;
+        cap = counts[0];
+    }
+    const uint64_t m = counts[0], blocks = counts[1];
+    if (e == cudaSuccess && (m > cap || blocks > m)) {
+        if (lists) cudaFreeAsync(lists, s);
+        cudaFreeAsync(scratch, s);
+        cudaStreamSynchronize(s);
+        return fail(PBX_E_INTERNAL, "replacement counted %llu rows in %llu blocks of %llu rows", (unsigned long long)m, (unsigned long long)blocks, (unsigned long long)n);
+    }
+    if (e == cudaSuccess && m) {
+        const uint2* d_pairs = reinterpret_cast<const uint2*>(lists);
+        const uint32_t* d_blocks = reinterpret_cast<const uint32_t*>(lists + cap * sizeof(uint2));
+        const uint64_t chunks = m * c->pitch16;
+        const unsigned grid = (unsigned)std::min<uint64_t>((chunks + 255) / 256, (uint64_t)c->sm_count * 8);
+        replace_write_kernel<<<grid, 256, 0, s>>>(d_pairs, m, reinterpret_cast<const uint4*>(scratch + off_rows), c->pitch16, reinterpret_cast<uint4*>(c->d_rows));
+        replace_row_meta_kernel<<<(unsigned)((m + 7) / 8), 256, 0, s>>>(d_pairs, m, reinterpret_cast<const uint4*>(c->d_rows), c->pitch16, c->dim, c->d_inv, c->d_rsum);
+        replace_block_meta_kernel<<<(unsigned)((blocks + 7) / 8), 256, 0, s>>>(d_blocks, blocks, c->d_inv, c->d_rsum, c->dim, n, c->d_bmeta);
+        e = cudaGetLastError();
+    }
+    if (lists) cudaFreeAsync(lists, s);
+    cudaFreeAsync(scratch, s);
+    const cudaError_t e2 = cudaStreamSynchronize(s);
+    if (e == cudaSuccess) e = e2;
+    if (e != cudaSuccess) return fail(PBX_E_CUDA, "replacement failed: %s", cudaGetErrorString(e));
+    if (out_replaced) *out_replaced = m;
+    return PBX_OK;
+}
+
+extern "C" int pbx_corpus_replace(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint64_t* out_replaced) {
+    if (out_replaced) *out_replaced = 0;
+    if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (n && (!image_ids || !hashes)) return fail(PBX_E_INVALID, "NULL ids or hashes with n > 0");
+    if (n == 0) return PBX_OK;
+    ReplaceRequest req;
+    int rc = replace_request(image_ids, hashes, n, c->dim, c->pitch, &req);
+    return rc == PBX_OK ? replace_sorted(c, req, out_replaced) : rc;
 }
 
 // ------------------------------------------------------------------------------------------------

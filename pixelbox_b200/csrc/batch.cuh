@@ -250,11 +250,9 @@ __device__ __forceinline__ int max3(int a, int b, int c) { return max(max(a, b),
 // ---- per-32-row block metadata (load time): what the epilogue's one-compare test needs from the rows --------------------
 // blk[b] = { norm_lo, norm_hi, rowterm_max, rowterm_min (as int bits) } over rows [32 b, 32 b + 32) below n_rows:
 // norm = 1 / inv_norm (f32 division, the same expression everywhere), rowterm = 2 sum r - 255 dim.
-__global__ void block_meta_kernel(const float* __restrict__ inv_norm, const int* __restrict__ row_sum, uint32_t dim,
-                                  uint64_t first_block, uint64_t n_blocks, uint64_t n_rows, float4* __restrict__ blk) {
-    const uint64_t b = first_block + (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (b >= first_block + n_blocks) return;
+// One warp computes block b.
+__device__ __forceinline__ void block_meta_warp(const float* __restrict__ inv_norm, const int* __restrict__ row_sum, uint32_t dim,
+                                                uint64_t b, int lane, uint64_t n_rows, float4* __restrict__ blk) {
     const uint64_t row = b * 32 + (uint64_t)lane;
     const bool ok = row < n_rows;
     float inv_lo = ok ? inv_norm[row] : __int_as_float(0x7f800000), inv_hi = ok ? inv_norm[row] : 0.0f;
@@ -275,6 +273,12 @@ __global__ void block_meta_kernel(const float* __restrict__ inv_norm, const int*
         m.w = __int_as_float(rt_min);
         blk[b] = m;
     }
+}
+__global__ void block_meta_kernel(const float* __restrict__ inv_norm, const int* __restrict__ row_sum, uint32_t dim,
+                                  uint64_t first_block, uint64_t n_blocks, uint64_t n_rows, float4* __restrict__ blk) {
+    const uint64_t b = first_block + (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (b >= first_block + n_blocks) return;
+    block_meta_warp(inv_norm, row_sum, dim, b, threadIdx.x & 31, n_rows, blk);
 }
 
 // ---- per-batch query preparation: one CTA per (padded) query ---------------------------------------------

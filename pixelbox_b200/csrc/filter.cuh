@@ -1,5 +1,6 @@
 // filter.cuh -- one bit per row from a set of image ids: the mark pass of pbx_corpus_remove (rows to remove) and of the
-// filtered searches (rows a search may return, pbx_search_filtered and its twins).
+// filtered searches (rows a search may return, pbx_search_filtered and its twins).  pbx_corpus_replace's mark pass
+// (replace.cuh) uses the same binary search.
 //
 // mark_ids_kernel is one pass over the row ids (8 bytes per row) with a binary search of each id in the sorted set; the
 // search kernels then test bit (row & 31) of word row >> 5 (row_allowed, common.cuh).
@@ -10,16 +11,17 @@ namespace pbx {
 
 constexpr int kMarkTileRows = 1024;          // one CTA of 1024 threads, one row per thread
 
-// Binary search in an ascending set (duplicates allowed).  Any input is memory-safe: an unsorted set gives a wrong
+// Binary search in an ascending set (duplicates allowed): the first index whose element is not below v (n_set if none).
+// v is in the set iff the result is < n_set and holds v.  Any input is memory-safe: an unsorted set gives a wrong
 // answer, never an out-of-bounds read.
-__device__ __forceinline__ bool sorted_contains(const int64_t* __restrict__ set, u64 n_set, int64_t v) {
+__device__ __forceinline__ u64 sorted_lower_bound(const int64_t* __restrict__ set, u64 n_set, int64_t v) {
     u64 lo = 0, hi = n_set;
     while (lo < hi) {
         const u64 mid = (lo + hi) >> 1;
         if (set[mid] < v) lo = mid + 1;
         else hi = mid;
     }
-    return lo < n_set && set[lo] == v;
+    return lo;
 }
 
 // flags[w] bit l: row 32 w + l (< n) has its id in the set, or with `invert` has not.  *marked += number of set bits.
@@ -27,7 +29,12 @@ __device__ __forceinline__ bool sorted_contains(const int64_t* __restrict__ set,
 __global__ void __launch_bounds__(kMarkTileRows) mark_ids_kernel(const int64_t* __restrict__ ids, u64 n, const int64_t* __restrict__ set,
                                                                  u64 n_set, uint32_t invert, uint32_t* __restrict__ flags, u64* __restrict__ marked) {
     const u64 row = (u64)blockIdx.x * kMarkTileRows + threadIdx.x;
-    const bool bit = row < n && (sorted_contains(set, n_set, ids[row]) != (invert != 0));
+    bool bit = false;
+    if (row < n) {
+        const int64_t id = ids[row];
+        const u64 at = sorted_lower_bound(set, n_set, id);
+        bit = (at < n_set && set[at] == id) != (invert != 0);
+    }
     const uint32_t word = __ballot_sync(0xFFFFFFFFu, bit);
     if ((threadIdx.x & 31) == 0 && row < n) flags[row >> 5] = word;
     const int cnt = __syncthreads_count(bit);

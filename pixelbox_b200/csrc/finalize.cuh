@@ -128,11 +128,9 @@ prep_seed_kernel(const PrepSeedParams p) {
 }
 
 // ---- per-row metadata: inv_norm[r] = 1/sqrt(sum c(r_i)^2) and row_sum[r] = sum r_i, one warp per row ----------------------
-__global__ void row_meta_kernel(const uint4* __restrict__ rows, uint32_t pitch16, uint32_t dim, uint64_t first, uint64_t n,
-                                float* __restrict__ inv_norm, int* __restrict__ row_sum) {
-    const uint64_t r = first + (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (r >= first + n) return;
+// The one definition of both values: every path that writes a row (load, append, replace) computes them here.
+__device__ __forceinline__ void row_meta_warp(const uint4* __restrict__ rows, uint32_t pitch16, uint32_t dim, uint64_t r, int lane,
+                                              float* __restrict__ inv_norm, int* __restrict__ row_sum) {
     unsigned s1 = 0, s2 = 0;
     for (uint32_t c = lane; c < pitch16; c += 32) {
         uint4 v = __ldg(rows + r * pitch16 + c);
@@ -148,6 +146,12 @@ __global__ void row_meta_kernel(const uint4* __restrict__ rows, uint32_t pitch16
         inv_norm[r] = (float)(1.0 / sqrt((double)n2));
         row_sum[r] = (int)s1;                      // sum of the raw bytes: the batched (u8 x u8) path needs it per row
     }
+}
+__global__ void row_meta_kernel(const uint4* __restrict__ rows, uint32_t pitch16, uint32_t dim, uint64_t first, uint64_t n,
+                                float* __restrict__ inv_norm, int* __restrict__ row_sum) {
+    const uint64_t r = first + (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (r >= first + n) return;
+    row_meta_warp(rows, pitch16, dim, r, threadIdx.x & 31, inv_norm, row_sum);
 }
 
 // ---- synthetic corpus (bench/tests): same function as pixelbox_b200/synth.py ---------------------

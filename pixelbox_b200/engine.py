@@ -256,3 +256,37 @@ class Engine:
         # as for inserts, the device corpus follows only what has been committed
         if self.corpus is not None:
             self.corpus.remove(np.asarray(ids, np.int64))
+
+    def update_image_hashes(self, pairs) -> None:
+        """`UPDATE semantic_hashes SET hash = ? WHERE image_id = ?` for every (image_id, hash) pair, in order, in one
+        transaction; then the device corpus follows the rows the UPDATE changed, as a re-open would load them: a row
+        that keeps a hash of the corpus' dim is replaced in place, a row whose new hash has another length (or is NULL)
+        leaves the device and counts in skipped_rows, and a row skipped before that now has the corpus' dim is
+        appended.  Ids without a semantic_hashes row change nothing.  The hook for a re-index of a modified file."""
+        pairs = [(int(i), None if h is None else bytes(h)) for i, h in pairs]
+        if not pairs:
+            return
+        conn = self.write_connection
+        changed: Dict[int, Tuple[Optional[bytes], Optional[bytes]]] = {}      # image_id -> (hash before, last hash set)
+        try:
+            for image_id, h in pairs:
+                old = conn.execute("SELECT hash FROM semantic_hashes WHERE image_id = ?", (image_id,)).fetchone()
+                if conn.execute("UPDATE semantic_hashes SET hash = ? WHERE image_id = ?", (h, image_id)).rowcount:
+                    changed[image_id] = (changed[image_id][0] if image_id in changed else old[0], h)
+            conn.commit()
+        except Exception:
+            conn.rollback()
+            raise
+        if self.corpus is None or not changed:
+            return
+        dim = self.corpus.dim
+        fits = lambda h: h is not None and len(h) == dim                            # noqa: E731
+        replace = [(i, new) for i, (old, new) in changed.items() if fits(old) and fits(new)]
+        leave = [i for i, (old, new) in changed.items() if fits(old) and not fits(new)]
+        enter = [(i, new) for i, (old, new) in changed.items() if not fits(old) and fits(new)]
+        if leave:
+            self.skipped_rows += self.corpus.remove(np.array(leave, np.int64))
+        for part, op in ((replace, self.corpus.replace), (enter, self.corpus.append)):
+            if part:
+                op(np.array([i for i, _ in part], np.int64), np.frombuffer(b"".join(h for _, h in part), np.uint8).reshape(len(part), dim))
+        self.skipped_rows -= len(enter)

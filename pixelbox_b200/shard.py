@@ -118,6 +118,12 @@ class ShardedCorpus:
         mine = np.array([self.local.remove(image_ids)], np.int64)
         return int(self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).sum())
 
+    def replace(self, image_ids, hashes) -> int:
+        """Every rank passes the same (ids, hashes) and replaces the hashes of the rows its shard holds; returns the number
+        of rows written over all ranks, on every rank."""
+        mine = np.array([self.local.replace(image_ids, hashes)], np.int64)
+        return int(self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).sum())
+
     def total_rows(self) -> int:
         t = torch.tensor([len(self.local)], dtype=torch.int64, device=self._comm_dev())
         dist.all_reduce(t, group=self.group)
