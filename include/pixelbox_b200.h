@@ -160,6 +160,49 @@ PBX_API int pbx_corpus_remove(pbx_corpus* c, const int64_t* image_ids, uint64_t 
  * (8 bytes per row) on the device, and a copy plus the row and 32-row-block metadata of the written rows only. */
 PBX_API int pbx_corpus_replace(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint64_t* out_replaced);
 
+/* ---- views: a prepared id set, searched at the cost of its own rows ------------------------------------------------------
+ * Replaces: the per-call filter of a search repeated over the same set -- "similar images in this folder", asked again and
+ * again while the folder changes only when images are indexed into it or removed.  A filtered search streams the whole
+ * shard every call; a search on a view streams the view's rows only.
+ * A view is a pbx_corpus on the parent's device holding a copy of the parent's rows whose image_id is in a set of ids
+ * (the INCLUDE semantics of the filtered searches: ids that match nothing are ignored, a repeated id counts once, an id on
+ * several rows brings all of them).  Every search call accepts it (pbx_search, _hits, _device, _filtered, _page, their
+ * device forms, pbx_exchange_search_hits*), and so do pbx_corpus_size / _read_rows / _synchronize / _flush, pbx_get_stats
+ * and the pbx_set_* knobs.  pbx_corpus_load / _append / _append_device / _remove / _replace / _fill_synthetic on a view
+ * return PBX_E_INVALID: a view follows its parent.  pbx_corpus_destroy destroys it.
+ *   - Same results: a search on a view returns exactly what pbx_search_filtered (PBX_FILTER_INCLUDE, the view's set) returns
+ *     on the parent at that moment -- count, ids, order, dist bit for bit, dot, norm2, and the plateau rule over the view's
+ *     rows -- on every path: single, batched, paged, device forms, sharded and exchange.  The one difference: rows with
+ *     equal (dist, image_id) may come in another order.  That needs an id on several rows, and a view's row order may
+ *     differ from the parent's after removals.  A filter on a search of a view intersects with the view's set.
+ *   - The view follows its parent inside the parent's mutating calls, which already hold the parent's locks and
+ *     synchronise: appended rows (pbx_corpus_append, _append_device, coalesced appends when they are uploaded) whose id is
+ *     in the set join the view; pbx_corpus_remove and pbx_corpus_replace are applied to the view as well (its rows, ids,
+ *     row metadata stay the parent's bit for bit); pbx_corpus_load and _fill_synthetic rebuild it from the new rows.
+ *     Removing a row does not take its id out of the set: a later append of that id joins the view, as it would pass the
+ *     filter.  Each mutation and its forwarding are one step for searches on the view, as the remove and replace contracts
+ *     say: work already enqueued on the view finishes against the old rows, every search issued after the call returns
+ *     sees the new ones.
+ *   - A search on a view first uploads the parent's pending appends (as a search of the parent does), and so do
+ *     pbx_corpus_size, _read_rows and _flush on a view.
+ *   - If the parent is destroyed first, its views are detached: they keep their rows and stay searchable;
+ *     pbx_corpus_view_add on a detached view returns PBX_E_INVALID (pbx_corpus_view_drop still works).
+ *   - NULL out_view / view / parent, NULL ids with n > 0, n > PBX_MAX_ROWS, a view of a view, or view_add / view_drop on a
+ *     corpus that is not a view: PBX_E_INVALID.
+ * Cost: m rows take m * (pitch + 16.5) bytes of device memory, allocated as a corpus' are (whole 2 MB pages per array under
+ * CUDA virtual memory management), plus 8 bytes per id of the set on the device and on the host, plus the search scratch
+ * every corpus has.  Building a view is a host sort of the ids, one mark pass over the parent's ids (8 bytes per row, a
+ * binary search in the set per row) and a copy of the m rows on the device; pbx_corpus_view_add is the same over the ids
+ * new to the set; view_drop is a pbx_corpus_remove on the view.  Each parent append adds, per view, a mark pass over the
+ * appended rows and a copy of those that join; each parent remove or replace adds the same call on the view's m rows.
+ * A search costs a search over m rows. */
+PBX_API int pbx_corpus_view_create(pbx_corpus* parent, const int64_t* ids, uint64_t n, pbx_corpus** out_view);
+/* The set grows or shrinks: rows of the parent with an added id join the view (*out_rows_added, may be NULL, counts them;
+ * ids already in the set add nothing), rows with a dropped id leave it (*out_rows_dropped, may be NULL).  Atomic for
+ * searches on the view, as pbx_corpus_remove. */
+PBX_API int pbx_corpus_view_add(pbx_corpus* view, const int64_t* ids, uint64_t n, uint64_t* out_rows_added);
+PBX_API int pbx_corpus_view_drop(pbx_corpus* view, const int64_t* ids, uint64_t n, uint64_t* out_rows_dropped);
+
 /* Bench/test only: fills the shard on the device with rows [first_row, first_row + n) of the
  * counter-based synthetic corpus (pixelbox_b200/synth.py), image_id = global row + 1. */
 PBX_API int pbx_corpus_fill_synthetic(pbx_corpus* c, uint64_t n, uint64_t seed, uint64_t first_row);
@@ -300,6 +343,12 @@ PBX_API int pbx_sharded_remove(pbx_sharded* s, const int64_t* image_ids, uint64_
 /* pbx_corpus_replace over all shards, in the same way: every shard applies the whole request (one after the other,
  * atomic with respect to pbx_sharded_search); *out_replaced (may be NULL) is the total. */
 PBX_API int pbx_sharded_replace(pbx_sharded* s, const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint64_t* out_replaced);
+/* Views over a pbx_sharded: one view per shard, each of its own shard (ids are global), with pbx_corpus_view_create's
+ * contract.  Every pbx_sharded_search* accepts the result; pbx_sharded_load / _append / _remove / _replace /
+ * _fill_synthetic on it return PBX_E_INVALID; pbx_sharded_destroy destroys it.  The outputs of _add / _drop are totals. */
+PBX_API int pbx_sharded_view_create(pbx_sharded* parent, const int64_t* ids, uint64_t n, pbx_sharded** out_view);
+PBX_API int pbx_sharded_view_add(pbx_sharded* view, const int64_t* ids, uint64_t n, uint64_t* out_rows_added);
+PBX_API int pbx_sharded_view_drop(pbx_sharded* view, const int64_t* ids, uint64_t n, uint64_t* out_rows_dropped);
 /* Bench/test only: shard i holds rows [i * rows_per_shard, (i + 1) * rows_per_shard) of the synthetic corpus. */
 PBX_API int pbx_sharded_fill_synthetic(pbx_sharded* s, uint64_t rows_per_shard, uint64_t seed);
 PBX_API int pbx_sharded_size(const pbx_sharded* s, uint64_t* n_rows);

@@ -31,6 +31,8 @@ EXPORTS = [
     "pbx_corpus_create", "pbx_corpus_destroy", "pbx_corpus_load", "pbx_corpus_append", "pbx_corpus_flush", "pbx_corpus_append_device",
     "pbx_quantize_device", "pbx_corpus_fill_synthetic", "pbx_corpus_remove", "pbx_sharded_remove",
     "pbx_corpus_replace", "pbx_sharded_replace",
+    "pbx_corpus_view_create", "pbx_corpus_view_add", "pbx_corpus_view_drop",
+    "pbx_sharded_view_create", "pbx_sharded_view_add", "pbx_sharded_view_drop",
     "pbx_corpus_size", "pbx_corpus_dim", "pbx_corpus_read_rows", "pbx_corpus_synchronize", "pbx_search", "pbx_search_hits", "pbx_search_device",
     "pbx_search_filtered", "pbx_search_device_filtered", "pbx_sharded_search_filtered", "pbx_exchange_search_hits_filtered",
     "pbx_search_page", "pbx_search_device_page", "pbx_sharded_search_page", "pbx_exchange_search_hits_page",
@@ -89,6 +91,12 @@ def lib() -> ctypes.CDLL:
         "pbx_sharded_remove": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
         "pbx_corpus_replace": (i32, [vp, vp, u8p, u64, ctypes.POINTER(u64)]),
         "pbx_sharded_replace": (i32, [vp, vp, u8p, u64, ctypes.POINTER(u64)]),
+        "pbx_corpus_view_create": (i32, [vp, vp, u64, ctypes.POINTER(vp)]),
+        "pbx_corpus_view_add": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
+        "pbx_corpus_view_drop": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
+        "pbx_sharded_view_create": (i32, [vp, vp, u64, ctypes.POINTER(vp)]),
+        "pbx_sharded_view_add": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
+        "pbx_sharded_view_drop": (i32, [vp, vp, u64, ctypes.POINTER(u64)]),
         "pbx_corpus_size": (i32, [vp, ctypes.POINTER(u64)]),
         "pbx_corpus_dim": (i32, [vp, ctypes.POINTER(u32)]),
         "pbx_corpus_read_rows": (i32, [vp, u64, u64, vp, u8p]),

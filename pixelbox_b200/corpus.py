@@ -39,6 +39,7 @@ def _hits_results(hits: np.ndarray, cnt: np.ndarray) -> List[SearchResult]:
 
 
 def _remove(fn, handle, image_ids) -> int:
+    """fn(handle, ids, n, &rows): a call that takes a list of image ids and returns a row count."""
     ids = np.ascontiguousarray(np.asarray(image_ids, dtype=np.int64)).reshape(-1)
     removed = ctypes.c_uint64(0)
     nat.check(fn(handle, nat.ptr(ids), ids.size, ctypes.byref(removed)))
@@ -127,6 +128,29 @@ class Corpus:
 
     def fill_synthetic(self, n: int, seed: int, first_row: int = 0) -> None:
         nat.check(nat.lib().pbx_corpus_fill_synthetic(self._h, int(n), int(seed), int(first_row)))
+
+    # -- views -------------------------------------------------------------------------------
+    def view(self, image_ids) -> "Corpus":
+        """pbx_corpus_view_create: a Corpus holding a copy of this corpus' rows whose image_id is listed, kept current by
+        this corpus' append / remove / replace / load.  Its searches return what search(..., within=image_ids) returns
+        here, at the cost of the view's rows only.  The view is read-only (it follows this corpus); close() it when done.
+        It stays searchable if this corpus is closed first."""
+        ids = np.ascontiguousarray(np.asarray(image_ids, dtype=np.int64)).reshape(-1)
+        v = Corpus.__new__(Corpus)
+        v._h = ctypes.c_void_p(0)
+        v.dim, v.device = self.dim, self.device
+        nat.check(nat.lib().pbx_corpus_view_create(self._h, nat.ptr(ids), ids.size, ctypes.byref(v._h)))
+        v._tls = threading.local()
+        v._pbx_search = nat.lib().pbx_search
+        return v
+
+    def view_add(self, image_ids) -> int:
+        """pbx_corpus_view_add (on a view): the parent's rows of the listed ids join it; returns the rows added."""
+        return _remove(nat.lib().pbx_corpus_view_add, self._h, image_ids)
+
+    def view_drop(self, image_ids) -> int:
+        """pbx_corpus_view_drop (on a view): the rows of the listed ids leave it; returns the rows dropped."""
+        return _remove(nat.lib().pbx_corpus_view_drop, self._h, image_ids)
 
     def read_rows(self, first: int, n: int) -> Tuple[np.ndarray, np.ndarray]:
         ids = np.zeros(n, np.int64)
@@ -339,6 +363,23 @@ class MultiDeviceCorpus:
 
     def fill_synthetic(self, rows_per_shard: int, seed: int) -> None:
         nat.check(nat.lib().pbx_sharded_fill_synthetic(self._h, int(rows_per_shard), int(seed)))
+
+    def view(self, image_ids) -> "MultiDeviceCorpus":
+        """pbx_sharded_view_create: one view per shard (see Corpus.view); searched like this corpus."""
+        ids = np.ascontiguousarray(np.asarray(image_ids, dtype=np.int64)).reshape(-1)
+        v = MultiDeviceCorpus.__new__(MultiDeviceCorpus)
+        v._h = ctypes.c_void_p(0)
+        v.dim, v.devices = self.dim, list(self.devices)
+        nat.check(nat.lib().pbx_sharded_view_create(self._h, nat.ptr(ids), ids.size, ctypes.byref(v._h)))
+        return v
+
+    def view_add(self, image_ids) -> int:
+        """pbx_sharded_view_add (on a view): returns the rows added over all shards."""
+        return _remove(nat.lib().pbx_sharded_view_add, self._h, image_ids)
+
+    def view_drop(self, image_ids) -> int:
+        """pbx_sharded_view_drop (on a view): returns the rows dropped over all shards."""
+        return _remove(nat.lib().pbx_sharded_view_drop, self._h, image_ids)
 
     def shard_stats(self, index: int) -> nat.PbxStats:
         h = ctypes.c_void_p(0)

@@ -7,9 +7,12 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <iterator>
 #include <limits>
 #include <mutex>
 #include <new>
+#include <shared_mutex>
+#include <string>
 #include <type_traits>
 #include <vector>
 
@@ -18,6 +21,7 @@
 #include "remove.cuh"
 #include "replace.cuh"
 #include "page.cuh"
+#include "view.cuh"
 
 using namespace pbx;
 
@@ -242,10 +246,26 @@ struct pbx_corpus {
     uint64_t batched_queries = 0;
     bool scan_timed = false;          // ev_s0/ev_s1 were recorded by the last enqueue
     bool profiling = false;           // record CUDA events around the search / the scan (pbx_set_profiling)
+
+    // views (pbx_corpus_view_create).  A parent lists its views (guarded by its append_mu); a view names its parent (NULL
+    // once the parent is destroyed; guarded by g_view_mu) and keeps its id set, sorted and unique, on the host and on the
+    // device (guarded by the view's append_mu).  Lock order: the parent's locks, then the view's.
+    bool is_view = false;
+    pbx_corpus* parent = nullptr;
+    std::vector<pbx_corpus*> views;
+    std::vector<int64_t> view_set;
+    int64_t* d_view_set = nullptr;
+    size_t view_set_cap = 0;
 };
+
+static std::shared_mutex g_view_mu;   // view -> parent links: shared to follow one, exclusive to cut one
 
 constexpr size_t kStageMinRows = 2048;              // pinned upload staging: covers the coalesced blocks (kAppendBlock + kAppendCoalesceBelow rows)
 static int ensure_stage(pbx_corpus* c, size_t rows_per_slot);
+static int flush_pending(pbx_corpus* c);
+static int views_follow_append(pbx_corpus* c, uint64_t r0, uint64_t r1);
+static void views_reset(pbx_corpus* c);
+static int reject_view();
 
 static uint32_t default_keep(uint32_t k, uint32_t slack) {
     uint32_t s = slack ? slack : std::max<uint32_t>(156u, k / 4u);
@@ -612,6 +632,18 @@ extern "C" int pbx_corpus_create(uint32_t dim, uint64_t capacity_hint, int devic
 
 extern "C" void pbx_corpus_destroy(pbx_corpus* c) {
     if (!c) return;
+    {
+        // a parent's views are detached (they keep their rows and stay searchable); a view leaves its parent's list
+        std::unique_lock<std::shared_mutex> g(g_view_mu);
+        for (pbx_corpus* v : c->views) v->parent = nullptr;
+        c->views.clear();
+        if (c->parent) {
+            std::lock_guard<std::mutex> alk(c->parent->append_mu);
+            auto& l = c->parent->views;
+            l.erase(std::remove(l.begin(), l.end(), c), l.end());
+            c->parent = nullptr;
+        }
+    }
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     free_corpus_buffers(c);
@@ -620,6 +652,7 @@ extern "C" void pbx_corpus_destroy(pbx_corpus* c) {
     cudaFree(c->d_bhist); cudaFree(c->d_binvq); cudaFree(c->d_seedlb);
     cudaFree(c->d_hits); cudaFree(c->d_cand); cudaFree(c->d_cand_cnt); cudaFree(c->d_tile_counter); cudaFree(c->d_hist);
     cudaFree(c->d_allow); cudaFree(c->d_filter_words); cudaFree(c->d_filter_ids); cudaFree(c->d_cut); cudaFree(c->d_after);
+    cudaFree(c->d_view_set);
     cudaFreeHost(c->h_queries); cudaFreeHost(c->h_hits); cudaFreeHost(c->h_stage); cudaFreeHost(c->h_flag);
     if (c->ev_chain) cudaEventDestroy(c->ev_chain);
     if (c->ev_t0) cudaEventDestroy(c->ev_t0);
@@ -637,6 +670,10 @@ extern "C" void pbx_corpus_destroy(pbx_corpus* c) {
 
 extern "C" int pbx_corpus_size(const pbx_corpus* c, uint64_t* n_rows) {
     if (!c || !n_rows) return fail(PBX_E_INVALID, "NULL argument");
+    if (c->is_view) {       // the parent's pending appends that belong to the view join it when they are uploaded
+        int rc = flush_pending(const_cast<pbx_corpus*>(c));
+        if (rc != PBX_OK) return rc;
+    }
     *n_rows = c->n.load() + c->pending.load(std::memory_order_acquire);      // pending (coalesced) appends are part of the table
     return PBX_OK;
 }
@@ -740,7 +777,7 @@ static int append_locked(pbx_corpus* c, const int64_t* image_ids, const uint8_t*
     int rc = upload_rows(c, at, image_ids, hashes, n);
     if (rc != PBX_OK) return rc;
     c->n.store(at + n);
-    return PBX_OK;
+    return views_follow_append(c, at, at + n);
 }
 
 // Small appends (the indexer inserts one image at a time, src/engine.rs:186-203) are collected on the host and uploaded
@@ -751,14 +788,19 @@ constexpr uint64_t kAppendBlock = 1024;             // ... and uploaded when thi
 static int flush_pending_locked(pbx_corpus* c) {
     const uint64_t m = c->pend_ids.size();
     if (m == 0) return PBX_OK;
+    const uint64_t n0 = c->n.load();
     int rc = append_locked(c, c->pend_ids.data(), c->pend_rows.data(), m);
-    if (rc != PBX_OK) return rc;                    // the rows stay pending
+    if (rc != PBX_OK && c->n.load() == n0) return rc;   // the rows stay pending (not if only a view failed to follow)
     c->pend_ids.clear();
     c->pend_rows.clear();
     c->pending.store(0, std::memory_order_release);
-    return PBX_OK;
+    return rc;
 }
 static int flush_pending(pbx_corpus* c) {
+    if (c->is_view) {       // a view holds none of its own: its parent's pending rows join it when they are uploaded
+        std::shared_lock<std::shared_mutex> g(g_view_mu);
+        return c->parent ? flush_pending(c->parent) : PBX_OK;
+    }
     if (c->pending.load(std::memory_order_acquire) == 0) return PBX_OK;
     std::lock_guard<std::mutex> alk(c->append_mu);
     return flush_pending_locked(c);
@@ -766,6 +808,7 @@ static int flush_pending(pbx_corpus* c) {
 
 extern "C" int pbx_corpus_append(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n) {
     if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (c->is_view) return reject_view();
     if (n == 0) return PBX_OK;
     if (!image_ids || !hashes) return fail(PBX_E_INVALID, "NULL ids or hashes with n > 0");
     if (c->use_vmm) {
@@ -799,6 +842,7 @@ extern "C" int pbx_corpus_flush(pbx_corpus* c) {
 // stream and publishes them.
 extern "C" int pbx_corpus_append_device(pbx_corpus* c, const int64_t* d_image_ids, const uint8_t* d_hashes, uint64_t n, void* cuda_stream) {
     if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (c->is_view) return reject_view();
     if (n == 0) return PBX_OK;
     if (!d_image_ids || !d_hashes) return fail(PBX_E_INVALID, "NULL ids or hashes with n > 0");
     std::lock_guard<std::mutex> alk(c->append_mu);
@@ -825,11 +869,12 @@ extern "C" int pbx_corpus_append_device(pbx_corpus* c, const int64_t* d_image_id
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(s));
     c->n.store(at + n);
-    return PBX_OK;
+    return views_follow_append(c, at, at + n);
 }
 
 extern "C" int pbx_corpus_load(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n) {
     if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (c->is_view) return reject_view();
     if (n && (!image_ids || !hashes)) return fail(PBX_E_INVALID, "NULL ids or hashes with n > 0");
     std::lock_guard<std::mutex> alk(c->append_mu);  // held across the reset and the upload: no append can land in between
     {
@@ -838,18 +883,21 @@ extern "C" int pbx_corpus_load(pbx_corpus* c, const int64_t* image_ids, const ui
         CU_TRY(cudaDeviceSynchronize());
         c->n.store(0);
         c->pend_ids.clear(); c->pend_rows.clear(); c->pending.store(0);
+        views_reset(c);                             // the views are rebuilt from the new rows by the append below
     }
     return n ? append_locked(c, image_ids, hashes, n) : PBX_OK;
 }
 
 extern "C" int pbx_corpus_fill_synthetic(pbx_corpus* c, uint64_t n, uint64_t seed, uint64_t first_row) {
     if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (c->is_view) return reject_view();
     std::lock_guard<std::mutex> alk(c->append_mu);
     std::lock_guard<std::mutex> lk(c->mu);
     CU_TRY(cudaSetDevice(c->device));
     CU_TRY(cudaDeviceSynchronize());
     c->n.store(0);
     c->pend_ids.clear(); c->pend_rows.clear(); c->pending.store(0);
+    views_reset(c);
     int rc = c->use_vmm ? grow_mapped(c, std::max<uint64_t>(n, 1)) : reserve_rows(c, std::max<uint64_t>(n, 1));
     if (rc != PBX_OK) return rc;
     if (n == 0) return PBX_OK;
@@ -865,7 +913,7 @@ extern "C" int pbx_corpus_fill_synthetic(pbx_corpus* c, uint64_t n, uint64_t see
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(c->stream));
     c->n.store(n);
-    return PBX_OK;
+    return views_follow_append(c, 0, n);
 }
 
 extern "C" int pbx_corpus_read_rows(const pbx_corpus* cc, uint64_t first, uint64_t n, int64_t* image_ids, uint8_t* hashes) {
@@ -899,8 +947,8 @@ static int sorted_request(const int64_t* image_ids, uint64_t n, std::vector<int6
 // pbx_corpus_load does: the pending appends are flushed first, so they are subject to the removal; with mu held no search
 // can be enqueued, and the removal stream waits for the last one already enqueued (ev_chain: every search waits for its
 // predecessor, so for all of them) before it touches a row.  The new n is published after the stream is synchronised.
-static int remove_sorted(pbx_corpus* c, const std::vector<int64_t>& req, uint64_t* out_removed) {
-    std::lock_guard<std::mutex> alk(c->append_mu);
+// Caller holds append_mu.
+static int remove_sorted_locked(pbx_corpus* c, const std::vector<int64_t>& req, uint64_t* out_removed) {
     int rc = flush_pending_locked(c);
     if (rc != PBX_OK) return rc;
     std::lock_guard<std::mutex> lk(c->mu);
@@ -965,9 +1013,22 @@ static int remove_sorted(pbx_corpus* c, const std::vector<int64_t>& req, uint64_
     return PBX_OK;
 }
 
+// The removal, then the same request on every view (their own removal, under the parent's append lock: no parent change
+// can come in between).
+static int remove_sorted(pbx_corpus* c, const std::vector<int64_t>& req, uint64_t* out_removed) {
+    std::lock_guard<std::mutex> alk(c->append_mu);
+    int rc = remove_sorted_locked(c, req, out_removed);
+    for (size_t i = 0; rc == PBX_OK && i < c->views.size(); ++i) {
+        std::lock_guard<std::mutex> valk(c->views[i]->append_mu);
+        rc = remove_sorted_locked(c->views[i], req, nullptr);
+    }
+    return rc;
+}
+
 extern "C" int pbx_corpus_remove(pbx_corpus* c, const int64_t* image_ids, uint64_t n, uint64_t* out_removed) {
     if (out_removed) *out_removed = 0;
     if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (c->is_view) return reject_view();
     if (n && !image_ids) return fail(PBX_E_INVALID, "NULL image_ids with n > 0");
     if (n == 0) return PBX_OK;
     std::vector<int64_t> req;
@@ -1005,9 +1066,8 @@ static int replace_request(const int64_t* image_ids, const uint8_t* hashes, uint
 // Writes the request's hash into every row whose id it lists, in place (replace.cuh).  Locks and orders as remove_sorted:
 // the pending appends are flushed first, so they are subject to the replacement; with mu held no search can be enqueued,
 // and the stream waits for the last one already enqueued (ev_chain) before it touches a row.  Returns after the stream is
-// synchronised.  Positions, ids and n do not change.
-static int replace_sorted(pbx_corpus* c, const ReplaceRequest& req, uint64_t* out_replaced) {
-    std::lock_guard<std::mutex> alk(c->append_mu);
+// synchronised.  Positions, ids and n do not change.  Caller holds append_mu.
+static int replace_sorted_locked(pbx_corpus* c, const ReplaceRequest& req, uint64_t* out_replaced) {
     int rc = flush_pending_locked(c);
     if (rc != PBX_OK) return rc;
     std::lock_guard<std::mutex> lk(c->mu);
@@ -1070,14 +1130,225 @@ static int replace_sorted(pbx_corpus* c, const ReplaceRequest& req, uint64_t* ou
     return PBX_OK;
 }
 
+// The replacement, then the same request on every view, as remove_sorted: the view's rows get the same bytes and the
+// same row metadata kernel, so they stay the parent's bit for bit.
+static int replace_sorted(pbx_corpus* c, const ReplaceRequest& req, uint64_t* out_replaced) {
+    std::lock_guard<std::mutex> alk(c->append_mu);
+    int rc = replace_sorted_locked(c, req, out_replaced);
+    for (size_t i = 0; rc == PBX_OK && i < c->views.size(); ++i) {
+        std::lock_guard<std::mutex> valk(c->views[i]->append_mu);
+        rc = replace_sorted_locked(c->views[i], req, nullptr);
+    }
+    return rc;
+}
+
 extern "C" int pbx_corpus_replace(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n, uint64_t* out_replaced) {
     if (out_replaced) *out_replaced = 0;
     if (!c) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (c->is_view) return reject_view();
     if (n && (!image_ids || !hashes)) return fail(PBX_E_INVALID, "NULL ids or hashes with n > 0");
     if (n == 0) return PBX_OK;
     ReplaceRequest req;
     int rc = replace_request(image_ids, hashes, n, c->dim, c->pitch, &req);
     return rc == PBX_OK ? replace_sorted(c, req, out_replaced) : rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// views
+// ------------------------------------------------------------------------------------------------
+static int reject_view() {
+    return fail(PBX_E_INVALID, "the corpus is a view: it follows its parent and cannot be changed directly");
+}
+
+// Appends the rows of p's range [r0, r1) whose id is in d_set[0, n_set) (sorted, unique, device memory) behind v's rows,
+// in row order (view.cuh), then publishes them.  One host read: the number of rows.  Runs on p->copy_stream.  Caller
+// holds p->append_mu (p's rows and size stay put; they were published after their stream was synchronised) and
+// v->append_mu (v's size stays put).  As for an append, v's searches are not held: rows past its size are not read.
+static int view_collect(pbx_corpus* p, pbx_corpus* v, uint64_t r0, uint64_t r1, const int64_t* d_set, uint64_t n_set, uint64_t* out_added) {
+    if (out_added) *out_added = 0;
+    if (r1 <= r0 || n_set == 0) return PBX_OK;
+    CU_TRY(cudaSetDevice(p->device));
+    const uint64_t nr = r1 - r0, tiles = (nr + kMarkTileRows - 1) / kMarkTileRows, at = v->n.load();
+    cudaStream_t s = p->copy_stream;
+    // scratch, stream-ordered: [marked rows u64, listed rows u32][flag words][tile counts x 2], then the row list
+    const size_t off_flags = 16, off_tiles = off_flags + ((nr + 31) / 32 * sizeof(uint32_t) + 15) / 16 * 16;
+    unsigned char* scratch = nullptr;
+    uint32_t* list = nullptr;
+    CU_TRY(cudaMallocAsync(reinterpret_cast<void**>(&scratch), off_tiles + 2 * tiles * sizeof(uint32_t), s));
+    u64* d_marked = reinterpret_cast<u64*>(scratch);
+    uint32_t* d_listed = reinterpret_cast<uint32_t*>(scratch + 8);
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(scratch + off_flags);
+    uint32_t* d_tile_rows = reinterpret_cast<uint32_t*>(scratch + off_tiles);
+    uint32_t* d_tile_none = d_tile_rows + tiles;
+    u64 m = 0;
+    cudaError_t e = cudaMemsetAsync(d_marked, 0, sizeof(u64), s);
+    if (e == cudaSuccess) {
+        mark_ids_kernel<<<(unsigned)tiles, kMarkTileRows, 0, s>>>(p->d_ids + r0, nr, d_set, n_set, 0u, d_flags, d_marked);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&m, d_marked, sizeof(u64), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);        // the one synchronisation before the end: m sizes the rest
+    if (e == cudaSuccess && m > nr) { cudaFreeAsync(scratch, s); cudaStreamSynchronize(s); return fail(PBX_E_INTERNAL, "view marked %llu of %llu rows", (unsigned long long)m, (unsigned long long)nr); }
+    int rc = PBX_OK;
+    if (e == cudaSuccess && m && at + m > v->capacity) {
+        if (v->use_vmm) {
+            rc = grow_mapped(v, at + m);
+        } else {
+            std::lock_guard<std::mutex> lk(v->mu);      // growth moves the buffers: no search of the view may be running
+            rc = reserve_rows(v, at + m);
+        }
+    }
+    if (e == cudaSuccess && rc == PBX_OK && m) e = cudaMallocAsync(reinterpret_cast<void**>(&list), m * sizeof(uint32_t), s);
+    if (e == cudaSuccess && rc == PBX_OK && m) {
+        // remove.cuh's compaction with n_keep = nr: every marked row is a hole below it and nothing is a source above it
+        remove_count_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(d_flags, nr, nr, d_tile_rows, d_tile_none);
+        remove_scan_kernel<<<1, 1024, 0, s>>>(d_tile_rows, d_tile_none, (uint32_t)tiles, d_listed);
+        remove_place_kernel<<<(unsigned)tiles, kRemoveTileRows, 0, s>>>(d_flags, nr, nr, d_tile_rows, d_tile_none, list, nullptr);
+        const uint64_t chunks = m * v->pitch16;
+        const unsigned grid = (unsigned)std::min<uint64_t>((chunks + 255) / 256, (uint64_t)p->sm_count * 8);
+        view_gather_kernel<<<grid, 256, 0, s>>>(list, m, r0, v->pitch16, reinterpret_cast<const uint4*>(p->d_rows), p->d_ids, p->d_inv,
+                                                p->d_rsum, at, reinterpret_cast<uint4*>(v->d_rows), v->d_ids, v->d_inv, v->d_rsum);
+        // every block that holds one of the new rows (the first may be shared with the view's rows: its bound only widens)
+        const uint64_t b0 = at / 32, b1 = (at + m + 31) / 32;
+        block_meta_kernel<<<(unsigned)((b1 - b0 + 7) / 8), 256, 0, s>>>(v->d_inv, v->d_rsum, v->dim, b0, b1 - b0, at + m, v->d_bmeta);
+        e = cudaGetLastError();
+    }
+    if (list) cudaFreeAsync(list, s);
+    cudaFreeAsync(scratch, s);
+    const cudaError_t e2 = cudaStreamSynchronize(s);
+    if (e == cudaSuccess) e = e2;
+    if (rc != PBX_OK) return rc;
+    if (e != cudaSuccess) return fail(PBX_E_CUDA, "view update failed: %s", cudaGetErrorString(e));
+    v->n.store(at + m);
+    if (out_added) *out_added = m;
+    return PBX_OK;
+}
+
+// The view's set on the device, after a change on the host.  Caller holds v->append_mu; nothing of the view is in flight
+// (every view update synchronises before it returns).
+static int view_upload_set(pbx_corpus* v) {
+    const size_t n = v->view_set.size();
+    CU_TRY(cudaSetDevice(v->device));
+    if (n > v->view_set_cap) {
+        const size_t want = std::max(n, v->view_set_cap + v->view_set_cap / 2);
+        cudaFree(v->d_view_set); v->d_view_set = nullptr; v->view_set_cap = 0;
+        CU_TRY(cudaMalloc(&v->d_view_set, want * sizeof(int64_t)));
+        v->view_set_cap = want;
+    }
+    if (n) CU_TRY(cudaMemcpy(v->d_view_set, v->view_set.data(), n * sizeof(int64_t), cudaMemcpyHostToDevice));
+    return PBX_OK;
+}
+
+// Rows [r0, r1) of c were just published: each view takes those whose id is in its set.  Caller holds c->append_mu.
+static int views_follow_append(pbx_corpus* c, uint64_t r0, uint64_t r1) {
+    for (pbx_corpus* v : c->views) {
+        std::lock_guard<std::mutex> valk(v->append_mu);
+        int rc = view_collect(c, v, r0, r1, v->d_view_set, v->view_set.size(), nullptr);
+        if (rc != PBX_OK) return rc;
+    }
+    return PBX_OK;
+}
+
+// c's contents are being discarded (load, fill_synthetic): every view is emptied, and follows the new rows as they are
+// published.  Caller holds c->append_mu and c->mu and has synchronised the device.
+static void views_reset(pbx_corpus* c) {
+    for (pbx_corpus* v : c->views) {
+        std::lock_guard<std::mutex> valk(v->append_mu);
+        std::lock_guard<std::mutex> vlk(v->mu);
+        v->n.store(0);
+    }
+}
+
+extern "C" int pbx_corpus_view_create(pbx_corpus* parent, const int64_t* ids, uint64_t n, pbx_corpus** out_view) {
+    if (!out_view) return fail(PBX_E_INVALID, "out_view is NULL");
+    *out_view = nullptr;
+    if (!parent) return fail(PBX_E_INVALID, "parent is NULL");
+    if (parent->is_view) return fail(PBX_E_INVALID, "the parent is a view: make the view of its parent instead");
+    if (n && !ids) return fail(PBX_E_INVALID, "NULL ids with n > 0");
+    if (n > PBX_MAX_ROWS) return fail(PBX_E_INVALID, "view of %llu ids (max %llu)", (unsigned long long)n, (unsigned long long)PBX_MAX_ROWS);
+    std::vector<int64_t> set;
+    if (n) { int rc0 = sorted_request(ids, n, &set); if (rc0 != PBX_OK) return rc0; }
+    std::unique_lock<std::mutex> alk(parent->append_mu);
+    int rc = flush_pending_locked(parent);
+    if (rc != PBX_OK) return rc;
+    // sized for one row per id (ids are unique in the table the corpus caches); more rows grow it
+    pbx_corpus* v = nullptr;
+    rc = pbx_corpus_create(parent->dim, std::min<uint64_t>(parent->n.load(), set.size()), parent->device, &v);
+    if (rc != PBX_OK) return rc;
+    v->is_view = true;
+    v->view_set = std::move(set);
+    rc = view_upload_set(v);
+    if (rc == PBX_OK) {
+        std::lock_guard<std::mutex> valk(v->append_mu);
+        rc = view_collect(parent, v, 0, parent->n.load(), v->d_view_set, v->view_set.size(), nullptr);
+    }
+    if (rc == PBX_OK) {
+        try { parent->views.push_back(v); } catch (...) { rc = fail(PBX_E_OOM, "host allocation failed"); }
+    }
+    if (rc != PBX_OK) {
+        alk.unlock();                               // destroy takes g_view_mu, which comes before the parent's locks
+        const std::string err = g_err;              // destroy may overwrite the message
+        pbx_corpus_destroy(v);                      // not linked: touches nothing of the parent
+        return fail(rc, "%s", err.c_str());
+    }
+    v->parent = parent;
+    *out_view = v;
+    return PBX_OK;
+}
+
+extern "C" int pbx_corpus_view_add(pbx_corpus* v, const int64_t* ids, uint64_t n, uint64_t* out_rows_added) {
+    if (out_rows_added) *out_rows_added = 0;
+    if (!v) return fail(PBX_E_INVALID, "view is NULL");
+    if (!v->is_view) return fail(PBX_E_INVALID, "the corpus is not a view");
+    if (n && !ids) return fail(PBX_E_INVALID, "NULL ids with n > 0");
+    if (n > PBX_MAX_ROWS) return fail(PBX_E_INVALID, "%llu ids (max %llu)", (unsigned long long)n, (unsigned long long)PBX_MAX_ROWS);
+    std::vector<int64_t> req;
+    if (n) { int rc0 = sorted_request(ids, n, &req); if (rc0 != PBX_OK) return rc0; }
+    std::shared_lock<std::shared_mutex> g(g_view_mu);
+    pbx_corpus* p = v->parent;
+    if (!p) return fail(PBX_E_INVALID, "the view's parent was destroyed: a detached view cannot take new ids");
+    if (req.empty()) return PBX_OK;
+    std::lock_guard<std::mutex> alk(p->append_mu);
+    int rc = flush_pending_locked(p);
+    if (rc != PBX_OK) return rc;
+    std::lock_guard<std::mutex> valk(v->append_mu);
+    // only ids new to the set bring rows: the rows of the others are in the view already
+    std::vector<int64_t> fresh, merged;
+    try {
+        std::set_difference(req.begin(), req.end(), v->view_set.begin(), v->view_set.end(), std::back_inserter(fresh));
+        if (fresh.empty()) return PBX_OK;
+        std::merge(v->view_set.begin(), v->view_set.end(), fresh.begin(), fresh.end(), std::back_inserter(merged));
+    } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
+    CU_TRY(cudaSetDevice(p->device));
+    int64_t* d_fresh = nullptr;
+    CU_TRY(cudaMallocAsync(reinterpret_cast<void**>(&d_fresh), fresh.size() * sizeof(int64_t), p->copy_stream));
+    cudaError_t e = cudaMemcpyAsync(d_fresh, fresh.data(), fresh.size() * sizeof(int64_t), cudaMemcpyHostToDevice, p->copy_stream);
+    rc = e == cudaSuccess ? view_collect(p, v, 0, p->n.load(), d_fresh, fresh.size(), out_rows_added)
+                          : fail(PBX_E_CUDA, "view id upload failed: %s", cudaGetErrorString(e));
+    cudaFreeAsync(d_fresh, p->copy_stream);
+    cudaStreamSynchronize(p->copy_stream);
+    if (rc != PBX_OK) return rc;
+    v->view_set.swap(merged);
+    return view_upload_set(v);
+}
+
+extern "C" int pbx_corpus_view_drop(pbx_corpus* v, const int64_t* ids, uint64_t n, uint64_t* out_rows_dropped) {
+    if (out_rows_dropped) *out_rows_dropped = 0;
+    if (!v) return fail(PBX_E_INVALID, "view is NULL");
+    if (!v->is_view) return fail(PBX_E_INVALID, "the corpus is not a view");
+    if (n && !ids) return fail(PBX_E_INVALID, "NULL ids with n > 0");
+    if (n == 0) return PBX_OK;
+    std::vector<int64_t> req, kept;
+    int rc = sorted_request(ids, n, &req);
+    if (rc != PBX_OK) return rc;
+    std::lock_guard<std::mutex> valk(v->append_mu);
+    try {
+        std::set_difference(v->view_set.begin(), v->view_set.end(), req.begin(), req.end(), std::back_inserter(kept));
+    } catch (...) { return fail(PBX_E_OOM, "host allocation failed"); }
+    rc = remove_sorted_locked(v, req, out_rows_dropped);
+    if (rc != PBX_OK) return rc;
+    v->view_set.swap(kept);
+    return view_upload_set(v);
 }
 
 // ------------------------------------------------------------------------------------------------

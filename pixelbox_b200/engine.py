@@ -74,6 +74,7 @@ class Engine:
         self.cached_search_results: Optional[List[IndexedImage]] = None
         self._last_query: Optional[dict] = None                          # load_more_results continues it
         self.corpus: Optional[Corpus] = None
+        self.folder_views: Dict[str, Corpus] = {}                         # folder prefix -> view of its images' rows
         self.skipped_rows = 0
         self._load_corpus()
 
@@ -120,6 +121,9 @@ class Engine:
         self.corpus.load(ids, hashes)
 
     def close(self) -> None:
+        for v in self.folder_views.values():
+            v.close()
+        self.folder_views.clear()
         if self.corpus is not None:
             self.corpus.close()
             self.corpus = None
@@ -143,8 +147,10 @@ class Engine:
     def query_by_image_hash_within_folder(self, indexed_image: IndexedImage, folder: str) -> None:
         """query_by_image_hash_from_image restricted to the images under `folder`: the similarity SQL with
         `AND substr(images.path, 1, length(?)) = ?` added (folder with a trailing separator, so that /a/b does not match
-        /a/bc; no LIKE, whose % and _ occur in real paths).  The folder's ids come from `images`; a row deleted between
-        the id query and the search is dropped by the join like any other hash without an image row."""
+        /a/bc; no LIKE, whose % and _ occur in real paths).  The folder's ids come from `images` on the folder's first
+        query; they are kept, with the folder's rows, in a view of the corpus (Corpus.view) that insert_image_from_memory
+        and remove_images keep current, so later queries of the folder cost its rows, not the table's.  A hash without an
+        image row is dropped by the join like any other."""
         self._similarity_query(indexed_image, folder)
 
     def load_more_results(self, count: int = DEFAULT_MAX_SEARCH_RESULTS) -> None:
@@ -168,14 +174,19 @@ class Engine:
         t0 = time.perf_counter()
         results: List[IndexedImage] = []
         if self.corpus is not None:
-            within = None
+            corpus = self.corpus
             if folder is not None:
+                # the folder's rows are kept as a view of the corpus, made on first use: its searches cost the folder's
+                # rows, not the table's, and the corpus keeps it current as hashes are appended, removed or replaced
                 prefix = folder if folder.endswith(("/", "\\")) else folder + "/"
-                within = np.fromiter((r[0] for r in self.read_connection.execute(
-                    "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
-            # what load_more_results continues from: the query, its max_dist and folder, the last GPU row consumed
+                corpus = self.folder_views.get(prefix)
+                if corpus is None:
+                    ids = np.fromiter((r[0] for r in self.read_connection.execute(
+                        "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
+                    corpus = self.folder_views[prefix] = self.corpus.view(ids)
+            # what load_more_results continues from: the query, its max_dist and folder's view, the last GPU row consumed
             self._last_query = dict(query=np.frombuffer(indexed_image.visual_hash, np.uint8), max_dist=self.max_distance_from_query,
-                                    within=within, cursor=None, exhausted=False)
+                                    corpus=corpus, cursor=None, exhausted=False)
             results = self._joined_rows(DEFAULT_MAX_SEARCH_RESULTS)                  # LIMIT 100, :381
         self.cached_search_results = results
         sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(results)}\n")
@@ -188,7 +199,7 @@ class Engine:
         out: List[IndexedImage] = []
         while len(out) < count and not st["exhausted"]:
             after = None if st["cursor"] is None else [st["cursor"]]
-            res = self.corpus.search(st["query"], DEFAULT_MAX_SEARCH_RESULTS, st["max_dist"], within=st["within"], after=after)[0]
+            res = st["corpus"].search(st["query"], DEFAULT_MAX_SEARCH_RESULTS, st["max_dist"], after=after)[0]
             for image_id, dist in zip(res.ids, res.dist):
                 st["cursor"] = (dist, int(image_id))
                 row = self.read_connection.execute(self._JOIN_SQL, (int(image_id),)).fetchone()
@@ -215,8 +226,8 @@ class Engine:
         conn = self.write_connection
         appended = None
         try:
-            conn.execute("INSERT OR IGNORE INTO images (filename, path, image_width, image_height, thumbnail) VALUES (?, ?, ?, ?, ?)",
-                         (img.filename, img.path, img.resolution[0], img.resolution[1], img.thumbnail))
+            new_image = conn.execute("INSERT OR IGNORE INTO images (filename, path, image_width, image_height, thumbnail) VALUES (?, ?, ?, ?, ?)",
+                                     (img.filename, img.path, img.resolution[0], img.resolution[1], img.thumbnail)).rowcount == 1
             img.id = conn.execute("SELECT last_insert_rowid()").fetchone()[0]
             if img.visual_hash is not None:
                 cur = conn.execute("INSERT OR IGNORE INTO semantic_hashes (image_id, hash) VALUES (?, ?)", (img.id, img.visual_hash))
@@ -226,6 +237,12 @@ class Engine:
         except Exception:
             conn.rollback()
             raise
+        # a new image is in the folders that prefix its path: its id joins their views (before the append, which the
+        # views then follow)
+        if new_image:
+            for prefix, v in self.folder_views.items():
+                if img.path[:len(prefix)] == prefix:
+                    v.view_add(np.array([img.id], np.int64))
         # the device corpus is a cache of the committed table: append only what the DB now holds
         if appended is not None:
             if self.corpus is None:
@@ -253,9 +270,12 @@ class Engine:
         except Exception:
             conn.rollback()
             raise
-        # as for inserts, the device corpus follows only what has been committed
+        # as for inserts, the device corpus follows only what has been committed; its folder views follow the removal.
+        # The ids also leave the views' sets: SQLite may give a deleted rowid to an image indexed later, elsewhere.
         if self.corpus is not None:
             self.corpus.remove(np.asarray(ids, np.int64))
+        for v in self.folder_views.values():
+            v.view_drop(np.asarray(ids, np.int64))
 
     def update_image_hashes(self, pairs) -> None:
         """`UPDATE semantic_hashes SET hash = ? WHERE image_id = ?` for every (image_id, hash) pair, in order, in one

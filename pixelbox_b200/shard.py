@@ -124,6 +124,29 @@ class ShardedCorpus:
         mine = np.array([self.local.replace(image_ids, hashes)], np.int64)
         return int(self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).sum())
 
+    def view(self, image_ids) -> "ShardedCorpus":
+        """A ShardedCorpus over a view of every rank's shard (Corpus.view; every rank passes the same global ids).  It shares
+        this corpus' process group and exchange, so its searches are the same collective calls with the same results as
+        search(..., within=image_ids) here, at the cost of the view's rows.  close() it before this corpus."""
+        if not isinstance(self.local, Corpus):
+            raise nat.PbxError(-1, "a view needs GPU shards")
+        v = ShardedCorpus.__new__(ShardedCorpus)
+        v.__dict__.update(self.__dict__)
+        v.local = self.local.view(image_ids)
+        v._bufs = {}
+        v._view_of = self
+        return v
+
+    def view_add(self, image_ids) -> int:
+        """Corpus.view_add on every rank's view; returns the rows added over all ranks, on every rank."""
+        mine = np.array([self.local.view_add(image_ids)], np.int64)
+        return int(self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).sum())
+
+    def view_drop(self, image_ids) -> int:
+        """Corpus.view_drop on every rank's view; returns the rows dropped over all ranks, on every rank."""
+        mine = np.array([self.local.view_drop(image_ids)], np.int64)
+        return int(self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).sum())
+
     def total_rows(self) -> int:
         t = torch.tensor([len(self.local)], dtype=torch.int64, device=self._comm_dev())
         dist.all_reduce(t, group=self.group)
@@ -252,6 +275,9 @@ class ShardedCorpus:
                              hits[i]["dot"][:cnt[i]].copy(), hits[i]["norm2"][:cnt[i]].copy()) for i in range(nq)]
 
     def close(self) -> None:
+        if getattr(self, "_view_of", None) is not None:     # a view: the exchange belongs to the corpus it views
+            self.local.close()
+            return
         if self._exchange is not None:
             torch.cuda.synchronize()
             dist.barrier(group=self.group)                 # nobody may still be writing into a mailbox that goes away
