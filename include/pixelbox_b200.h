@@ -116,7 +116,9 @@ PBX_API int pbx_corpus_load(pbx_corpus* c, const int64_t* image_ids, const uint8
 PBX_API int pbx_corpus_append(pbx_corpus* c, const int64_t* image_ids, const uint8_t* hashes, uint64_t n);
 /* Appends of fewer than 64 rows are collected on the host and uploaded 1024 at a time (the writer loop inserts one image
  * at a time); they count as part of the table at once: pbx_corpus_size includes them and every search uploads them before
- * it runs.  pbx_corpus_flush uploads them now.  The shard grows by mapping more device memory behind its arrays (CUDA
+ * it runs.  pbx_corpus_flush uploads them now.  An append that would take the shard (pending rows included) past
+ * PBX_MAX_ROWS rows, or past the rows its address range was reserved for, returns PBX_E_CAPACITY and changes nothing,
+ * coalesced or not.  The shard grows by mapping more device memory behind its arrays (CUDA
  * virtual memory management): no copy, no moved pointer, searches keep running while it grows. */
 PBX_API int pbx_corpus_flush(pbx_corpus* c);
 /* The same for rows that are already in device memory on the corpus' device (e.g. produced by pbx_quantize_device):

@@ -820,6 +820,12 @@ extern "C" int pbx_corpus_append(pbx_corpus* c, const int64_t* image_ids, const 
     }
     std::lock_guard<std::mutex> alk(c->append_mu);
     if (n < kAppendCoalesceBelow) {
+        // Refuse here what the upload would refuse later: rows queued past the shard's limit would stay pending for good,
+        // and every later search, removal, replacement and read would fail on them.
+        const uint64_t limit = c->use_vmm ? c->reserved_rows : PBX_MAX_ROWS;
+        if (c->n.load() + c->pend_ids.size() + n > limit)
+            return fail(PBX_E_CAPACITY, "shard would hold %llu rows (max %llu)",
+                        (unsigned long long)(c->n.load() + c->pend_ids.size() + n), (unsigned long long)limit);
         try {
             c->pend_ids.insert(c->pend_ids.end(), image_ids, image_ids + n);
             c->pend_rows.insert(c->pend_rows.end(), hashes, hashes + n * c->dim);

@@ -6,6 +6,7 @@ import pytest
 from oracle import oracle
 from pixelbox_b200 import synth
 from pixelbox_b200.corpus import Corpus
+from tests import synth_oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -122,11 +123,10 @@ def test_batched_bound_with_wild_norm_spread_and_negative_thresholds(d, n):
 
 
 def test_full_size_10m_batch_of_1024_properties():
-    """BASELINE configs[2] at full size (10M x 256, 1024 queries, top-100) through the tensor-core path: too big for an oracle pass
-    over the corpus, so size-independent properties on a spread of the queries: planted self-matches lead with the reference's
-    self-distance, the returned rows re-rank identically under the oracle (ids, order, distance bits, integer terms), and in
-    a random 100k-row stripe per checked query no row beats the k-th hit without being in the answer (nothing was missed);
-    the same 16 queries through the single-query path give the same answers."""
+    """BASELINE configs[2] at full size (10M x 256, 1024 queries, top-100) through the tensor-core path, every query checked in
+    full against the complete reference of the synthetic corpus (tests/synth_oracle.py): ids, order, distance bits, integer
+    terms.  Planted self-matches lead with the reference's self-distance; 16 of the queries through the single-query path
+    give the same answers."""
     n, d, k, nq, seed = 10_000_000, 256, 100, 1024, 42
     with Corpus(d, capacity_hint=n) as c:
         c.fill_synthetic(n, seed, 0)
@@ -137,25 +137,17 @@ def test_full_size_10m_batch_of_1024_properties():
         before = c.stats().batched_queries
         res = c.search(queries, k)
         assert c.stats().batched_queries == before + nq, "the tensor-core path did not run"
-        rng = np.random.default_rng(8)
-        checked = sorted(set(probes) | set(int(x) for x in rng.integers(0, nq, 13)))
-        for qi in checked:
-            r = res[qi]
+        want = synth_oracle.SynthReference(n, seed, d, 0, device="cuda").topk(queries, k)
+        for qi in range(nq):
+            r, (o_ids, o_dist, o_dot, o_n2) = res[qi], want[qi]
             assert len(r.ids) == k
-            rows = np.concatenate([synth.synth_rows(seed, int(i) - 1, 1, d) for i in r.ids])
-            o_ids, o_dist, o_dot, o_n2 = oracle.topk(rows, r.ids, queries[qi], k, 1e3)
-            assert list(r.ids) == list(o_ids) and np.array_equal(bits(r.dist), bits(o_dist)), f"q{qi}: returned rows re-rank differently"
+            assert list(r.ids) == list(o_ids) and np.array_equal(bits(r.dist), bits(o_dist)), f"q{qi}: differs from the reference"
             assert np.array_equal(r.dot, o_dot) and np.array_equal(r.norm2, o_n2)
             if qi in probes:
                 assert r.ids[0] == probes[qi] + 1
                 assert bits(r.dist[0]) == bits(oracle.cosine_distance(queries[qi], queries[qi]))
-            s0 = int(rng.integers(0, n - 100_000))
-            stripe = synth.synth_rows(seed, s0, 100_000, d)
-            s_ids = np.arange(s0 + 1, s0 + 100_001, dtype=np.int64)
-            t_ids, t_dist, _, _ = oracle.topk(stripe, s_ids, queries[qi], k, 1e3, threads=oracle.max_threads())
-            kth, have = (float(r.dist[-1]), int(r.ids[-1])), set(int(x) for x in r.ids)
-            for i, dd in zip(t_ids, t_dist):
-                assert not ((float(dd), int(i)) < kth) or int(i) in have, f"stripe row {i} (dist {dd}) missing from q{qi}"
+        rng = np.random.default_rng(8)
+        checked = sorted(set(probes) | set(int(x) for x in rng.integers(0, nq, 13)))
         c.set_batch_min(0xFFFFFFFF)
         single = c.search(queries[checked], k)
         for qi, b in zip(checked, single):
