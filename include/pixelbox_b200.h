@@ -311,6 +311,29 @@ PBX_API int pbx_search_device_page(pbx_corpus* c, const uint8_t* d_queries, uint
                                    const pbx_hit* d_after, const int64_t* d_filter_ids, uint64_t n_filter, uint32_t filter_mode,
                                    pbx_hit* d_hits, uint32_t* d_count, void* cuda_stream);
 
+/* ---- range search: every row within max_dist, and its exact count ------------------------------------------------------
+ * Replaces: the similarity query without its LIMIT ("every copy of this photo", "everything inside max_distance"), and
+ * its COUNT(*):
+ *   SELECT image_id, cosine_distance(?, hash) AS dist FROM semantic_hashes WHERE dist < :max_dist
+ *   [AND (dist > :d0 OR (dist = :d0 AND image_id > :id0))]  [AND image_id IN / NOT IN (...)]  ORDER BY dist ASC, image_id ASC
+ *   - after (NULL or [nq] cursors) and the filter triple as in pbx_search_page (same argument rules; a NaN cursor dist is
+ *     PBX_E_INVALID).  max_dist is compared as the f64 `dist < max_dist`: NaN gives no row; above 999999 every row is
+ *     inside, the plateau rows ordered by image_id; a row at dist -1.19e-7 (an identical row) is inside even at max_dist 0.
+ *   - out_total[q] is always the exact COUNT(*) of query q, whatever the capacity.
+ *   - Rows are written query after query, each query's rows in order, until `capacity` rows are written: query q's rows
+ *     are out_hits[out_offsets[q] .. out_offsets[q + 1]), a prefix of its answer (out_offsets has nq + 1 entries).  A query
+ *     whose answer was cut continues with the same call and after = its last written row.
+ *   - capacity = 0 counts only (out_hits may be NULL); NULL out_offsets / out_total, or NULL out_hits with capacity > 0,
+ *     is PBX_E_INVALID.
+ *   - Records carry dist bit for bit, dot and norm2, as the top-k records do (flags = 0).
+ *   - Ordered like any search of the corpus (the previous search's kernels, pending appends uploaded first): a range
+ *     search sees all of a removal or replacement or none of it.  A view (pbx_corpus_view_create) is searched like a corpus.
+ * Cost: one streaming pass per query, plus the exact replay of the rows near max_dist (count only) or of the answer and a
+ * sort that grows with it.  A host call: it reads the candidate count of each query once, and its result. */
+PBX_API int pbx_search_range(pbx_corpus* c, const uint8_t* queries, uint32_t nq, double max_dist, const pbx_hit* after,
+                             const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode, pbx_hit* out_hits, uint64_t capacity,
+                             uint64_t* out_offsets, uint64_t* out_total);
+
 /* Merge step after the all-gather (SURVEY.md section 8e): gathered is [n_shards][nq][k] hits and
  * counts is [n_shards][nq], both in HOST memory; every shard list is already ordered by
  * (dist, image_id).  Writes the global first k per query under the same order.  Pure host
@@ -372,6 +395,11 @@ PBX_API int pbx_sharded_search_filtered(pbx_sharded* s, const uint8_t* queries, 
 PBX_API int pbx_sharded_search_page(pbx_sharded* s, const uint8_t* queries, uint32_t nq, uint32_t k, double max_dist,
                                     const pbx_hit* after, const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode,
                                     pbx_hit* out_hits, uint32_t* out_count);
+/* pbx_search_range over all shards, same arguments and contract: every shard runs the range search of its rows, the root
+ * device gathers each shard's first min(total, capacity) rows and orders them; the totals are summed. */
+PBX_API int pbx_sharded_search_range(pbx_sharded* s, const uint8_t* queries, uint32_t nq, double max_dist, const pbx_hit* after,
+                                     const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode, pbx_hit* out_hits,
+                                     uint64_t capacity, uint64_t* out_offsets, uint64_t* out_total);
 
 /* ---- the exchange step over NVLink peer memory (one process per GPU) ---------------------------------
  * Replaces: nothing upstream (PixelBox is single-process); it is the one exchange step of the row-sharded path

@@ -36,6 +36,7 @@ EXPORTS = [
     "pbx_corpus_size", "pbx_corpus_dim", "pbx_corpus_read_rows", "pbx_corpus_synchronize", "pbx_search", "pbx_search_hits", "pbx_search_device",
     "pbx_search_filtered", "pbx_search_device_filtered", "pbx_sharded_search_filtered", "pbx_exchange_search_hits_filtered",
     "pbx_search_page", "pbx_search_device_page", "pbx_sharded_search_page", "pbx_exchange_search_hits_page",
+    "pbx_search_range", "pbx_sharded_search_range",
     "pbx_merge_hits", "pbx_merge_hits_device", "pbx_exchange_create", "pbx_exchange_handle", "pbx_exchange_connect",
     "pbx_exchange_allgather_merge", "pbx_exchange_search_hits", "pbx_exchange_destroy",
     "pbx_sharded_create", "pbx_sharded_destroy", "pbx_sharded_load", "pbx_sharded_append", "pbx_sharded_fill_synthetic", "pbx_sharded_size",
@@ -108,6 +109,8 @@ def lib() -> ctypes.CDLL:
         "pbx_search_device_filtered": (i32, [vp, vp, u32, u32, f64, vp, vp, vp, vp, u64, u32]),
         "pbx_search_page": (i32, [vp, u8p, u32, u32, f64, vp, vp, u64, u32, vp, vp]),
         "pbx_search_device_page": (i32, [vp, vp, u32, u32, f64, vp, vp, u64, u32, vp, vp, vp]),
+        "pbx_search_range": (i32, [vp, u8p, u32, f64, vp, vp, u64, u32, vp, u64, vp, vp]),
+        "pbx_sharded_search_range": (i32, [vp, u8p, u32, f64, vp, vp, u64, u32, vp, u64, vp, vp]),
         "pbx_merge_hits": (i32, [vp, vp, u32, u32, u32, vp, vp]),
         "pbx_merge_hits_device": (i32, [i32, vp, vp, u32, u32, u32, vp, vp, vp]),
         "pbx_exchange_create": (i32, [i32, u32, u32, u32, u32, ctypes.POINTER(vp)]),

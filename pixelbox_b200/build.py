@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 SO = os.path.join(LIBDIR, "libpixelbox_b200.so")
-SOURCES = ["api.cu"]
+SOURCES = ["api.cu", "range_sort.cu"]
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh")) + [os.path.join("..", "..", "include", "pixelbox_b200.h")]
 
 NVCC_FLAGS = [

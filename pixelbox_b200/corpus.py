@@ -21,6 +21,15 @@ class SearchResult(NamedTuple):
     norm2: np.ndarray   # int32: sum c(r)^2
 
 
+class RangeResult(NamedTuple):
+    """The rows of one query within max_dist, ordered by (dist asc, image_id asc), and the exact count of all of them."""
+    ids: np.ndarray     # int64
+    dist: np.ndarray    # float32, bit for bit
+    dot: np.ndarray     # int32
+    norm2: np.ndarray   # int32
+    total: int          # COUNT(*) of the rows within max_dist (after the cursor, within the filter): >= len(ids)
+
+
 def _as_u8_2d(a, dim: int, what: str) -> np.ndarray:
     a = np.ascontiguousarray(np.asarray(a, dtype=np.uint8))
     if a.ndim == 1:
@@ -54,6 +63,54 @@ def _replace(fn, handle, dim, image_ids, hashes) -> int:
     replaced = ctypes.c_uint64(0)
     nat.check(fn(handle, nat.ptr(ids), nat.ptr(hashes), ids.size, ctypes.byref(replaced)))
     return int(replaced.value)
+
+
+def _search_range(fn, handle, dim: int, size, queries, max_dist, limit, within, excluding, after) -> List[RangeResult]:
+    """pbx_search_range / pbx_sharded_search_range (fn), one call per query.  limit = rows wanted per query (None: all of
+    them; an answer cut short by rows appended meanwhile is continued from its last row)."""
+    fids, mode = nat.page_filter_args(within, excluding)
+    q = _as_u8_2d(queries, dim, "search_range")
+    nq = q.shape[0]
+    cur = None if after is None else nat.page_cursors(after, nq)
+    if limit is not None and int(limit) < 0:
+        raise ValueError("limit must be >= 0")
+    out = []
+    offsets = np.zeros(2, np.uint64)
+    total = np.zeros(1, np.uint64)
+    for i in range(nq):
+        cursor = None if cur is None else cur[i:i + 1].copy()
+        parts = []
+        want = None if limit is None else int(limit)
+        first_total = None
+        while True:
+            cap = size() if want is None else want
+            hits = np.empty(cap, nat.HIT_DTYPE)
+            nat.check(fn(handle, nat.ptr(q[i:i + 1]), 1, float(max_dist), nat.ptr(cursor), nat.ptr(fids), fids.size, mode,
+                         nat.ptr(hits) if cap else None, cap, nat.ptr(offsets), nat.ptr(total)))
+            got = hits[:int(offsets[1])]
+            parts.append(got)
+            if first_total is None:
+                first_total = int(total[0])
+            if want is not None or len(got) == int(total[0]) or len(got) == 0:
+                break
+            cursor = got[-1:].copy()                   # rows appended since size() was read: continue after the last row
+        rows = np.concatenate(parts) if len(parts) > 1 else parts[0]
+        out.append(RangeResult(rows["image_id"].copy(), rows["dist"].copy(), rows["dot"].copy(), rows["norm2"].copy(),
+                               max(first_total, len(rows))))
+    return out
+
+
+def _count_within(fn, handle, dim: int, queries, max_dist, within, excluding, after) -> np.ndarray:
+    """The exact counts of pbx_search_range with capacity 0, one per query (uint64)."""
+    fids, mode = nat.page_filter_args(within, excluding)
+    q = _as_u8_2d(queries, dim, "count_within")
+    nq = q.shape[0]
+    cur = None if after is None else nat.page_cursors(after, nq)
+    offsets = np.zeros(nq + 1, np.uint64)
+    total = np.zeros(nq, np.uint64)
+    nat.check(fn(handle, nat.ptr(q), nq, float(max_dist), nat.ptr(cur), nat.ptr(fids), fids.size, mode, None, 0,
+                 nat.ptr(offsets), nat.ptr(total)))
+    return total
 
 
 class Corpus:
@@ -226,6 +283,18 @@ class Corpus:
         nat.check(nat.lib().pbx_search_page(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(cur), nat.ptr(fids), fids.size, mode,
                                             nat.ptr(hits), nat.ptr(cnt)))
         return _hits_results(hits, cnt)
+
+    def search_range(self, queries, max_dist: float = nat.DEFAULT_MAX_DIST, *, limit: Optional[int] = None, within=None,
+                     excluding=None, after=None) -> List[RangeResult]:
+        """pbx_search_range: every row with dist < max_dist, ordered by (dist, image_id), and the exact count -- the
+        similarity query without its LIMIT.  One RangeResult per query.  limit: at most this many rows per query (the
+        first ones; total stays exact), None for all.  within / excluding and after as in search()."""
+        return _search_range(nat.lib().pbx_search_range, self._h, self.dim, self.__len__, queries, max_dist, limit, within,
+                             excluding, after)
+
+    def count_within(self, queries, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None, excluding=None, after=None) -> np.ndarray:
+        """pbx_search_range with capacity 0: COUNT(*) of the rows with dist < max_dist, per query (uint64 array)."""
+        return _count_within(nat.lib().pbx_search_range, self._h, self.dim, queries, max_dist, within, excluding, after)
 
     def search_hits(self, queries, k: int = nat.DEFAULT_K, max_dist: float = nat.DEFAULT_MAX_DIST) -> Tuple[np.ndarray, np.ndarray]:
         """pbx_search_hits: ([nq][k] pbx_hit records, [nq] counts) -- the per-shard half of a sharded search."""
@@ -425,6 +494,16 @@ class MultiDeviceCorpus:
             nat.check(nat.lib().pbx_sharded_search(self._h, nat.ptr(q), nq, k, float(max_dist), nat.ptr(ids), nat.ptr(dist), nat.ptr(dot),
                                                    nat.ptr(n2), nat.ptr(cnt)))
         return [SearchResult(ids[i, :c].copy(), dist[i, :c].copy(), dot[i, :c].copy(), n2[i, :c].copy()) for i, c in enumerate(cnt.tolist())]
+
+    def search_range(self, queries, max_dist: float = nat.DEFAULT_MAX_DIST, *, limit: Optional[int] = None, within=None,
+                     excluding=None, after=None) -> List[RangeResult]:
+        """pbx_sharded_search_range, as Corpus.search_range."""
+        return _search_range(nat.lib().pbx_sharded_search_range, self._h, self.dim, self.__len__, queries, max_dist, limit,
+                             within, excluding, after)
+
+    def count_within(self, queries, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None, excluding=None, after=None) -> np.ndarray:
+        """pbx_sharded_search_range with capacity 0, as Corpus.count_within."""
+        return _count_within(nat.lib().pbx_sharded_search_range, self._h, self.dim, queries, max_dist, within, excluding, after)
 
 
 def merge_hits(gathered: np.ndarray, counts: np.ndarray, k: int) -> Tuple[np.ndarray, np.ndarray]:

@@ -22,6 +22,7 @@
 #include "replace.cuh"
 #include "page.cuh"
 #include "view.cuh"
+#include "range.cuh"
 
 using namespace pbx;
 
@@ -196,6 +197,17 @@ struct pbx_corpus {
     pbx_hit* d_after = nullptr;       // [cut_cap] the cursors of a host-form call
     uint32_t cut_cap = 0;
     PageCut* cur_cut = nullptr;       // cuts of the search (or batch) being enqueued, one per query (NULL: first pages)
+    // range searches (range.cuh): grown on demand and kept, stream-ordered like the rest of the search scratch
+    uint32_t* d_range_cnt = nullptr;  // [kRangeCounters]
+    uint32_t* h_range_cnt = nullptr;  // pinned copy
+    uint2* d_range_cand = nullptr;    // (row, kappa) candidates
+    size_t range_cand_cap = 0;
+    unsigned char* d_range_sort = nullptr;   // per-candidate sort keys, indices and records (RangeSort)
+    size_t range_sort_cap = 0;        // candidates
+    void* d_range_tmp = nullptr;      // radix sort temporary storage
+    size_t range_tmp_bytes = 0;
+    pbx_hit* h_range = nullptr;       // pinned rows of a host-form call
+    size_t h_range_cap = 0;
     // pinned staging
     uint8_t* h_queries = nullptr;
     size_t h_queries_cap = 0;
@@ -653,6 +665,8 @@ extern "C" void pbx_corpus_destroy(pbx_corpus* c) {
     cudaFree(c->d_hits); cudaFree(c->d_cand); cudaFree(c->d_cand_cnt); cudaFree(c->d_tile_counter); cudaFree(c->d_hist);
     cudaFree(c->d_allow); cudaFree(c->d_filter_words); cudaFree(c->d_filter_ids); cudaFree(c->d_cut); cudaFree(c->d_after);
     cudaFree(c->d_view_set);
+    cudaFree(c->d_range_cnt); cudaFree(c->d_range_cand); cudaFree(c->d_range_sort); cudaFree(c->d_range_tmp);
+    cudaFreeHost(c->h_range_cnt); cudaFreeHost(c->h_range);
     cudaFreeHost(c->h_queries); cudaFreeHost(c->h_hits); cudaFreeHost(c->h_stage); cudaFreeHost(c->h_flag);
     if (c->ev_chain) cudaEventDestroy(c->ev_chain);
     if (c->ev_t0) cudaEventDestroy(c->ev_t0);
@@ -2317,6 +2331,274 @@ extern "C" int pbx_search_device_page(pbx_corpus* c, const uint8_t* d_queries, u
     const SearchFilter f = {d_filter_ids, n_filter, filter_mode, true};
     return search_device_impl(c, d_queries, nq, k, max_dist, d_hits, d_count, cuda_stream,
                               filter_mode == PBX_FILTER_EXCLUDE && n_filter == 0 ? nullptr : &f, d_after, true);
+}
+
+// ---- range searches (range.cuh) ------------------------------------------------------------------------------------------
+constexpr size_t kRangeCandMin = size_t(1) << 16;       // first candidate buffer: 512 KB
+
+template <int L, int C, bool RAGGED, int MINB = scan_minb(L * C)>
+static cudaError_t launch_range_scan_as(const pbx_corpus* c, const RangeScanParams& p, cudaStream_t s) {
+    // persistent grid: as many CTAs as are resident at once
+    int per_sm = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, range_scan_kernel<L, C, RAGGED, MINB>, kScanThreads, 0);
+    if (e != cudaSuccess) return e;
+    const int grid = std::min<int>(c->sm_count * std::max(per_sm, 1), (int)kMaxScanGrid);
+    range_scan_kernel<L, C, RAGGED, MINB><<<grid, kScanThreads, 0, s>>>(p);
+    return cudaGetLastError();
+}
+
+// the lane layouts and occupancies of launch_scan_as: compile-time shapes, every other pitch RAGGED
+static cudaError_t launch_range_scan(const pbx_corpus* c, const RangeScanParams& p, cudaStream_t s) {
+    switch (c->pitch16) {
+        case 1: return launch_range_scan_as<1, 1, false>(c, p, s);
+        case 2: return launch_range_scan_as<2, 1, false>(c, p, s);
+        case 4: return launch_range_scan_as<4, 1, false>(c, p, s);
+        case 8: return launch_range_scan_as<8, 1, false>(c, p, s);
+        case 16: return launch_range_scan_as<16, 1, false, 3>(c, p, s);
+        case 32: return launch_range_scan_as<32, 1, false>(c, p, s);
+        case 64: return launch_range_scan_as<32, 2, false>(c, p, s);
+        case 128: return launch_range_scan_as<32, 4, false>(c, p, s);
+#define PBX_RANGE_CASE_M(LL, CC, MM) case (LL) * (CC): return launch_range_scan_as<LL, CC, false, MM>(c, p, s);
+        PBX_EXTRA_SHAPES(PBX_RANGE_CASE_M)
+#undef PBX_RANGE_CASE_M
+        default:
+#define PBX_RANGE_CASE_R(LL, CC, MM) if (c->pitch16 <= (LL) * (CC)) return launch_range_scan_as<LL, CC, true, MM>(c, p, s);
+            PBX_RAGGED_SHAPES(PBX_RANGE_CASE_R)
+#undef PBX_RANGE_CASE_R
+            return cudaErrorInvalidValue;
+    }
+}
+
+// The per-candidate arrays of the (dist, image_id) sort, carved out of one allocation.
+struct RangeSort {
+    uint32_t *key_dist, *key_dist2, *index, *index2;
+    u64 *key_id, *key_id2;
+    pbx_hit *recs, *out;
+};
+static RangeSort range_sort_arrays(unsigned char* base, size_t cap) {
+    auto take = [&](size_t bytes) { unsigned char* p = base; base += (bytes + 255) & ~size_t(255); return p; };
+    RangeSort a;
+    a.key_dist = reinterpret_cast<uint32_t*>(take(cap * 4)); a.key_dist2 = reinterpret_cast<uint32_t*>(take(cap * 4));
+    a.index = reinterpret_cast<uint32_t*>(take(cap * 4)); a.index2 = reinterpret_cast<uint32_t*>(take(cap * 4));
+    a.key_id = reinterpret_cast<u64*>(take(cap * 8)); a.key_id2 = reinterpret_cast<u64*>(take(cap * 8));
+    a.recs = reinterpret_cast<pbx_hit*>(take(cap * sizeof(pbx_hit))); a.out = reinterpret_cast<pbx_hit*>(take(cap * sizeof(pbx_hit)));
+    return a;
+}
+static size_t range_sort_bytes(size_t cap) { return 4 * ((cap * 4 + 255) & ~size_t(255)) + 2 * ((cap * 8 + 255) & ~size_t(255)) + 2 * ((cap * sizeof(pbx_hit) + 255) & ~size_t(255)); }
+
+static int ensure_range_cand(pbx_corpus* c, size_t n) {
+    if (!c->d_range_cnt) {
+        CU_TRY(cudaMalloc(&c->d_range_cnt, kRangeCounters * sizeof(uint32_t)));
+        CU_TRY(cudaMallocHost(&c->h_range_cnt, kRangeCounters * sizeof(uint32_t)));
+    }
+    n = std::max(n, kRangeCandMin);
+    if (n <= c->range_cand_cap) return PBX_OK;
+    CU_TRY(cudaDeviceSynchronize());
+    cudaFree(c->d_range_cand); c->d_range_cand = nullptr; c->range_cand_cap = 0;
+    CU_TRY(cudaMalloc(&c->d_range_cand, n * sizeof(uint2)));
+    c->range_cand_cap = n;
+    return PBX_OK;
+}
+
+static int ensure_range_sort(pbx_corpus* c, size_t n) {
+    if (n <= c->range_sort_cap) return PBX_OK;
+    n = std::max(n, c->range_sort_cap + c->range_sort_cap / 2);
+    if (n > 0xFFFFFFFFull) return fail(PBX_E_CAPACITY, "range answer of %llu candidates", (unsigned long long)n);
+    size_t t64 = 0, t32 = 0;
+    CU_TRY(range_sort_pairs(nullptr, t64, (const u64*)nullptr, (u64*)nullptr, nullptr, nullptr, (uint32_t)n, nullptr));
+    CU_TRY(range_sort_pairs(nullptr, t32, (const uint32_t*)nullptr, (uint32_t*)nullptr, nullptr, nullptr, (uint32_t)n, nullptr));
+    CU_TRY(cudaDeviceSynchronize());
+    cudaFree(c->d_range_sort); cudaFree(c->d_range_tmp);
+    c->d_range_sort = nullptr; c->d_range_tmp = nullptr; c->range_sort_cap = 0; c->range_tmp_bytes = 0;
+    CU_TRY(cudaMalloc(&c->d_range_sort, range_sort_bytes(n)));
+    CU_TRY(cudaMalloc(&c->d_range_tmp, std::max(t64, t32)));
+    c->range_sort_cap = n;
+    c->range_tmp_bytes = std::max(t64, t32);
+    return PBX_OK;
+}
+
+static int ensure_range_host(pbx_corpus* c, size_t n) {
+    if (n <= c->h_range_cap) return PBX_OK;
+    n = std::max(n, c->h_range_cap + c->h_range_cap / 2);
+    cudaFreeHost(c->h_range); c->h_range = nullptr; c->h_range_cap = 0;
+    CU_TRY(cudaMallocHost(&c->h_range, n * sizeof(pbx_hit)));
+    c->h_range_cap = n;
+    return PBX_OK;
+}
+
+static unsigned range_blocks(const pbx_corpus* c, size_t n, unsigned threads) {
+    return (unsigned)std::max<size_t>(1, std::min<size_t>((n + threads - 1) / threads, (size_t)c->sm_count * 8));
+}
+
+// Orders a.recs[0, n) by (dist, image_id) -- a.key_id / a.key_dist / a.index filled -- and writes the first n_out to a.out.
+// Two stable LSD radix sorts: by image_id, then by dist.
+static int range_sort(pbx_corpus* c, const RangeSort& a, uint32_t n, uint32_t n_out, cudaStream_t s) {
+    size_t tb = c->range_tmp_bytes;
+    CU_TRY(range_sort_pairs(c->d_range_tmp, tb, a.key_id, a.key_id2, a.index, a.index2, n, s));
+    range_permute_keys_kernel<<<range_blocks(c, n, 256), 256, 0, s>>>(a.key_dist, a.index2, n, a.key_dist2);
+    CU_TRY(cudaGetLastError());
+    tb = c->range_tmp_bytes;
+    CU_TRY(range_sort_pairs(c->d_range_tmp, tb, a.key_dist2, a.key_dist, a.index2, a.index, n, s));
+    if (n_out) {
+        range_gather_kernel<<<range_blocks(c, n_out, 256), 256, 0, s>>>(a.recs, a.index, n_out, a.out);
+        CU_TRY(cudaGetLastError());
+    }
+    return PBX_OK;
+}
+
+// One query of a range search.  Caller holds c->mu; stream s is ordered after ev_chain; `allow` is the filter bitmap
+// (NULL: none) and `cut` the query's cursor cut (NULL: none), both on the device.  cap = the rows wanted at most (0: count
+// only).  On return *total is the exact count and the first min(total, cap) rows are at *d_rows on the device, and also in
+// c->h_range when to_host.  Host reads: the candidate count, then the hit count (with the rows).
+static int range_query(pbx_corpus* c, const uint8_t* d_query, uint32_t n, double max_dist, const uint32_t* allow, const PageCut* cut,
+                       uint64_t cap, cudaStream_t s, bool to_host, uint64_t* total, const pbx_hit** d_rows) {
+    *total = 0;
+    if (d_rows) *d_rows = nullptr;
+    if (n == 0) return PBX_OK;
+    int rc = ensure_query_scratch(c, 1);
+    if (rc == PBX_OK) rc = ensure_range_cand(c, 0);
+    if (rc != PBX_OK) return rc;
+    {   // the query's centred values and sums: prep_seed_kernel without its sample
+        PrepSeedParams ps;
+        memset(&ps, 0, sizeof(ps));
+        ps.query = d_query;
+        ps.dim = c->dim; ps.pitch = c->pitch; ps.pitch16 = c->pitch16;
+        ps.q16 = c->d_q16; ps.qbytes = c->d_qbytes; ps.qh = c->d_qh;
+        ps.rows = reinterpret_cast<const uint4*>(c->d_rows); ps.inv_norm = c->d_inv; ps.n = n; ps.keep = 1;
+        ps.do_seed = 0;
+        ps.seed_hist = c->d_hist + kHistBins; ps.ticket = c->d_tile_counter + 96; ps.gbin = c->d_tile_counter + 32;
+        CU_TRY(launch_pdl<PrepSeedParams>(prep_seed_kernel, 1, kSeedThreads, (size_t)c->pitch * 2, s, ps));
+    }
+    const bool count_only = cap == 0;
+    const float m = dist_bound(max_dist);
+    RangeScanParams rp;
+    rp.rows = reinterpret_cast<const uint4*>(c->d_rows); rp.inv_norm = c->d_inv; rp.n = n; rp.pitch16 = c->pitch16;
+    rp.q16 = c->d_q16; rp.qh = c->d_qh; rp.allow = allow; rp.cut = cut; rp.m = m; rp.count_only = count_only ? 1u : 0u;
+    rp.margin = (double)certificate_margin(c->dim); rp.counters = c->d_range_cnt;
+    uint32_t n_cand = 0;
+    for (;;) {
+        rp.cand = c->d_range_cand;
+        rp.cand_cap = (uint32_t)std::min<size_t>(c->range_cand_cap, 0xFFFFFFFFull);
+        CU_TRY(cudaMemsetAsync(c->d_range_cnt, 0, kRangeCounters * sizeof(uint32_t), s));
+        CU_TRY(launch_range_scan(c, rp, s));
+        CU_TRY(cudaMemcpyAsync(c->h_range_cnt, c->d_range_cnt, kRangeCounters * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CU_TRY(cudaStreamSynchronize(s));
+        n_cand = c->h_range_cnt[kRangeCand];
+        if (n_cand <= rp.cand_cap) break;
+        rc = ensure_range_cand(c, n_cand);       // overflowed: the exact size, and the pass once more
+        if (rc != PBX_OK) return rc;
+    }
+    const uint32_t direct = c->h_range_cnt[kRangeDirect];
+    if (n_cand == 0) { *total = direct; return PBX_OK; }
+    RangeReplayParams xp;
+    memset(&xp, 0, sizeof(xp));
+    xp.rows = c->d_rows; xp.ids = c->d_ids; xp.pitch = c->pitch; xp.dim = c->dim;
+    xp.qbytes = c->d_qbytes; xp.q16 = c->d_q16; xp.qh = c->d_qh; xp.cut = cut; xp.m = m;
+    xp.n_cand = n_cand; xp.cand = c->d_range_cand; xp.counters = c->d_range_cnt;
+    RangeSort a;
+    memset(&a, 0, sizeof(a));
+    if (!count_only) {
+        rc = ensure_range_sort(c, n_cand);
+        if (rc != PBX_OK) return rc;
+        a = range_sort_arrays(c->d_range_sort, c->range_sort_cap);
+        xp.key_dist = a.key_dist; xp.key_id = a.key_id; xp.index = a.index; xp.recs = a.recs;
+    }
+    range_replay_kernel<<<range_blocks(c, n_cand, kRangeReplayThreads), kRangeReplayThreads, 0, s>>>(xp);
+    CU_TRY(cudaGetLastError());
+    const uint32_t n_out = (uint32_t)std::min<uint64_t>(n_cand, cap);    // >= the rows returned: every hit is a candidate
+    if (!count_only) {
+        rc = range_sort(c, a, n_cand, n_out, s);
+        if (rc != PBX_OK) return rc;
+        if (d_rows) *d_rows = a.out;
+        if (to_host) {
+            rc = ensure_range_host(c, n_out);
+            if (rc != PBX_OK) return rc;
+            CU_TRY(cudaMemcpyAsync(c->h_range, a.out, (size_t)n_out * sizeof(pbx_hit), cudaMemcpyDeviceToHost, s));
+        }
+    }
+    CU_TRY(cudaMemcpyAsync(c->h_range_cnt + kRangeHits, c->d_range_cnt + kRangeHits, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    *total = (uint64_t)direct + c->h_range_cnt[kRangeHits];
+    return PBX_OK;
+}
+
+// The set-up of a range search on one corpus: order after the previous search, mark the filter, derive the cursor cuts.
+// Caller holds c->mu.  *cuts = NULL without cursors.
+static int range_begin(pbx_corpus* c, uint32_t n, const SearchFilter* filter, const pbx_hit* after, uint32_t nq, cudaStream_t s,
+                       const uint32_t** allow, const PageCut** cuts) {
+    *allow = nullptr; *cuts = nullptr;
+    c->cur_allow = nullptr; c->cur_allowed = nullptr; c->cur_cut = nullptr;
+    if (c->chain_valid) CU_TRY(cudaStreamWaitEvent(s, c->ev_chain, 0));
+    if (filter) {
+        int rc = enqueue_filter_mark(c, *filter, n, s);
+        if (rc != PBX_OK) return rc;
+        *allow = c->cur_allow;
+        c->cur_allow = nullptr; c->cur_allowed = nullptr;
+    }
+    if (after) {
+        int rc = ensure_page_scratch(c, nq);
+        if (rc != PBX_OK) return rc;
+        CU_TRY(cudaMemcpyAsync(c->d_after, after, (size_t)nq * sizeof(pbx_hit), cudaMemcpyHostToDevice, s));
+        page_cut_kernel<<<(nq + 255) / 256, 256, 0, s>>>(c->d_after, nq, (double)certificate_margin(c->dim), c->d_cut);
+        CU_TRY(cudaGetLastError());
+        *cuts = c->d_cut;
+    }
+    return PBX_OK;
+}
+
+static int range_end(pbx_corpus* c, cudaStream_t s) {
+    CU_TRY(cudaEventRecord(c->ev_chain, s));
+    c->chain_valid = true;
+    return PBX_OK;
+}
+
+static int check_range_args(const void* handle, const uint8_t* queries, uint32_t nq, pbx_hit* out_hits, uint64_t capacity,
+                            uint64_t* out_offsets, uint64_t* out_total) {
+    if (!handle) return fail(PBX_E_INVALID, "corpus is NULL");
+    if (nq && !queries) return fail(PBX_E_INVALID, "queries is NULL");
+    if (!out_offsets || !out_total) return fail(PBX_E_INVALID, "NULL output");
+    if (capacity && !out_hits) return fail(PBX_E_INVALID, "NULL output: out_hits with capacity = %llu", (unsigned long long)capacity);
+    return PBX_OK;
+}
+
+extern "C" int pbx_search_range(pbx_corpus* c, const uint8_t* queries, uint32_t nq, double max_dist, const pbx_hit* after,
+                                const int64_t* filter_ids, uint64_t n_filter, uint32_t filter_mode, pbx_hit* out_hits, uint64_t capacity,
+                                uint64_t* out_offsets, uint64_t* out_total) {
+    std::vector<int64_t> sorted;
+    SearchFilter f;
+    const SearchFilter* fp = nullptr;
+    int rc = host_page(after, nq, filter_ids, n_filter, filter_mode, &sorted, &f, &fp);
+    if (rc != PBX_OK) return rc;
+    rc = check_range_args(c, queries, nq, out_hits, capacity, out_offsets, out_total);
+    if (rc != PBX_OK) return rc;
+    out_offsets[0] = 0;
+    if (nq == 0) return PBX_OK;
+    rc = flush_pending(c);                          // coalesced appends become visible before the search (append lock only)
+    if (rc != PBX_OK) return rc;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CU_TRY(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    const uint32_t n = (uint32_t)c->n.load();
+    const uint32_t* allow = nullptr;
+    const PageCut* cuts = nullptr;
+    rc = range_begin(c, n, fp, after, nq, s, &allow, &cuts);
+    if (rc != PBX_OK) return rc;
+    rc = ensure_query_scratch(c, 1);
+    if (rc != PBX_OK) return rc;
+    uint64_t written = 0;
+    for (uint32_t q = 0; q < nq; ++q) {
+        CU_TRY(cudaMemcpyAsync(c->d_queries, queries + (size_t)q * c->dim, c->dim, cudaMemcpyHostToDevice, s));
+        uint64_t total = 0;
+        rc = range_query(c, c->d_queries, n, max_dist, allow, cuts ? cuts + q : nullptr, capacity - written, s, true, &total, nullptr);
+        if (rc != PBX_OK) return rc;
+        const uint64_t w = std::min<uint64_t>(total, capacity - written);
+        if (w) memcpy(out_hits + written, c->h_range, (size_t)w * sizeof(pbx_hit));
+        written += w;
+        out_offsets[q + 1] = written;
+        out_total[q] = total;
+    }
+    c->queries += nq;
+    return range_end(c, s);
 }
 
 extern "C" int pbx_merge_hits(const pbx_hit* gathered, const uint32_t* counts, uint32_t n_shards, uint32_t nq, uint32_t k,

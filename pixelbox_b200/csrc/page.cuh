@@ -39,6 +39,36 @@ __device__ __forceinline__ PageCut page_cut(const pbx_hit& h, double margin) {
     return pc;
 }
 
+// The two cuts of a range search (range.cuh) for the f32 bound m = dist_bound(max_dist), with c* = 1/(m + 1) and the
+// certificate margin M (DESIGN.md section 5, "Range searches"):
+//   kappa > kappa_in  ->  dist < m  (certainly inside: page_cut's kappa_hi(m), rounded up)
+//   kappa < kappa_lo  ->  dist >= m (certainly outside: c* - M * max(1, c*), rounded down)
+//   m NaN            -> no row is inside: both +inf
+//   m > 999999       -> every dist is <= 999999 < m: both -inf
+//   m + 1 <= 0       -> every dist is > -1 >= m: both +inf
+struct RangeCut {
+    float kappa_lo, kappa_in;
+};
+__device__ __forceinline__ RangeCut range_cut(float m, double margin) {
+    const float inf = __int_as_float(0x7f800000);
+    RangeCut rc;
+    if (m != m) {
+        rc.kappa_lo = inf; rc.kappa_in = inf;
+    } else if (m > PBX_PLATEAU_DIST) {
+        rc.kappa_lo = -inf; rc.kappa_in = -inf;
+    } else {
+        const double den = (double)m + 1.0;
+        if (den <= 0.0) {
+            rc.kappa_lo = inf; rc.kappa_in = inf;
+        } else {
+            const double cs = 1.0 / den, w = margin * fmax(1.0, cs);
+            rc.kappa_in = __double2float_ru(cs + w);
+            rc.kappa_lo = __double2float_rd(cs - w);
+        }
+    }
+    return rc;
+}
+
 __global__ void page_cut_kernel(const pbx_hit* __restrict__ after, uint32_t nq, double margin, PageCut* __restrict__ out) {
     for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += gridDim.x * blockDim.x) out[q] = page_cut(after[q], margin);
 }

@@ -174,22 +174,44 @@ class Engine:
         t0 = time.perf_counter()
         results: List[IndexedImage] = []
         if self.corpus is not None:
-            corpus = self.corpus
-            if folder is not None:
-                # the folder's rows are kept as a view of the corpus, made on first use: its searches cost the folder's
-                # rows, not the table's, and the corpus keeps it current as hashes are appended, removed or replaced
-                prefix = folder if folder.endswith(("/", "\\")) else folder + "/"
-                corpus = self.folder_views.get(prefix)
-                if corpus is None:
-                    ids = np.fromiter((r[0] for r in self.read_connection.execute(
-                        "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
-                    corpus = self.folder_views[prefix] = self.corpus.view(ids)
+            corpus = self.corpus if folder is None else self._folder_view(folder)
             # what load_more_results continues from: the query, its max_dist and folder's view, the last GPU row consumed
             self._last_query = dict(query=np.frombuffer(indexed_image.visual_hash, np.uint8), max_dist=self.max_distance_from_query,
                                     corpus=corpus, cursor=None, exhausted=False)
             results = self._joined_rows(DEFAULT_MAX_SEARCH_RESULTS)                  # LIMIT 100, :381
         self.cached_search_results = results
         sys.stderr.write(f"Time to search DB: {time.perf_counter() - t0:.6f}s  Results: {len(results)}\n")
+
+    def _folder_view(self, folder: str) -> Corpus:
+        """The folder's rows are kept as a view of the corpus, made on first use: its searches cost the folder's rows, not
+        the table's, and the corpus keeps it current as hashes are appended, removed or replaced."""
+        prefix = folder if folder.endswith(("/", "\\")) else folder + "/"
+        view = self.folder_views.get(prefix)
+        if view is None:
+            ids = np.fromiter((r[0] for r in self.read_connection.execute(
+                "SELECT id FROM images WHERE substr(path, 1, length(?)) = ? ORDER BY id", (prefix, prefix))), dtype=np.int64)
+            view = self.folder_views[prefix] = self.corpus.view(ids)
+        return view
+
+    def similar_image_ids(self, indexed_image: IndexedImage, max_distance: Optional[float] = None,
+                          folder: Optional[str] = None) -> List[Tuple[int, float]]:
+        """[(image_id, dist)] of every image with dist < max_distance (default max_distance_from_query), ordered by dist
+        then id: the similarity SQL of query_by_image_hash_from_image without its LIMIT, INNER JOIN with `images` included
+        (a hash without an image row is dropped).  folder: only the images under it, as query_by_image_hash_within_folder.
+        Nothing is hydrated -- the ids are for a bulk action such as "select every duplicate" then remove_images.  One
+        range search (Corpus.search_range) and one indexed lookup per 500 rows of its answer."""
+        if indexed_image.visual_hash is None or self.corpus is None:
+            return []
+        corpus = self.corpus if folder is None else self._folder_view(folder)
+        md = self.max_distance_from_query if max_distance is None else float(max_distance)
+        res = corpus.search_range(np.frombuffer(indexed_image.visual_hash, np.uint8), md)[0]
+        ids = res.ids.tolist()
+        joined = set()
+        for i in range(0, len(ids), 500):
+            part = ids[i:i + 500]
+            joined.update(r[0] for r in self.read_connection.execute(
+                f"SELECT id FROM images WHERE id IN ({','.join('?' * len(part))})", part))
+        return [(i, float(d)) for i, d in zip(ids, res.dist.tolist()) if i in joined]
 
     def _joined_rows(self, count: int) -> List[IndexedImage]:
         """The next `count` rows of the last similarity query that have an `images` row (INNER JOIN semantics), hydrated

@@ -19,7 +19,7 @@ import torch
 import torch.distributed as dist
 
 from . import _native as nat
-from .corpus import Corpus, SearchResult, merge_hits
+from .corpus import Corpus, RangeResult, SearchResult, merge_hits
 
 HIT_BYTES = nat.HIT_DTYPE.itemsize
 
@@ -273,6 +273,52 @@ class ShardedCorpus:
             hits, cnt = merge_hits(gathered, counts, k)
         return [SearchResult(hits[i]["image_id"][:cnt[i]].copy(), hits[i]["dist"][:cnt[i]].copy(),
                              hits[i]["dot"][:cnt[i]].copy(), hits[i]["norm2"][:cnt[i]].copy()) for i in range(nq)]
+
+    def _all_gather_i64(self, values) -> np.ndarray:
+        """[world][len(values)] int64 of every rank's values."""
+        mine = np.ascontiguousarray(np.asarray(values, dtype=np.int64).reshape(-1))
+        return self._all_gather_bytes(mine.view(np.uint8)).view(np.int64).reshape(self.world, -1)
+
+    def count_within(self, queries, max_dist: float = nat.DEFAULT_MAX_DIST, *, within=None, excluding=None, after=None) -> np.ndarray:
+        """Corpus.count_within over the table (every rank passes the same arguments): the shards' counts, summed."""
+        if not isinstance(self.local, Corpus):
+            raise nat.PbxError(-1, "a range search needs GPU shards")
+        mine = self.local.count_within(queries, max_dist, within=within, excluding=excluding, after=after)
+        return self._all_gather_i64(mine.astype(np.int64)).sum(axis=0).astype(np.uint64)
+
+    def search_range(self, queries, max_dist: float = nat.DEFAULT_MAX_DIST, *, limit: Optional[int] = None, within=None,
+                     excluding=None, after=None) -> List[RangeResult]:
+        """Corpus.search_range over the table (every rank passes the same arguments), on every rank: each shard's range
+        search, an all-gather of the totals and of the shards' first rows (each padded to the same length with dist =
+        +inf), then the merge kernel on this rank's device.  The first `limit` rows of the table lie among the first
+        `limit` rows of each shard, so the merge is exact."""
+        if not isinstance(self.local, Corpus):
+            raise nat.PbxError(-1, "a range search needs GPU shards")
+        local = self.local.search_range(queries, max_dist, limit=limit, within=within, excluding=excluding, after=after)
+        nq = len(local)
+        g = self._all_gather_i64([r.total for r in local] + [len(r.ids) for r in local])
+        totals, lens = g[:, :nq].sum(axis=0), g[:, nq:]
+        out = []
+        for i, r in enumerate(local):
+            k = int(lens[:, i].sum()) if limit is None else min(int(limit), int(lens[:, i].sum()))
+            if k == 0:
+                e = np.zeros(0, nat.HIT_DTYPE)
+                out.append(RangeResult(e["image_id"], e["dist"], e["dot"], e["norm2"], int(totals[i])))
+                continue
+            mine = np.zeros(k, nat.HIT_DTYPE)
+            mine["image_id"], mine["dist"] = np.iinfo(np.int64).max, np.inf      # padding: no row has dist = +inf
+            m = min(len(r.ids), k)
+            mine["image_id"][:m], mine["dist"][:m], mine["dot"][:m], mine["norm2"][:m] = r.ids[:m], r.dist[:m], r.dot[:m], r.norm2[:m]
+            gathered = torch.from_numpy(self._all_gather_bytes(mine.view(np.uint8)).reshape(-1)).to(self._dev())
+            merged = torch.empty(k * HIT_BYTES, dtype=torch.uint8, device=self._dev())
+            cnt = torch.empty(1, dtype=torch.int32, device=self._dev())
+            stream = torch.cuda.current_stream().cuda_stream
+            nat.check(nat.lib().pbx_merge_hits_device(self.device, gathered.data_ptr(), None, self.world, 1, k, merged.data_ptr(),
+                                                      cnt.data_ptr(), stream if stream else 1))
+            hits = merged.cpu().numpy().view(nat.HIT_DTYPE)[:int(cnt.cpu().item())]
+            out.append(RangeResult(hits["image_id"].copy(), hits["dist"].copy(), hits["dot"].copy(), hits["norm2"].copy(),
+                                   int(totals[i])))
+        return out
 
     def close(self) -> None:
         if getattr(self, "_view_of", None) is not None:     # a view: the exchange belongs to the corpus it views
